@@ -3,6 +3,7 @@
 line, the other configurations of SURVEY.md §8(d).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode random|step|config3|policy|train]
+                    [--dump-outputs DIR]
 
 Headline (mode "random", the default): one bench "step" = ONE launch of the fused rollout kernel (azb_rollout_random:
 legal mask + random agent + Azul.step + scoring + refill + auto-reset) that advances every one of the G games by
@@ -23,6 +24,10 @@ The JSON line carries
              per GPU), policy (configs[3]: fused tcgen05 policy kernel self-play) and train (configs[4]: rollouts + A2C
              update + gradient all-reduce), each measured like the headline with its own clocks and roofline
 --impl reference times the reference arm for this tier: the oracle port on all host threads, same config / metric / unit.
+--dump-outputs DIR writes what the measured path (the headline, or the --mode) returned in its last timed step: random and
+config3: state (packed words [W, G]), legal_mask ([6, G]), counters; step: state, legal_mask, done, status; policy: state,
+counters; train: the network's parameters (param.*) and the last batch's statistics (stat.*).  The inputs are seeded, so
+two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -72,9 +77,18 @@ def parse_args():
                     help="--mode step: random-agent env steps before the timed step (0 = fresh games: no round can end)")
     ap.add_argument("--policy-k", type=int, default=64, help="policy: decisions per game per launch of the persistent self-play kernel")
     ap.add_argument("--no-graph", action="store_true", help="train: run the batch launch by launch instead of as one CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the measured path returned in its last step as DIR/<name>.npy "
+                         "(integers as float64, floating point as float32; rank 0's games; at most 64 MB, a fixed sample "
+                         "of the games beyond that)")
     ap.add_argument("--pyref-worker", type=float, default=None, help=argparse.SUPPRESS)
     ap.add_argument("--pyref-kind", default="runner", choices=["runner", "selfplay", "train"], help=argparse.SUPPRESS)
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
+    return args
 
 
 def workload_config(args, n_gpus, games=None, players=None):
@@ -501,6 +515,9 @@ def measure_random(args, ctx, players, games, steps, warmup, e2e=True):
     kernel_ms = [a.elapsed_time(b) for a, b in ev]
     dev_ms = sum(kernel_ms)
     dev_ms_max = ctx.max_over_ranks(dev_ms)
+    outputs = None
+    if args.dump_outputs:                        # copied now: the e2e leg below rolls the same engine on
+        outputs = ({"state": eng.state.clone(), "legal_mask": mask.clone()}, {"counters": eng.counters.clone()})
     out_e2e = None
     if e2e:
         # ---- end to end through the host API ----
@@ -559,7 +576,7 @@ def measure_random(args, ctx, players, games, steps, warmup, e2e=True):
             "ms_per_step": dev_ms_max / steps, "e2e": out_e2e, "gpu_launches": steps, "roofline": roof, "clocks": clocks,
             "wall_s": wall, "games_per_sec": (cnt[1] / max(cnt[0], 1)) * value,
             "rollout_counters": {"steps": cnt[0], "games": cnt[1], "rounds": cnt[2], "stuck": cnt[6]},
-            "config": workload_config(args, world, games=G, players=players)}
+            "config": workload_config(args, world, games=G, players=players), "outputs": outputs}
 
 
 def measure_step(args, ctx, games, players, steps, warmup):
@@ -621,8 +638,9 @@ def measure_step(args, ctx, games, players, steps, warmup):
     cfg["actions"] = "%s legal action per game after %d random-agent steps; %.1f %% of the games end their round (score + refill) in the timed step" % (
         args.step_actions, args.presteps, 100 * round_ends)
     cfg["l2"] = "working set %.0f MB per launch (state %d B + 28 B per game) exceeds the 126 MB L2; the state is restored from a snapshot before every launch" % (G * b_alg / 1e6, 4 * eng.W)
+    outputs = ({"state": eng.state, "legal_mask": mask, "done": done, "status": status}, {}) if args.dump_outputs else None
     return {"value": ctx.world * G / t, "unit": UNIT, "n_gpus": ctx.world, "steps": steps, "warmup": warmup, "ms_per_step": 1e3 * t,
-            "dtype": "u32", "config": cfg, "gpu_launches": steps, "clocks": clocks,
+            "dtype": "u32", "config": cfg, "gpu_launches": steps, "clocks": clocks, "outputs": outputs,
             "roofline": {"bound": "hbm", "achieved": G * b_alg / t / 1e9, "peak": peak, "unit": "GB/s",
                          "frac": G * b_alg / t / 1e9 / peak,
                          "traffic": profiled("step_p%d_%s_g%d_%s" % (players, pool_name, G, args.step_actions)),
@@ -679,6 +697,9 @@ def measure_policy(args, ctx, games, steps, warmup):
     ctx.barrier()
     clocks = sampler.stop() if ctx.rank == 0 else None
     dev_ms = ctx.max_over_ranks(ev0.elapsed_time(ev1))
+    outputs = None
+    if args.dump_outputs:                        # copied now: the e2e leg below plays the same games on
+        outputs = ({"state": eng.state.clone()}, {"counters": eng.counters.clone()})
     # end to end: pinned host state in, K decisions per game, state + the last decision's action / logp / value + counters out
     host_state = torch.empty(eng.state.shape, dtype=torch.int32).pin_memory()
     host_state.copy_(eng.state)
@@ -716,7 +737,8 @@ def measure_policy(args, ctx, games, steps, warmup):
                          "algorithmic_flop_per_decision": flop, "decisions_per_launch": G * K,
                          "kernel": "pol::k_policy_rollout<%d>" % ctx.pool},
             "clocks": clocks, "decisions_per_sec": value, "games_per_sec": (cnt[1] / max(cnt[0], 1)) * value,
-            "accuracy": accuracy, "rollout_counters": {"steps": cnt[0], "games": cnt[1], "rounds": cnt[2], "stuck": cnt[6]}}
+            "accuracy": accuracy, "rollout_counters": {"steps": cnt[0], "games": cnt[1], "rounds": cnt[2], "stuck": cnt[6]},
+            "outputs": outputs}
 
 
 def measure_train(args, ctx, games, steps, warmup):
@@ -760,6 +782,10 @@ def measure_train(args, ctx, games, steps, warmup):
     last = None
     for _ in range(steps):
         last = tr.fetch_stats()                      # every batch's statistics reached the host
+    outputs = None
+    if args.dump_outputs:                        # the trained network and the last batch's statistics (not its host wait time)
+        outputs = ({}, {**{"param." + n: p.detach() for n, p in tr.net.named_parameters()},
+                        **{"stat." + k: torch.tensor(float(v), dtype=torch.float64) for k, v in last.items() if k != "update_sync_s"}})
     env_steps, n_games = steps_word() - s0, games * steps
     dev_ms = ctx.max_over_ranks(ev0.elapsed_time(ev1))
     tot = torch.tensor([float(env_steps), float(n_games)], dtype=torch.float64, device=ctx.dev)
@@ -783,7 +809,8 @@ def measure_train(args, ctx, games, steps, warmup):
             "rollout_ms": statistics.median(roll_ms), "update_ms": statistics.median(upd_ms),
             "allreduce_and_stats_ms": statistics.median(sync_ms), "cuda_graph": graph,
             "launch_by_launch_step_ms": [round(a + b, 2) for a, b in zip(roll_ms, upd_ms)],
-            "last_batch": {k: last[k] for k in ("reward", "ac_loss", "win_percent", "unfinished")} if last else None}
+            "last_batch": {k: last[k] for k in ("reward", "ac_loss", "win_percent", "unfinished")} if last else None,
+            "outputs": outputs}
 
 
 def finish_line(args, m, extra_keys=()):
@@ -792,9 +819,34 @@ def finish_line(args, m, extra_keys=()):
             "warmup": m["warmup"], "ms_per_step": m["ms_per_step"], "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": m.get("dtype", "u32"), "data": "synthetic", "config": m["config"]}
     for k, v in m.items():
-        if k not in line:
+        if k not in line and k != "outputs":
             line[k] = v
     return line
+
+
+DUMP_BYTES = 63 * 10 ** 6           # array data; the .npy headers stay within the 64 MB of --dump-outputs
+
+
+def dump_outputs(out_dir, per_game, whole):
+    """--dump-outputs: one DIR/<name>.npy per tensor, integers as float64 (exact for 32-bit words and the counters),
+    floating point as float32 (float64 stays float64).  ``per_game`` tensors have the game as their last axis; when
+    everything does not fit DUMP_BYTES, all of them keep the same seeded sample of games, listed in game_index.npy."""
+    import numpy as np
+    import torch
+    wide = lambda t: not t.is_floating_point() or t.dtype == torch.float64      # noqa: E731  written as float64
+    fixed = sum(t.numel() * (8 if wide(t) else 4) for t in whole.values())
+    per = sum(t[..., 0].numel() * (8 if wide(t) else 4) for t in per_game.values())
+    n = next(iter(per_game.values())).shape[-1] if per_game else 0
+    os.makedirs(out_dir, exist_ok=True)
+    if fixed + n * per > DUMP_BYTES:
+        keep = (DUMP_BYTES - fixed) // (per + 8)
+        assert keep > 0, "--dump-outputs: the outputs without a game axis alone exceed the budget"
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        np.save(os.path.join(out_dir, "game_index.npy"), idx.astype(np.float64))
+        per_game = {k: v.index_select(-1, torch.from_numpy(idx).to(v.device)) for k, v in per_game.items()}
+    for name, t in {**per_game, **whole}.items():
+        t = t.detach()
+        np.save(os.path.join(out_dir, name + ".npy"), (t.double() if wide(t) else t.float()).cpu().numpy())
 
 
 def run_b200(args):
@@ -802,14 +854,18 @@ def run_b200(args):
     warm = max(args.warmup, 3)
     mode = args.mode
     if mode == "step":
-        line = finish_line(args, measure_step(args, ctx, args.games, args.players, args.steps, warm))
+        head = measure_step(args, ctx, args.games, args.players, args.steps, warm)
+        line = finish_line(args, head)
     elif mode == "policy":
-        line = finish_line(args, measure_policy(args, ctx, args.games, args.steps, warm))
+        head = measure_policy(args, ctx, args.games, args.steps, warm)
+        line = finish_line(args, head)
     elif mode == "train":
-        line = finish_line(args, measure_train(args, ctx, args.games, args.steps, warm))
+        head = measure_train(args, ctx, args.games, args.steps, warm)
+        line = finish_line(args, head)
     elif mode == "config3":
         ms = {"p%d" % p: measure_random(args, ctx, p, args.games, args.steps, warm, e2e=False) for p in (2, 3, 4)}
-        line = finish_line(args, ms["p%d" % args.players])
+        head = ms["p%d" % args.players]
+        line = finish_line(args, head)
         line["config3"] = {k: {kk: v[kk] for kk in ("value", "ms_per_step", "roofline", "clocks", "games_per_sec")} for k, v in ms.items()}
     else:
         head = measure_random(args, ctx, args.players, args.games, args.steps, warm, e2e=True)
@@ -831,6 +887,8 @@ def run_b200(args):
             extra["train"] = {k: m[k] for k in brief + ("agent_decisions_per_batch", "rollout_ms", "update_ms", "allreduce_and_stats_ms", "launch_by_launch_step_ms", "cuda_graph", "last_batch", "dtype") if k in m}
             line["extra"] = extra
     if ctx.rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *head["outputs"])
         if ctx.world == 1 and not args.no_cpu_baseline and mode == "random":
             threads = os.cpu_count() or 1
             v, n, k, dt = cpu_rollout_rate(args, args.cpu_seconds, threads)

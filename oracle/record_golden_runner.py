@@ -15,12 +15,12 @@ the ``Azul`` traces; this module records what sits on top of them (SURVEY.md §8
   ``forward_critic`` on ``N_MODEL`` reachable states (records, reference ``get_state`` observation from
   the mover's perspective, legal mask): value, entropy term, log-probabilities of sampled legal
   actions, argmax, and the full logit rows of the first ``N_MODEL_FULL`` states; for the default
-  initialisation and for the same parameters scaled by 3 (peaked policies).
+  initialisation and for the same parameters scaled by 3 (peaked policies; those outputs in ``model_s3.npz``).
 * ``update.npz`` -- ``NNRunner.train(batch_size=B, batches=2)`` (nn_runner.py:53-84) on the reference
   ``Agent`` (agent.py:39-62): every decision of both batches (record, observation, mask, sampled
   action, reward), the discounted returns the reference fed to ``Agent.update``, the four loss
   statistics of each update, the gradients left in ``p.grad`` by the first update and the parameters
-  after each Adam step.
+  after each Adam step (those in ``update_steps.npz``).
 
 Hooks are attribute swaps in the reference's module namespaces (the ``random`` module object seen by
 ``azulnet.azul``, the ``Azul`` name seen by ``azulnet.game_runner``, bound methods of live objects);
@@ -235,8 +235,8 @@ def record_model(ref, out_dir, model_pool):
     torch.manual_seed(0)
     agent = ref.Agent()                                        # agent.py:31-34: ActorCritic(136, 180)
     net = agent.ac_net
+    # the parameters are not stored here: they equal update.npz's param0_* (the same Agent() under torch.manual_seed(0))
     out = dict(records=recs, obs=obs, mask=masks, sel_actions=sel)
-    out.update({"param_" + n: v for n, v in get_params(net).items()})
     x = torch.from_numpy(obs.astype(np.float32))
     m = torch.from_numpy(valid)
     for tag, scale in (("s1", 1.0), ("s3", 3.0)):
@@ -259,6 +259,7 @@ def record_model(ref, out_dir, model_pool):
         out[tag + "_logits_sel"] = np.take_along_axis(logits.numpy(), sel.astype(np.int64), axis=1).astype(np.float32)
     out["scales"] = np.asarray([1.0, 3.0], dtype=np.float32)
     path = os.path.join(out_dir, "model.npz")
+    np.savez_compressed(os.path.join(out_dir, "model_s3.npz"), **{k: out.pop(k) for k in list(out) if k.startswith("s3_")})
     np.savez_compressed(path, **out)
     print("model.npz: %d states (%d with full logit rows), %.1f KiB" % (N_MODEL, N_MODEL_FULL, os.path.getsize(path) / 1024))
 
@@ -335,6 +336,8 @@ def record_update(ref, out_dir):
         out["param1_" + n] = updates[0]["params"][n]
         out["param2_" + n] = updates[1]["params"][n]
     path = os.path.join(out_dir, "update.npz")
+    np.savez_compressed(os.path.join(out_dir, "update_steps.npz"),
+                        **{k: out.pop(k) for k in list(out) if k.startswith(("param1_", "param2_"))})
     np.savez_compressed(path, **out)
     print("update.npz: %d decisions in 2 batches of %d episodes, losses %s, %.1f KiB" % (
         D, UPDATE_EPISODES, np.array2string(out["losses"], precision=4), os.path.getsize(path) / 1024))

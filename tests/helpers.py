@@ -100,14 +100,28 @@ PARAM_NAMES = ["actor_linear1.weight", "actor_linear1.bias", "actor_linear2.weig
                "critic_linear1.weight", "critic_linear1.bias", "critic_linear2.weight", "critic_linear2.bias"]
 
 
+def _load_golden(*names):
+    out = {}
+    for name in names:
+        z = np.load(os.path.join(GOLDEN, name))
+        out.update({k: z[k] for k in z.files})
+    return out
+
+
 def load_model_golden():
-    z = np.load(os.path.join(GOLDEN, "model.npz"))
-    return {k: z[k] for k in z.files}
+    """model.npz: the decision states and the outputs at the default parameters (s1_*); model_s3.npz: the outputs at the
+    parameters scaled by 3.  The parameters (param_*) are update.npz's param0_*: both goldens record ``Agent()`` under
+    ``torch.manual_seed(0)``, so they are stored once."""
+    z = _load_golden("model.npz", "model_s3.npz")
+    u = np.load(os.path.join(GOLDEN, "update.npz"))
+    z.update({"param_" + n: u["param0_" + n] for n in PARAM_NAMES})
+    return z
 
 
 def load_update_golden():
-    z = np.load(os.path.join(GOLDEN, "update.npz"))
-    return {k: z[k] for k in z.files}
+    """update.npz: the decisions, losses, initial parameters and first gradient; update_steps.npz: the parameters after
+    each of the two Adam steps (param1_*, param2_*)."""
+    return _load_golden("update.npz", "update_steps.npz")
 
 
 def mask_words_to_bool(words):

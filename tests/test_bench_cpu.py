@@ -42,3 +42,34 @@ def test_python_reference_leg_when_the_reference_is_staged():
         pytest.skip("baseline/_ref not staged")
     assert py["kind"] == "reference" and py["cores"] >= 1 and py["games"] > 0 and py["value"] > 100
     assert py["single_core_value"] > 100 and py["unit"] == "env_steps/s" and "cpu_model" in py
+
+
+def test_dump_outputs_types_budget_and_seeded_sample(tmp_path, monkeypatch):
+    """--dump-outputs' writer: integers as float64, floats as float32; over the budget every per-game array keeps the same
+    seeded sample of games (game_index.npy), identical from run to run."""
+    import numpy as np
+    import torch
+    import bench
+    state = torch.arange(17 * 1000, dtype=torch.int32).reshape(17, 1000) - (1 << 31)
+    per_game = {"state": state, "logp": torch.linspace(-1.0, 0.0, 1000)}
+    whole = {"counters": torch.arange(16, dtype=torch.int64)}
+    bench.dump_outputs(str(tmp_path / "full"), per_game, whole)
+    assert sorted(os.listdir(tmp_path / "full")) == ["counters.npy", "logp.npy", "state.npy"]
+    assert np.array_equal(np.load(tmp_path / "full" / "state.npy"), state.numpy().astype(np.float64))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 40000)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), per_game, whole)
+    z = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in ("state", "logp", "counters", "game_index")}
+    assert z["state"].dtype == np.float64 and z["logp"].dtype == np.float32 and z["counters"].dtype == np.float64
+    assert sum(a.nbytes for a in z.values()) <= 40000
+    idx = z["game_index"].astype(np.int64)
+    assert 0 < len(idx) < 1000 and np.array_equal(z["state"], state.numpy()[:, idx].astype(np.float64))
+    assert np.array_equal(z["logp"], per_game["logp"].numpy()[idx])
+    for n in z:
+        assert np.array_equal(z[n], np.load(tmp_path / "b" / (n + ".npy")))
+
+
+def test_dump_outputs_is_refused_for_the_reference_arm():
+    out = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--impl", "reference", "--dump-outputs", "x"],
+                         capture_output=True, text=True, timeout=120, cwd=REPO)
+    assert out.returncode == 2 and "--dump-outputs" in out.stderr

@@ -7,7 +7,7 @@ import pytest
 
 from azul_deep_reinforcement_learning_b200.layout import UnpackedLayout
 from oracle import oracle as O
-from tests.helpers import RUNNER_RULES, RunnerEpisode, load_runner
+from tests.helpers import RUNNER_RULES, RunnerEpisode, load_model_golden, load_runner
 
 
 @pytest.mark.parametrize("rules", RUNNER_RULES)
@@ -71,7 +71,7 @@ def test_oracle_replays_reference_game_runner(rules):
 def test_oracle_observation_matches_reference_get_state():
     """``get_state(perspective=current_player-1)`` as the opponent sees it (game_runner.py:38) and from seat 1:
     the 4,096 decision states of model.npz."""
-    z = np.load("tests/golden/model.npz")
+    z = load_model_golden()
     recs, obs = z["records"].astype(np.int32), z["obs"].astype(np.int32)
     for i in range(recs.shape[0]):
         assert np.array_equal(O.observe(recs[i], 2, -1), obs[i]), i
