@@ -54,8 +54,10 @@ __global__ void __launch_bounds__(256) k_a2c_loss_grad(Args A)
         const uint32_t mw = lane < 6 ? A.mask_rows[row * 6 + lane] : 0u;
         float l[PER_LANE];
         bool legal[PER_LANE];
+        const int act = (int)A.action[row];
         float mx = -INFINITY, sl = 0.0f;
         int k = 0;
+        bool act_legal = false;
 #pragma unroll
         for (int j = 0; j < PER_LANE; j++) {
             const int a = lane + 32 * j;
@@ -64,6 +66,7 @@ __global__ void __launch_bounds__(256) k_a2c_loss_grad(Args A)
             legal[j] = a < ACT && ((w >> b) & 1u);
             l[j] = a < ACT ? lr[a] : 0.0f;
             if (legal[j]) { mx = fmaxf(mx, l[j]); sl += l[j]; k++; }
+            act_legal |= legal[j] && a == act;
         }
         mx = warp_max(mx);
         float se = 0.0f;
@@ -72,10 +75,11 @@ __global__ void __launch_bounds__(256) k_a2c_loss_grad(Args A)
         se = warp_sum(se);
         sl = warp_sum(sl);
         k = (int)warp_sum((float)k);
-        const int act = (int)A.action[row];
         const float v = A.value[row], q = A.qval[row];
         float* dr = A.dlogits + row * ACT;
-        if (k == 0 || act < 0 || act >= ACT) {              // model.py:33-34 IllegalMask: such rows are never recorded
+        // the lane holding the action reports whether it is legal: rows without a legal action or whose action is not
+        // legal (model.py:33-34 IllegalMask: such rows are never recorded) contribute nothing
+        if (!__any_sync(0xFFFFFFFFu, act_legal)) {
 #pragma unroll
             for (int j = 0; j < PER_LANE; j++)
                 if (lane + 32 * j < ACT) dr[lane + 32 * j] = 0.0f;

@@ -275,7 +275,8 @@ __global__ void __launch_bounds__(THREADS, 1) k_update_fwd_bwd(FwdArgs A)
         }
         {
             const int slot = part * TILE_M + row;
-            const bool owns = act >= col0 && act < col0 + PART_COLS;
+            // this part holds the taken action's column AND the action is legal there
+            const bool owns = act >= col0 && act < col0 + PART_COLS && ((mybits >> (act - col0)) & 1ull);
             scr[0 * THREADS + slot] = mx; scr[1 * THREADS + slot] = se; scr[2 * THREADS + slot] = sl;
             scr[3 * THREADS + slot] = value_p;
             scr[4 * THREADS + slot] = __int_as_float(__popcll(mybits) | (owns ? 256 : 0));
@@ -303,8 +304,9 @@ __global__ void __launch_bounds__(THREADS, 1) k_update_fwd_bwd(FwdArgs A)
             const int nf = __float_as_int(scr[4 * THREADS + slot]);
             if ((nf & 255) > 0) gse += scr[1 * THREADS + slot] * __expf(scr[0 * THREADS + slot] - gmx);
         }
-        // rows past the end, rows without a legal action or with an action outside the mask contribute nothing (model.py:33-34)
-        const bool ok = valid && n_valid > 0 && act_seen && act < ACT;
+        // rows past the end and rows whose action is not legal (no legal action at all, action >= 180, or a masked-out
+        // action) contribute nothing (model.py:33-34): act_seen is set only by the part where the action is legal
+        const bool ok = valid && act_seen;
         const float lse = ok ? gmx + __logf(gse) : 0.0f;
         const float log_prob = ok ? la_row - lse : 0.0f;                                   // nn_runner.py:32
         const float inv_k = ok ? 1.0f / (float)n_valid : 0.0f;

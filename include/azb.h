@@ -229,7 +229,10 @@ int azb_train_stats(azb_t* h, const uint32_t* state, const uint32_t* n_dec, int6
  *                           + entropy_coeff * entropy)                   agent.py:47-56 (means: scale = 1/N)
  * Writes dlogits float [n][180] = d loss / d logits, dvalue float [n] = d loss / d value, and ADDS the unscaled sums
  * of the three terms to sums double [3] (optional).  The caller back-propagates (dlogits, dvalue) through the
- * network (torch.autograd.backward) -- the dense layers stay in the caller's framework. */
+ * network (torch.autograd.backward) -- the dense layers stay in the caller's framework.
+ * Excluded decisions (here and in azb_a2c_update_gradients): a decision whose action is not legal in its mask -- no legal
+ * action at all, an action outside [0, 180), or a masked-out action -- contributes nothing: its dlogits row and dvalue
+ * are 0, and it adds nothing to sums or to the parameter gradients. */
 int azb_a2c_loss_grad(azb_t* h, int64_t n, const float* logits, const float* value, const uint32_t* mask_rows,
                       const int64_t* action, const float* qval, float scale, float actor_coeff, float critic_coeff,
                       float entropy_coeff, float* dlogits, float* dvalue, double* sums, void* stream);
@@ -241,8 +244,8 @@ int azb_a2c_loss_grad(azb_t* h, int64_t n, const float* logits, const float* val
  * capacity; no host synchronisation) or n_fixed when n_dec is NULL; `packed` = the current parameters' image
  * (azb_policy_pack_weights).  Forward recomputation (model.py:23-41), masked log-softmax, the three loss terms with the
  * reference's non-detached advantage, and the backward pass through both heads run as tcgen05 GEMMs (fp16 operands, fp32
- * accumulation).  The gradient SUMS over the decisions are ADDED to the eight fp32 buffers in torch layout ([out][in]):
- * grad_w1a [180][136], grad_b1a [180], grad_w2a [180][180], grad_b2a [180], grad_w1c [180][136], grad_b1c [180],
+ * accumulation); decisions are excluded as for azb_a2c_loss_grad.  The gradient SUMS over the decisions are ADDED to
+ * the eight fp32 buffers in torch layout ([out][in]): grad_w1a [180][136], grad_b1a [180], grad_w2a [180][180], grad_b2a [180], grad_w1c [180][136], grad_b1c [180],
  * grad_w2c [180], grad_b2c [1]; sums double [3] += the unscaled actor / critic / entropy loss terms.  workspace: device
  * scratch of azb_update_workspace_bytes(capacity) bytes.  logits_out float [n][180] / value_out float [n] (optional): the
  * recomputed network outputs. */

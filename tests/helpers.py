@@ -1,4 +1,4 @@
-"""Shared helpers for the parity tests (golden-trace access; no game logic)."""
+"""Shared helpers for the parity tests (golden-trace access, the emulated-precision network forward; no game logic)."""
 import hashlib
 import os
 
@@ -145,3 +145,44 @@ def free_port():
     with socket.socket(socket.AF_INET, socket.SOCK_STREAM) as sk:
         sk.bind(("127.0.0.1", 0))
         return sk.getsockname()[1]
+
+
+# ---- the network as the tensor-core kernels evaluate it (azb_policy.cu k_pack_weights, azb_tc.cuh) --------------------
+def f16(x):
+    """Round to fp16 and back (float32)."""
+    import torch
+    return x.to(torch.float16).to(torch.float32)
+
+
+def torch_forward(net, obs, emulate_f16):
+    """ActorCritic on ``obs`` [N, 136] in float64 on the GPU.  With ``emulate_f16`` the operands are rounded where the
+    tensor-core kernels round them: the observation, W1a / W1c / W2a (clamped to +-65504) and the actor's hidden
+    activations to fp16; the biases b1a / b1c / b2a enter as fp16 hi + lo (hi = half(b), lo = half(b - hi)); w2c, b2c and
+    the critic's hidden activations stay unrounded.  Returns a dict of float64 tensors: x, the weights as used (w1a, b1a,
+    w2a, b2a, w1c, b1c, w2c [180], b2c), ha_pre / hc_pre (pre-activations), ha (relu'd, rounded as layer 2 reads it),
+    logits [N, 180] and value [N]."""
+    import torch
+    p = {k: v.detach().cuda().float() for k, v in net.state_dict().items()}
+    w1a, b1a = p["actor_linear1.weight"], p["actor_linear1.bias"]
+    w2a, b2a = p["actor_linear2.weight"], p["actor_linear2.bias"]
+    w1c, b1c = p["critic_linear1.weight"], p["critic_linear1.bias"]
+    x = obs.cuda().float()
+    if emulate_f16:
+        def w16(w):
+            return f16(w.clamp(-65504.0, 65504.0))
+
+        def b16(b):
+            hi = w16(b)
+            return hi.double() + w16(b - hi).double()
+        x, w1a, w2a, w1c = f16(x), w16(w1a), w16(w2a), w16(w1c)
+        b1a, b2a, b1c = b16(b1a), b16(b2a), b16(b1c)
+    o = {"x": x.double(), "w1a": w1a.double(), "b1a": b1a.double(), "w2a": w2a.double(), "b2a": b2a.double(),
+         "w1c": w1c.double(), "b1c": b1c.double(), "w2c": p["critic_linear2.weight"].double().reshape(-1),
+         "b2c": p["critic_linear2.bias"].double().reshape(())}
+    o["ha_pre"] = o["x"] @ o["w1a"].T + o["b1a"]
+    o["hc_pre"] = o["x"] @ o["w1c"].T + o["b1c"]
+    ha = torch.relu(o["ha_pre"])
+    o["ha"] = f16(ha.clamp_max(65504.0).float()).double() if emulate_f16 else ha
+    o["logits"] = o["ha"] @ o["w2a"].T + o["b2a"]
+    o["value"] = torch.relu(o["hc_pre"]) @ o["w2c"] + o["b2c"]
+    return o

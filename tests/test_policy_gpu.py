@@ -29,46 +29,23 @@ def _setup(n=4096, pool=1, seed=7, k=23):
     return net, eng, packed
 
 
-def _f16(x):
-    return x.to(torch.float16).to(torch.float32)
-
-
-def _torch_forward(net, obs, emulate_f16):
-    W1a, b1a = net.actor_linear1.weight.cuda(), net.actor_linear1.bias.cuda()
-    W2a, b2a = net.actor_linear2.weight.cuda(), net.actor_linear2.bias.cuda()
-    W1c, b1c = net.critic_linear1.weight.cuda(), net.critic_linear1.bias.cuda()
-    W2c, b2c = net.critic_linear2.weight.cuda(), net.critic_linear2.bias.cuda()
-    x = obs
-    prev = torch.backends.cuda.matmul.allow_tf32
-    torch.backends.cuda.matmul.allow_tf32 = False
-    try:
-        if emulate_f16:
-            x, W1a, W2a, W1c = _f16(x), _f16(W1a), _f16(W2a), _f16(W1c)
-        ha = torch.relu(x.double() @ W1a.double().T + b1a.double())
-        hc = torch.relu(x.double() @ W1c.double().T + b1c.double())
-        if emulate_f16:
-            ha = _f16(ha.float()).double()
-        logits = ha @ W2a.double().T + b2a.double()
-        value = hc @ W2c.double().T + b2c.double()
-    finally:
-        torch.backends.cuda.matmul.allow_tf32 = prev
-    return logits.float(), value.float().squeeze(1)
-
-
 def test_policy_logits_and_value_match_torch():
     from azul_deep_reinforcement_learning_b200.engine import policy_step
+    from tests.helpers import torch_forward
     with torch.no_grad():
         for pool in (0, 1):
             net, eng, packed = _setup(pool=pool)
             obs = eng.observe(-1)
             out = policy_step(eng, packed, mode=1, apply_step=False, want_logits=True)
             torch.cuda.synchronize()
-            ref_l, ref_v = _torch_forward(net, obs, emulate_f16=True)
+            ref = torch_forward(net, obs, emulate_f16=True)
+            ref_l, ref_v = ref["logits"].float(), ref["value"].float()
             scale = float(ref_l.abs().max())
             err = float((out["logits"] - ref_l).abs().max())
             assert err <= 2e-4 * scale, (err, scale)
             assert float((out["value"] - ref_v).abs().max()) <= 2e-4 * max(1.0, float(ref_v.abs().max()))
-            full_l, full_v = _torch_forward(net, obs, emulate_f16=False)
+            full = torch_forward(net, obs, emulate_f16=False)
+            full_l, full_v = full["logits"].float(), full["value"].float()
             assert float((out["logits"] - full_l).abs().max()) <= 1e-3 * float(full_l.abs().max())
             assert float((out["value"] - full_v).abs().max()) <= 1e-3 * max(1.0, float(full_v.abs().max()))
 

@@ -185,6 +185,141 @@ def test_fused_a2c_loss_gradient_matches_autograd():
     assert float(((sums - ref).abs() / ref.abs().clamp_min(1.0)).max()) < 1e-5
 
 
+def _a2c_reference(logits, value, legal, action, qval, scale, coeffs):
+    """float64 statement of azb_a2c_loss_grad: (dlogits, dvalue, sums); rows whose action is not legal contribute nothing."""
+    ca, cc, ce = coeffs
+    ok = (action >= 0) & (action < 180) & legal.gather(1, action.clamp(0, 179)[:, None]).squeeze(1)
+    l, m = logits.double()[ok], legal[ok]
+    masked = l.masked_fill(~m, float("-inf"))
+    lse = torch.logsumexp(masked, 1)
+    log_prob = l.gather(1, action[ok][:, None]).squeeze(1) - lse
+    k = m.sum(1).double()
+    entropy = -((l * m).sum(1) / k - lse)
+    adv = qval.double()[ok] - value.double()[ok]
+    p = torch.exp(masked - lse[:, None])
+    onehot = torch.nn.functional.one_hot(action[ok], 180).double()
+    dl = torch.zeros(logits.shape, dtype=torch.float64, device=logits.device)
+    dv = torch.zeros(value.shape, dtype=torch.float64, device=logits.device)
+    dl[ok] = scale * torch.where(m, ca * (-adv)[:, None] * (onehot - p) + ce * (p - 1.0 / k[:, None]), 0.0)
+    dv[ok] = scale * (ca * log_prob - 2.0 * cc * adv)
+    return dl, dv, torch.stack([(-log_prob * adv).sum(), (adv * adv).sum(), entropy.sum()]), ok
+
+
+@pytest.mark.parametrize("kind", ["one_legal", "all_legal", "only_150_179", "logits_1e4", "no_legal", "action_-1",
+                                  "action_180", "illegal_action"])
+def test_fused_a2c_loss_grad_edge_rows(kind):
+    """azb_a2c_loss_grad against a float64 reference on synthetic masks: every other row of 128 is of the given kind.
+    A single legal action has log-prob and entropy 0 (its gradient row is exactly zero); all 180 legal and only 150..179
+    legal reach the lanes that hold columns past 180; logits of size 1e4 need the max subtraction; rows whose action
+    is not legal (no legal action, action -1 or 180, an action outside the mask) get zero gradients and stay out of
+    the sums."""
+    from azul_deep_reinforcement_learning_b200.engine import BatchedAzul
+    gen = torch.Generator(device="cuda").manual_seed(5)
+    n, edge = 128, torch.arange(0, 128, 2, device="cuda")
+    logits = torch.randn(n, 180, generator=gen, device="cuda") * 3.0
+    value = torch.randn(n, generator=gen, device="cuda") * 10.0
+    qval = torch.rand(n, generator=gen, device="cuda") * 80.0 - 40.0
+    u = torch.rand(n, 180, generator=gen, device="cuda")
+    legal = u < 0.3
+    legal[:, 7] = True
+    if kind == "one_legal":
+        legal[edge] = False
+        legal[edge, (u[edge, 0] * 180).long()] = True
+    elif kind == "all_legal":
+        legal[edge] = True
+    elif kind == "only_150_179":
+        legal[edge] = False
+        legal[edge, 150:] = True
+    elif kind == "logits_1e4":
+        logits[edge] *= 1e4 / 3.0
+    elif kind == "no_legal":
+        legal[edge] = False
+    action = torch.where(legal, u, -1.0).argmax(1)
+    if kind.startswith("action_"):
+        action[edge] = int(kind[len("action_"):])
+    elif kind == "illegal_action":
+        action[edge] = torch.where(legal, -1.0, u).argmax(1)[edge]
+    words = (legal.view(n, 6, 30).long() << torch.arange(30, device="cuda")).sum(2).to(torch.int32).contiguous()
+    eng = BatchedAzul(1, 2, 0, 0, seed=1)
+    coeffs, scale = (1.0, 0.5, 0.1), 0.5
+    sums = torch.zeros(3, dtype=torch.float64, device="cuda")
+    dl, dv = eng.a2c_loss_grad(logits, value, words, action, qval, scale, coeffs, sums)
+    want_dl, want_dv, want_sums, ok = _a2c_reference(logits, value, legal, action, qval, scale, coeffs)
+    assert int(ok.sum()) == (n if kind in ("one_legal", "all_legal", "only_150_179", "logits_1e4") else n // 2)
+    assert int(torch.count_nonzero(dl[~ok])) == 0 and int(torch.count_nonzero(dv[~ok])) == 0
+    if kind == "one_legal":
+        assert int(torch.count_nonzero(dl[edge])) == 0
+    assert float((dl.double() - want_dl).abs().max()) <= 1e-5 * float(want_dl.abs().max())
+    assert float((dv.double() - want_dv).abs().max()) <= 1e-5 * float(want_dv.abs().max())
+    assert float(((sums - want_sums).abs() / want_sums.abs().clamp_min(1.0)).max()) <= 1e-5, (sums, want_sums)
+
+
+@pytest.mark.parametrize("n", [1000, 256 * 148 + 3])
+def test_train_stats_match_per_game_statistics(n):
+    """azb_train_stats decodes the 2-player packed words itself: its 18 outputs equal the sums of azb_stats and of the
+    exported records, exactly, with some games ended; the decision count is clamped to the record capacity (+1e9 on the
+    unfinished count when it overflowed); the loss and reward sums pass through.  Other player counts are rejected."""
+    from types import SimpleNamespace
+    from azul_deep_reinforcement_learning_b200.engine import BatchedAzul, _ptr, train_stats
+    eng = BatchedAzul(n, 2, 1, 0, seed=n)
+    eng.rollout_random(45)
+    eng.state[3, torch.arange(n, device="cuda") % 7 == 3] |= 1 << 12            # MISC bit 12: end_of_game
+    per_game = eng.stats().long().sum(0).tolist()
+    rec = eng.export_records().cpu().numpy()
+    L = UnpackedLayout(2)
+    wins = int((rec[:, L.score] > rec[:, L.score + 1]).sum())
+    unfinished = int((rec[:, L.end_of_game] == 0).sum())
+    assert 0 < unfinished < n and 0 < wins < n
+    loss = torch.tensor([1.5, -2.25, 3.0], dtype=torch.float64, device="cuda")
+    for n_dec, cap in ((500, 700), (700, 700), (701, 700)):
+        recs = SimpleNamespace(meta=torch.tensor([n_dec, 0], dtype=torch.int32, device="cuda"), cap=cap,
+                               reward_sum=torch.tensor([-17.0], dtype=torch.float64, device="cuda"))
+        out = torch.full((18,), 123.0, dtype=torch.float64, device="cuda")
+        train_stats(eng, recs, loss, out)
+        want = [min(n_dec, cap), 1.5, -2.25, 3.0, -17.0, n] + per_game + [wins, unfinished + (1e9 if n_dec > cap else 0)]
+        assert out.tolist() == want, (n_dec, cap)
+    for players in (3, 4):
+        other = BatchedAzul(64, players, 0, 0, seed=1)
+        assert other.lib.azb_train_stats(other._h, _ptr(other.state), _ptr(recs.meta), 700, _ptr(loss), _ptr(recs.reward_sum),
+                                         _ptr(out), other._stream()) == -1                # AZB_E_INVALID
+
+
+@pytest.mark.parametrize("k", [1, 3, 4, 5, 161])
+def test_discounted_returns_on_synthetic_records(k):
+    """azb_discounted_returns against a float64 loop of nn_runner.py:72-75 cast to float32 (1 ulp: r + gamma * q may be
+    fused) on synthetic records: gaps in the decision flags, decisions without a slot, a walk bounded by the iterations
+    the rollout ran.  Slots never named keep their contents; the reward sum is the exact sum of the walked rewards."""
+    from azul_deep_reinforcement_learning_b200.engine import BatchedAzul, EpisodeRecords, discounted_returns_records
+    n, gamma = 1000, 0.99
+    rng = np.random.default_rng(k)
+    eng = BatchedAzul(n, 2, 0, 0, seed=k, reset=False)
+    recs = EpisodeRecords(eng, k, capacity=k * n)
+    flags = (rng.random((k, n)) < 0.7).astype(np.uint8) | (rng.integers(0, 2, (k, n)) << 1).astype(np.uint8)
+    reward = rng.integers(-40, 41, (k, n)).astype(np.int16)
+    slot = rng.permutation(k * n).reshape(k, n).astype(np.int32)
+    slot[rng.random((k, n)) < 0.1] = -1
+    used = k - k // 3
+    recs.flags_rec.copy_(torch.from_numpy(flags))
+    recs.reward_rec.copy_(torch.from_numpy(reward))
+    recs.slot_rec.copy_(torch.from_numpy(slot))
+    recs.qval.fill_(float("nan"))
+    recs.meta[1] = used
+    discounted_returns_records(eng, recs, gamma)
+    want = np.full(k * n, np.nan, np.float32)
+    q, total = np.zeros(n), 0
+    for t in reversed(range(used)):
+        on = (flags[t] & 1) == 1
+        q = np.where(on, reward[t] + gamma * q, q)
+        total += int(reward[t][on].sum())
+        w = on & (slot[t] >= 0)
+        want[slot[t][w]] = q[w].astype(np.float32)
+    got = recs.qval.cpu().numpy()
+    named = ~np.isnan(want)
+    assert named.sum() > 0 and bool(np.isnan(got[~named]).all())
+    assert bool((np.abs(got[named] - want[named]) <= np.spacing(np.abs(want[named]))).all())
+    assert float(recs.reward_sum) == total
+
+
 def test_training_cli_csv_checkpoint_and_resume(tmp_path):
     """scripts/training.py equivalent (train.py main): writes <net>.csv (one row per batch) and <net>.pt; --resume continues
     the batch numbering, appends to the CSV, restores parameters + Adam state; the checkpoint loads as an opponent Agent."""
