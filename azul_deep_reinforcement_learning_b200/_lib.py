@@ -29,12 +29,11 @@ def load():
     global _lib
     if _lib is not None:
         return _lib
-    path = os.environ.get("AZB_LIB", LIB_PATH)        # tuning sweeps load variant builds of the same library
-    if not os.path.exists(path):
+    if not os.path.exists(LIB_PATH):
         raise AzbError(
             "CUDA library %s is missing: run `python -m azul_deep_reinforcement_learning_b200.build` "
-            "(or __graft_entry__.build()).  There is no CPU fallback." % path)
-    L = ctypes.CDLL(path)
+            "(or __graft_entry__.build()).  There is no CPU fallback." % LIB_PATH)
+    L = ctypes.CDLL(LIB_PATH)
     vp, i32, i64, u64 = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_uint64
     L.azb_abi_version.restype = i32
     L.azb_last_error.restype = ctypes.c_char_p

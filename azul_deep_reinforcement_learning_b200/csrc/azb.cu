@@ -136,33 +136,14 @@ __device__ __forceinline__ void step_finish(const Launch& L, const StepOut& O, G
 // on the aligned path -- written back through the tile with 16-byte global stores, so that a row costs
 // ceil(W/4) + 2 global store instructions instead of W + 6 and every 128-byte line is written whole.
 
+constexpr int STEP_CLAIM = 4;                      // consecutive rows a warp takes from the device-wide counter at a time
+constexpr int STEP_SCHED_WORDS = 16;               // row counter, exit counter
 // games waiting in a warp's queue that trigger a pass: fuller passes cost fewer instructions, earlier passes patch lines that
 // are still in L2 (measured 16 / 20 / 24 / 28 / 32: 201 / 191 / 183 / 186 / 196 us for 4.2 M two-player games)
-// (the AZB_STEP_* macros exist for tuning sweeps: tools/build_variant.py builds variants of the library with -D,
-// tools/sweep_step.sh benches them through AZB_LIB)
-#ifndef AZB_STEP_DRAIN_AT
-#define AZB_STEP_DRAIN_AT 24
-#endif
-#ifndef AZB_STEP_QCAP
-#define AZB_STEP_QCAP 56
-#endif
-#ifndef AZB_STEP_WARPS
-#define AZB_STEP_WARPS 2
-#endif
-#ifndef AZB_STEP_MINBLOCKS
-#define AZB_STEP_MINBLOCKS 8
-#endif
-#ifndef AZB_STEP_STAGES_P2
-#define AZB_STEP_STAGES_P2 4
-#endif
-#ifndef AZB_STEP_CLAIM
-#define AZB_STEP_CLAIM 4
-#endif
-constexpr int STEP_CLAIM = AZB_STEP_CLAIM;         // consecutive rows a warp takes from the device-wide counter at a time
-constexpr int STEP_SCHED_WORDS = 16;               // row counter, exit counter
-constexpr int STEP_DRAIN_AT = AZB_STEP_DRAIN_AT;
-constexpr int STEP_QCAP = AZB_STEP_QCAP;           // a row that would overflow the queue drains it first
-constexpr int STEP_WARPS = AZB_STEP_WARPS;         // warps per block (fine-grained shared-memory occupancy)
+constexpr int STEP_DRAIN_AT = 24;
+constexpr int STEP_QCAP = 56;                      // a row that would overflow the queue drains it first
+constexpr int STEP_WARPS = 2;                      // warps per block (fine-grained shared-memory occupancy)
+constexpr int STEP_MINBLOCKS = 8;
 
 template <int P, int STAGES>
 struct StepSmem {
@@ -184,21 +165,13 @@ __device__ __forceinline__ void cp_async16(uint32_t* smem_dst, const uint32_t* g
 __device__ __forceinline__ uint64_t l2_policy_evict_last()
 {
     uint64_t p;
-#ifdef AZB_STEP_NOHINT          // tuning only
-    asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p));
-#else
     asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-#endif
     return p;
 }
 __device__ __forceinline__ uint64_t l2_policy_evict_first()
 {
     uint64_t p;
-#ifdef AZB_STEP_NOHINT          // tuning only
-    asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p));
-#else
     asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-#endif
     return p;
 }
 __device__ __forceinline__ void cp_async16_hint(uint32_t* smem_dst, const uint32_t* gsrc, uint64_t policy)
@@ -250,7 +223,7 @@ __device__ __forceinline__ void row_flush(const uint32_t* tile, uint32_t* __rest
 }
 
 template <int P, int POOL, int STAGES>
-__global__ void __launch_bounds__(32 * STEP_WARPS, AZB_STEP_MINBLOCKS) k_step(Launch L, const uint8_t* __restrict__ action,
+__global__ void __launch_bounds__(32 * STEP_WARPS, STEP_MINBLOCKS) k_step(Launch L, const uint8_t* __restrict__ action,
                                                            const int8_t* __restrict__ draws, StepOut O, int aligned,
                                                            unsigned int* __restrict__ sched)
 {
@@ -327,13 +300,8 @@ __global__ void __launch_bounds__(32 * STEP_WARPS, AZB_STEP_MINBLOCKS) k_step(La
             }
             bool round_over = false, moved = false;
             uint32_t status = 0;
-#ifdef AZB_STEP_NOCOMPUTE      // tuning only: the memory path of k_step without the rules
-            if (false) {
-                if (gm.ended()) {
-#else
             if (valid && a != AZB_ACTION_SKIP) {
                 if (gm.ended()) {
-#endif
                     status = ST_ENDED;                                        // azul.py:298-299
                 } else {
                     if (!move_if_legal<P, POOL>(gm, a)) {                     // azul.py:301-304
@@ -346,12 +314,6 @@ __global__ void __launch_bounds__(32 * STEP_WARPS, AZB_STEP_MINBLOCKS) k_step(La
                     }
                 }
             }
-#ifdef AZB_STEP_NOCOMPUTE
-            moved = valid;
-#endif
-#ifdef AZB_STEP_NODRAIN        // tuning only: no game enters the queue of finished rounds (results are wrong)
-            round_over = false;
-#endif
             if (fast) {
                 // whole lines through the tile; the lanes whose round ended write their interim state and outputs here
                 // and the final ones in the drain -- later in program order of this warp, ordered by __syncwarp.  (Parking only
@@ -359,11 +321,7 @@ __global__ void __launch_bounds__(32 * STEP_WARPS, AZB_STEP_MINBLOCKS) k_step(La
                 // 0.71 of the HBM peak -- 17 more registers for the loads in flight and an L2 round trip in every pass)
                 const bool any_moved = __any_sync(0xFFFFFFFFu, moved);
                 uint32_t m[6];
-#ifdef AZB_STEP_NOCOMPUTE
-                for (int p = 0; p < 6; p++) m[p] = gm.pl0 + a + p;
-#else
                 legal_mask(gm, m);
-#endif
                 if (!round_over && !gm.ended() && m[0] == 0u /* words 1..5 are subsets of word 0 */ && gm.current_player() != 0u)
                     status |= ST_STUCK;
                 if (any_moved) gm.store(tile, 32, lane);
@@ -403,7 +361,6 @@ __global__ void __launch_bounds__(32 * STEP_WARPS, AZB_STEP_MINBLOCKS) k_step(La
                 Game<P> h;
                 uint32_t gidx, st;
                 queue_get<P, QCAP>(q, waiting - count + lane, h, gidx, st);
-#ifndef AZB_STEP_DRAIN_NOCOMPUTE   // tuning only: the drain's stores without its rules work (results are wrong)
                 count_score<P, POOL>(h);                                      // azul.py:307
                 if (is_end_of_game(h)) {                                      // azul.py:308-309
                     h.misc |= 1u << 12;
@@ -413,10 +370,6 @@ __global__ void __launch_bounds__(32 * STEP_WARPS, AZB_STEP_MINBLOCKS) k_step(La
                 } else {
                     new_round_philox<P, POOL>(h, rng, L.gid0 + gidx, PURPOSE_REFILL);
                 }
-#endif
-#ifdef AZB_STEP_DRAIN_NOSTORE      // tuning only: the drain's rules work without its stores (results are wrong)
-                if (h.steps == 0xFFFFFFF3u)
-#endif
                 step_finish<P, POOL>(L, O, h, (int64_t)gidx, st, true, pol_first);
             }
             waiting -= count;
@@ -428,110 +381,6 @@ __global__ void __launch_bounds__(32 * STEP_WARPS, AZB_STEP_MINBLOCKS) k_step(La
     cp_async_wait<0>();
     if (lane == 0) {
         const unsigned int warps_total = gridDim.x * STEP_WARPS;
-        __threadfence();
-        if (atomicAdd(&sched[1], 1u) == warps_total - 1u) { sched[0] = 0u; sched[1] = 0u; __threadfence(); }
-    }
-}
-
-// ---- k_step_plain: the same step with plain coalesced loads / stores and occupancy instead of staging ----
-// One game per lane, rows claimed from the device-wide counter, every state word read and written with one 128-byte
-// line per warp instruction straight from / to global memory (a streaming kernel of this access pattern reaches 0.93 of
-// the measured HBM peak: tools/microbench/stream.cu; the cp.async tile ring of k_step 0.77 without any rules work).
-// Latency is hidden by resident warps: the register budget is capped so that 32 (2 players) / 24 / 20 warps fit an SM, and
-// shared memory only holds the warp-private queues of finished rounds.
-#ifndef AZB_STEP_PLAIN
-#define AZB_STEP_PLAIN 0
-#endif
-#ifndef AZB_PLAIN_WARPS
-#define AZB_PLAIN_WARPS 4
-#endif
-constexpr int PLAIN_WARPS = AZB_PLAIN_WARPS;
-template <int P> struct PlainCfg { static constexpr int MINBLOCKS = P == 2 ? 32 / PLAIN_WARPS : P == 3 ? 24 / PLAIN_WARPS : 20 / PLAIN_WARPS; };
-
-template <int P, int POOL>
-__global__ void __launch_bounds__(32 * PLAIN_WARPS, PlainCfg<P>::MINBLOCKS) k_step_plain(Launch L, const uint8_t* __restrict__ action,
-                                                                    const int8_t* __restrict__ draws, StepOut O,
-                                                                    unsigned int* __restrict__ sched)
-{
-    constexpr int W = 7 + 5 * P, QCAP = STEP_QCAP;
-    static_assert(QCAP >= STEP_DRAIN_AT - 1 + 32, "a row must fit behind a queue that is just below the drain threshold");
-    extern __shared__ __align__(16) uint32_t step_smem[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint32_t* q = step_smem + (size_t)warp * ((W + 2) * QCAP);
-    const int64_t n_rows = (L.n + 31) / 32;
-    const Philox rng{L.k0, L.k1};
-    int waiting = 0;                                        // warp-uniform: entries in this warp's queue
-    const uint64_t pol_first = l2_policy_evict_first(), pol_last = l2_policy_evict_last();
-    for (;;) {
-        unsigned int claimed = 0;
-        if (lane == 0) claimed = atomicAdd(&sched[0], 1u);
-        const int64_t row = (int64_t)__shfl_sync(0xFFFFFFFFu, claimed, 0);
-        const bool have_row = row < n_rows;
-        if (have_row) {
-            const int64_t g = row * 32 + lane;
-            const bool valid = g < L.n;
-            Game<P> gm;
-            uint32_t a = AZB_ACTION_SKIP;
-            if (valid) {
-                gm.load(L.state, L.n, g);
-                a = action[g];
-            }
-            bool round_over = false, moved = false;
-            uint32_t status = 0;
-#ifdef AZB_STEP_NOCOMPUTE
-            moved = valid; gm.steps += a;
-            if (false) {
-                if (gm.ended()) {
-#else
-            if (valid && a != AZB_ACTION_SKIP) {
-                if (gm.ended()) {
-#endif
-                    status = ST_ENDED;                                        // azul.py:298-299
-                } else if (!move_is_legal(gm, a)) {
-                    status = ST_ILLEGAL;                                      // azul.py:301-302
-                } else {
-                    apply_move<P, POOL>(gm, a);                               // azul.py:304
-                    gm.steps += 1u;
-                    moved = true;
-                    round_over = is_end_of_round(gm);                         // azul.py:306
-                    if (!round_over) next_player(gm);                         // azul.py:313
-                }
-            }
-            // the lanes whose round ended write nothing here: the drain writes their final state and outputs, into lines
-            // that the other lanes' stores (L2 evict_last) keep resident until then
-            if (valid && !round_over) step_finish<P, POOL>(L, O, gm, g, status, moved, pol_last);
-            const uint32_t over = __ballot_sync(0xFFFFFFFFu, round_over);
-            if (over) {                                                       // waiting < STEP_DRAIN_AT here: the row fits
-                if (round_over) queue_put<P, QCAP>(q, waiting + __popc(over & ((1u << lane) - 1u)), gm, (uint32_t)g, status);
-                waiting += __popc(over);
-                __syncwarp();
-            }
-        }
-        if (waiting >= STEP_DRAIN_AT || (!have_row && waiting > 0)) {
-            const int count = waiting < 32 ? waiting : 32;                    // finish `count` games from the tail of the queue
-            if (lane < count) {
-                Game<P> h;
-                uint32_t gidx, st;
-                queue_get<P, QCAP>(q, waiting - count + lane, h, gidx, st);
-                count_score<P, POOL>(h);                                      // azul.py:307
-                if (is_end_of_game(h)) {                                      // azul.py:308-309
-                    h.misc |= 1u << 12;
-                } else if (draws) {                                           // azul.py:311
-                    const int8_t* d = draws + 20 * (int64_t)gidx;
-                    new_round_injected<P, POOL>(h, [&](int k) { return (int)d[k]; });
-                } else {
-                    new_round_philox<P, POOL>(h, rng, L.gid0 + gidx, PURPOSE_REFILL);
-                }
-                step_finish<P, POOL>(L, O, h, (int64_t)gidx, st, true, pol_first);
-            }
-            waiting -= count;
-            __syncwarp();
-        } else if (!have_row) {
-            break;
-        }
-    }
-    if (lane == 0) {
-        const unsigned int warps_total = gridDim.x * PLAIN_WARPS;
         __threadfence();
         if (atomicAdd(&sched[1], 1u) == warps_total - 1u) { sched[0] = 0u; sched[1] = 0u; __threadfence(); }
     }
@@ -609,11 +458,8 @@ struct RoundWords {
     }
 };
 
-#ifndef AZB_ROLLOUT_BOUNDS
-#define AZB_ROLLOUT_BOUNDS
-#endif
 template <int P, int POOL>
-__global__ void AZB_ROLLOUT_BOUNDS k_rollout_random(Launch L, int k_steps, int defer, uint32_t* __restrict__ mask6_out,
+__global__ void k_rollout_random(Launch L, int k_steps, int defer, uint32_t* __restrict__ mask6_out,
                                  unsigned long long* __restrict__ counters)
 {
     extern __shared__ uint32_t round_words[];          // [ROUND_WORDS][blockDim.x]
@@ -972,17 +818,10 @@ template <int P, int POOL>
 static int launch_step(const azb_t* h, const Launch& L, const uint8_t* action, const int8_t* draws, const StepOut& O,
                        int aligned, cudaStream_t stream)
 {
-#if AZB_STEP_PLAIN
-    (void)aligned;
-    auto kern = k_step_plain<P, POOL>;
-    constexpr int WARPS = PLAIN_WARPS;
-    const size_t smem = (size_t)WARPS * (7 + 5 * P + 2) * STEP_QCAP * sizeof(uint32_t);
-#else
-    constexpr int STAGES = P == 2 ? AZB_STEP_STAGES_P2 : 3;       // 2 / 3 / 4 / 5 stages: 183 / 192 / 183 / 198 us for 4.2 M two-player games
+    constexpr int STAGES = P == 2 ? 4 : 3;       // 2 / 3 / 4 / 5 stages: 183 / 192 / 183 / 198 us for 4.2 M two-player games
     auto kern = k_step<P, POOL, STAGES>;
     constexpr int WARPS = STEP_WARPS;
     const size_t smem = StepSmem<P, STAGES>::bytes(STEP_WARPS);
-#endif
     static thread_local int per_sm_cached[64] = {0};      // function attributes are per device
     int uncached = 0;
     int& per_sm = h->device < 64 ? per_sm_cached[h->device] : uncached;
@@ -996,11 +835,7 @@ static int launch_step(const azb_t* h, const Launch& L, const uint8_t* action, c
     int64_t blocks = (rows + WARPS - 1) / WARPS;
     const int64_t resident = (int64_t)h->sm_count * per_sm;
     if (blocks > resident) blocks = resident;
-#if AZB_STEP_PLAIN
-    kern<<<dim3((unsigned)blocks), 32 * WARPS, smem, stream>>>(L, action, draws, O, h->sched);
-#else
     kern<<<dim3((unsigned)blocks), 32 * WARPS, smem, stream>>>(L, action, draws, O, aligned, h->sched);
-#endif
     return 0;
 }
 
@@ -1130,10 +965,7 @@ int azb_rollout_random(azb_t* h, uint32_t* state, int k_steps, uint32_t* mask6_o
             threads = 128;
         }
     }
-#ifndef AZB_ROLLOUT_NO_ROTATE
-#ifndef AZB_ROTATE_PASSES
-#define AZB_ROTATE_PASSES 32      // 1 / 2 / 4 / 8 / 16 / 24 / 32 / 64 / 128 passes per turn: 2.96 / 4.06 / 4.54 / 4.75 / 4.82 / 4.87 / 4.85 / 4.84 / 4.88e10 env steps/s (never: 4.67)
-#endif
+    constexpr int ROTATE_PASSES = 32;      // 1 / 2 / 4 / 8 / 16 / 24 / 32 / 64 / 128 passes per turn: 2.96 / 4.06 / 4.54 / 4.75 / 4.82 / 4.87 / 4.85 / 4.84 / 4.88e10 env steps/s (never: 4.67)
     // one block per SM whose 32-game batches spread 4, 4, 3, 3 (or 3, 3, 2, 2, ...) over the warp schedulers: two warps more than
     // batches, and the batches rotate (k_rollout_rotate)
     if (!h->block_threads_set && h->defer >= 32 && (threads / 32) % 4 == 2 && threads + 64 <= 512 && k_steps > 0 &&
@@ -1143,11 +975,10 @@ int azb_rollout_random(azb_t* h, uint32_t* state, int k_steps, uint32_t* mask6_o
         const dim3 rgrid((unsigned)((h->n_games + threads - 1) / threads));
         DISPATCH_PP(h, AZB_CUDA(cudaFuncSetAttribute(k_rollout_rotate<P, POOL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024)));
         DISPATCH_PP(h, (k_rollout_rotate<P, POOL><<<rgrid, launch_threads, smem, (cudaStream_t)stream>>>(
-                           L, k_steps, h->defer, mask6_out, counters, threads / 32, AZB_ROTATE_PASSES)));
+                           L, k_steps, h->defer, mask6_out, counters, threads / 32, ROTATE_PASSES)));
         CHECK_LAUNCH();
         return 0;
     }
-#endif
     const size_t words_bytes = (size_t)ROUND_WORDS * threads * sizeof(uint32_t);
     if (words_bytes > 48 * 1024) return azb_fail(AZB_E_INVALID, "block threads too large for the rollout kernel's word buffer%s");
     const dim3 grid((unsigned)((h->n_games + threads - 1) / threads));

@@ -43,15 +43,6 @@
 #define AZB_M inline
 #endif
 
-#if defined(__CUDACC__)
-// operands of the multiply-add helpers below ("pipe placement"): values the compiler cannot fold
-static __constant__ uint32_t AZB_ONE = 1u;
-static __constant__ uint32_t AZB_POW2[33] = {
-    1u << 0,  1u << 1,  1u << 2,  1u << 3,  1u << 4,  1u << 5,  1u << 6,  1u << 7,  1u << 8,  1u << 9,  1u << 10,
-    1u << 11, 1u << 12, 1u << 13, 1u << 14, 1u << 15, 1u << 16, 1u << 17, 1u << 18, 1u << 19, 1u << 20, 1u << 21,
-    1u << 22, 1u << 23, 1u << 24, 1u << 25, 1u << 26, 1u << 27, 1u << 28, 1u << 29, 1u << 30, 1u << 31, 0u};
-#endif
-
 namespace azb {
 
 enum : int { POOL_RANDOM = 0, POOL_LID = 1 };
@@ -102,42 +93,6 @@ constexpr uint32_t PLANE_MASK = 0x3FFFFFFFu;
 AZB_HD uint32_t spread5to6(uint32_t x) { return (x * M5) & M6; }
 // stride 6 -> 5 contiguous bits (bit 6c -> bit c)
 AZB_HD uint32_t gather6to5(uint32_t x) { return (((x & M6) * M5) >> 20) & 31u; }
-
-// ---- pipe placement (sm_100a) ------------------------------------------------------------------
-// Bit logic, shifts, selects and compares all issue to ONE half-rate pipe (a warp instruction every 2 cycles per SM
-// sub-partition), integer multiply-adds to another (measured: tools/microbench/pipes.cu); the rules are almost pure
-// bit logic, so the kernels are bound by the first pipe while the second idles.  The helpers below phrase sums,
-// left shifts by a shared amount and constant right shifts as multiply-adds with an operand the compiler cannot see
-// through (a __constant__ word), which keeps them on the multiply-add pipe.  Host builds use the plain operators.
-#ifndef AZB_FORCE_FMA
-#define AZB_FORCE_FMA 0
-#endif
-#ifndef AZB_SELECT_ARITH
-#define AZB_SELECT_ARITH 0
-#endif
-#if defined(__CUDA_ARCH__) && AZB_FORCE_FMA
-// a * b + c on the multiply-add pipe, b a run-time value
-AZB_HD uint32_t fmad(uint32_t a, uint32_t b, uint32_t c)
-{
-    uint32_t d;
-    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
-    return d;
-}
-AZB_HD uint32_t fadd(uint32_t a, uint32_t b) { return fmad(a, AZB_ONE, b); }
-// x >> K for a compile-time K in 1..31: the high word of x * 2^(32-K)
-template <int K>
-AZB_HD uint32_t fshr(uint32_t x)
-{
-    uint32_t lo, hi;
-    asm("{ .reg .b64 t; mul.wide.u32 t, %2, %3; mov.b64 {%0, %1}, t; }" : "=r"(lo), "=r"(hi) : "r"(x), "r"(AZB_POW2[32 - K]));
-    return hi;
-}
-#else
-AZB_HD uint32_t fmad(uint32_t a, uint32_t b, uint32_t c) { return a * b + c; }
-AZB_HD uint32_t fadd(uint32_t a, uint32_t b) { return a + b; }
-template <int K>
-AZB_HD uint32_t fshr(uint32_t x) { return x >> K; }
-#endif
 
 // ---- Philox4x32-10 (Salmon et al. SC'11), the counter-based generator of the draw schedule ----
 struct Philox {
@@ -264,10 +219,10 @@ AZB_HD void legal_mask_open(const Game<P>& g, const uint32_t (&open)[P], uint32_
     const uint32_t o = g.sel(open, g.seat());
     m[0] = src;
     m[1] = src & ((o & M6) * 63u);
-    m[2] = src & ((fshr<1>(o) & M6) * 63u);
-    m[3] = src & ((fshr<2>(o) & M6) * 63u);
-    m[4] = src & ((fshr<3>(o) & M6) * 63u);
-    m[5] = src & ((fshr<4>(o) & M6) * 63u);
+    m[2] = src & (((o >> 1) & M6) * 63u);
+    m[3] = src & (((o >> 2) & M6) * 63u);
+    m[4] = src & (((o >> 3) & M6) * 63u);
+    m[5] = src & (((o >> 4) & M6) * 63u);
 }
 
 // floors[] += n capped at 7 (azul.py:119-123)
@@ -281,9 +236,7 @@ AZB_HD uint32_t floor_add(uint32_t scf, uint32_t n)
 // ---- move (azul.py:118-161); no legality check, like the reference ----
 // p = destination (0 floor, 1..5 pattern line), b = d + 6c = the bit of (source d, colour c) in the planes.
 // Branch-free: a warp holds 32 different games, so "display or centre" and "pattern line or floor" are selects, not
-// branches.  A centre take is the display case with an empty "rest".  Written for the sm_100a integer pipes: bit logic
-// and shifts share one half-rate pipe, multiply-adds run on the other, so sums and left shifts by a common amount are
-// phrased as multiply-adds where that is free.
+// branches.  A centre take is the display case with an empty "rest".
 template <int P, int POOL, bool TRACK>
 AZB_HD void apply_move_core(Game<P>& g, uint32_t p, uint32_t b, uint32_t* open)
 {
@@ -294,7 +247,7 @@ AZB_HD void apply_move_core(Game<P>& g, uint32_t p, uint32_t b, uint32_t* open)
     // the planes moved down by d: bit 6c' = (source d, colour c'); pl3 only has bits at d = 0
     const uint32_t t0 = g.pl0 >> d, t1 = g.pl1 >> d, t2 = g.pl2 >> d, t3 = g.pl3 >> d;
     // tiles taken, still in place: n * cbit
-    const uint32_t n6 = fmad(t3 & cbit, 8u, fmad(t2 & cbit, 4u, fmad(t1 & cbit, 2u, t0 & cbit)));
+    const uint32_t n6 = (t3 & cbit) * 8u + ((t2 & cbit) * 4u + ((t1 & cbit) * 2u + (t0 & cbit)));
     const uint32_t n = n6 >> c6;
     // azul.py:125-133: the chosen colour leaves, the rest of display d joins the centre -- a bit-sliced
     // 4-bit ripple add over all five colours at once.  azul.py:134-138: from the centre only colour c leaves.
@@ -312,30 +265,30 @@ AZB_HD void apply_move_core(Game<P>& g, uint32_t p, uint32_t b, uint32_t* open)
     // azul.py:139-143: the first-player token goes with the first centre take, onto the floor first;
     // next_first_player [11:9] := current_player [8:6]
     const uint32_t t32 = centre ? (g.misc & 32u) : 0u;
-    const uint32_t nf_mask = fmad(t32, 112u, 0u);        // 0xE00 when the token moves
+    const uint32_t nf_mask = t32 * 112u;                  // 0xE00 when the token moves
     const uint32_t misc = g.misc ^ t32;
-    g.misc = (misc & ~nf_mask) | (fmad(misc, 8u, 0u) & nf_mask);
+    g.misc = (misc & ~nf_mask) | ((misc << 3) & nf_mask);
     // azul.py:145-161: fill row p-1 up to its capacity p, the rest (everything when p = 0) falls to the floor
     const bool to_row = p != 0u;
     const uint32_t pat = g.sel(g.pat, s);
-    const uint32_t r = to_row ? p - 1u : 0u, sh = fmad(r, 6u, 0u);
-    const uint32_t cnt = (pat >> fadd(sh, 3u)) & 7u;
-    const uint32_t room = fmad(cnt, 0xFFFFFFFFu, p);     // p - cnt >= 0 when to_row
+    const uint32_t r = to_row ? p - 1u : 0u, sh = 6u * r;
+    const uint32_t cnt = (pat >> (sh + 3u)) & 7u;
+    const uint32_t room = p - cnt;                       // >= 0 when to_row
     const uint32_t placed = to_row ? (n < room ? n : room) : 0u;
-    const uint32_t to_floor = fmad(placed, 0xFFFFFFFFu, n);
+    const uint32_t to_floor = n - placed;
     const uint32_t pw = 1u << sh;
     // to_row: cnt + placed >= 1 (a tile was placed, or the line was already full), so the colour is always written
-    const uint32_t field = fmad(fadd(cnt, placed), 8u, c);
-    const uint32_t newpat = (pat & ~fmad(pw, 63u, 0u)) | fmad(field, pw, 0u);
+    const uint32_t field = (cnt + placed) * 8u + c;
+    const uint32_t newpat = (pat & ~(pw * 63u)) | field * pw;
     g.put(g.pat, s, to_row ? newpat : pat);
     // floors[] += n capped at 7 (azul.py:119-123): both candidates share the score bits, so min() compares the floor fields
     const uint32_t scf = g.sel(g.scf, s);
-    const uint32_t added = fmad(t32, 2048u, fmad(to_floor, 65536u, scf)), capped = scf | (7u << 16);
+    const uint32_t added = t32 * 2048u + (to_floor * 65536u + scf), capped = scf | (7u << 16);
     g.put(g.scf, s, added < capped ? added : capped);
-    if (POOL == POOL_LID) g.lid = fmad(to_floor, cbit, g.lid);       // azul.py:156-157,160-161
+    if (POOL == POOL_LID) g.lid += to_floor * cbit;                  // azul.py:156-157,160-161
     if (TRACK) {                                                      // open rows of the mover: line p-1 now takes only c
         const uint32_t pr = 1u << r;
-        const uint32_t line = fmad(pr, M6, 0u), only = fmad(pr, cbit, 0u);
+        const uint32_t line = pr * M6, only = pr * cbit;
 #pragma unroll
         for (int q = 0; q < P; q++) {
             const uint32_t o = open[q];
@@ -688,28 +641,8 @@ AZB_HD bool move_if_legal(Game<P>& g, uint32_t action)
     return legal;
 }
 
-// position of the k-th (0-based) set bit of a 30-bit word; k < popc(m).  Binary search on the popcount of the low half,
-// with the comparison taken from a sign bit and the three updates written as multiply-adds (see "pipe placement").
-#if AZB_SELECT_ARITH
-AZB_HD uint32_t select_bit(uint32_t m, uint32_t k)
-{
-    uint32_t nk = ~k, pos = 0;                                   // nk = -1 - k: c + nk < 0  <=>  k >= c
-#define AZB_SELECT_LEVEL(MASK, S)                                                          \
-    {                                                                                      \
-        const uint32_t c = (uint32_t)popc(m & (MASK));                                     \
-        const uint32_t ge = fadd(c, nk) >> 31;                  /* 1 when k >= c */          \
-        nk = fmad(c, ge, nk);                                                              \
-        m >>= fmad(ge, (S), 0u);                                                           \
-        pos = fmad(ge, (S), pos);                                                          \
-    }
-    AZB_SELECT_LEVEL(0xFFFFu, 16u)
-    AZB_SELECT_LEVEL(0xFFu, 8u)
-    AZB_SELECT_LEVEL(0xFu, 4u)
-    AZB_SELECT_LEVEL(0x3u, 2u)
-#undef AZB_SELECT_LEVEL
-    return pos + (fadd(m & 1u, nk) >> 31);
-}
-#else
+// position of the k-th (0-based) set bit of a 30-bit word; k < popc(m).  Binary search: at each level, when k is at least
+// the popcount c of the low half, the bit lies in the high half: skip the low half and look for the (k - c)-th bit there.
 AZB_HD uint32_t select_bit(uint32_t m, uint32_t k)
 {
     uint32_t pos = 0, c;
@@ -720,7 +653,6 @@ AZB_HD uint32_t select_bit(uint32_t m, uint32_t k)
     c = m & 1u;                      if (k >= c) { pos += 1; }
     return pos;
 }
-#endif
 
 // The integer random agent (game_runner.py:87-97): legal floor actions (p = 0) weigh 1, every
 // other legal action 100; the point r = mulhi(word, total) walks words 1..5 first, then word 0.

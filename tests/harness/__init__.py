@@ -62,26 +62,6 @@ def random_action(mask6, word):
     return lib().hh_random_action(m.ctypes.data, int(word) & 0xFFFFFFFF)
 
 
-_alt = None
-
-
-def random_action_alt(mask6, word):
-    """The same through a second build of the header with the tuning toggles switched (arithmetic select_bit)."""
-    global _alt
-    if _alt is None:
-        so = os.path.join(_HERE, "_build", "librules_host_alt.so")
-        src = os.path.join(_HERE, "rules_host.cpp")
-        newest = max(os.path.getmtime(src), os.path.getmtime(_HDR))
-        if not os.path.exists(so) or os.path.getmtime(so) < newest:
-            os.makedirs(os.path.dirname(so), exist_ok=True)
-            subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-Wno-unknown-pragmas",
-                                   "-DAZB_SELECT_ARITH=1", "-DAZB_FORCE_FMA=1", "-o", so, src])
-        _alt = ctypes.CDLL(so)
-        _alt.hh_random_action.argtypes = [ctypes.c_void_p, ctypes.c_uint32]
-    m = np.ascontiguousarray(mask6, dtype=np.uint32)
-    return _alt.hh_random_action(m.ctypes.data, int(word) & 0xFFFFFFFF)
-
-
 def opponent(rec, players, pool, seed, gid, require_two=True):
     mask = np.zeros(6, np.uint32)
     diff = np.zeros(1, np.int32)

@@ -59,6 +59,25 @@ def test_create_rejects_bad_rules_and_missing_device(lib):
             BatchedAzul(16)
 
 
+def test_native_source_has_no_compile_time_switches():
+    """The shipped CUDA sources compile one way: preprocessor conditionals only tell the device pass from the host pass
+    and C from C++ (and guard the public header), so no -D flag builds a library that computes something else."""
+    allowed = {"__CUDACC__", "__CUDA_ARCH__", "__cplusplus", "AZB_H"}
+    csrc = os.path.join(REPO, "azul_deep_reinforcement_learning_b200", "csrc")
+    paths = [os.path.join(csrc, f) for f in sorted(os.listdir(csrc))] + [os.path.join(REPO, "include", "azb.h")]
+    found = []
+    for path in paths:
+        if not os.path.isfile(path):
+            continue
+        for no, line in enumerate(open(path), 1):
+            m = re.match(r"\s*#\s*(?:if|ifdef|ifndef|elif)\b(.*)", line)
+            if m:
+                names = set(re.findall(r"[A-Za-z_]\w*", m.group(1).split("//")[0])) - {"defined"}
+                if not names or not names <= allowed:           # `#if 0` switches code off just as well
+                    found.append("%s:%d: %s" % (os.path.relpath(path, REPO), no, line.strip()))
+    assert not found, found
+
+
 def test_product_never_imports_oracle():
     pkg = os.path.join(REPO, "azul_deep_reinforcement_learning_b200")
     for root, _, files in os.walk(pkg):

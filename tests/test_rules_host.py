@@ -111,7 +111,6 @@ def test_packed_random_action_matches_oracle():
         w = int(rng.integers(0, 2 ** 32, dtype=np.uint64))
         a, b = O.random_action(m, w), H.random_action(m, w)
         assert (a == b) or (a == -1 and b == 180)
-        assert H.random_action_alt(m, w) == b          # the arithmetic select_bit (tuning toggle) picks the same bit
 
 
 def test_packed_score_preview_and_predicates():
