@@ -64,6 +64,9 @@ struct PolicyArgs {
     int16_t* __restrict__ reward_rec;        // GameRunner.step reward (game_runner.py:51)
     uint8_t* __restrict__ flags_rec;         // bit 0 a decision was taken, bit 1 game over after it
     uint32_t* __restrict__ steps_used;       // [1] optional: max over CTAs of the decision iterations actually run
+    // ---- runner mode against a frozen policy opponent (azb_policy_rollout_vs_policy, k_policy<..., OPP = true>) ----
+    const unsigned char* __restrict__ opponent_packed;   // the opponent's weight image (seat 2 and seat 1's forced moves)
+    uint32_t* __restrict__ opp_passes;       // [1] optional: max over CTAs and decisions of the opponent passes in one decision
 };
 
 constexpr uint32_t PURPOSE_POLICY = 4;
@@ -157,6 +160,29 @@ __device__ __forceinline__ int32_t opponent_random_warp(Game<2>& h, const Philox
     return (int32_t)(cp.scf[0] & 0xFFFFu) - (int32_t)(cp.scf[1] & 0xFFFFu);
 }
 
+// The loop condition of GameRunner.step (game_runner.py:46) for a game whose round is not pending: the opponent is to move
+// (or seat 1 has a single legal action), the game is not over and has a legal action, and no earlier bound froze it.
+__device__ __forceinline__ bool opponent_to_move(const Game<2>& h)
+{
+    if (h.ended() || (h.status() & ST_STUCK)) return false;
+    uint32_t m[6];
+    legal_mask(h, m);
+    const int n_valid = popc(m[0]) + popc(m[1]) + popc(m[2]) + popc(m[3]) + popc(m[4]) + popc(m[5]);
+    return n_valid > 0 && !(h.current_player() == 1u && n_valid >= 2);
+}
+
+// Thread 0: the fp16 weight image `src` -> shared memory [0, PACKED_BYTES) as chunked bulk async copies completing on bar_w.
+__device__ __forceinline__ void issue_image_copy(unsigned char* smem, const unsigned char* src, uint32_t bar_w)
+{
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_w), "r"((uint32_t)PACKED_BYTES) : "memory");
+    constexpr uint32_t CHUNK = 32768;
+    for (uint32_t off = 0; off < (uint32_t)PACKED_BYTES; off += CHUNK) {
+        const uint32_t bytes = (uint32_t)PACKED_BYTES - off < CHUNK ? (uint32_t)PACKED_BYTES - off : CHUNK;
+        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                     ::"r"(smem_u32(smem) + off), "l"(src + off), "r"(bytes), "r"(bar_w) : "memory");
+    }
+}
+
 // bits [start, start + 48) of the 180-bit linear mask; start is 0, 48, 96 or 144
 __device__ __forceinline__ uint64_t mask_window(const uint32_t (&lin)[6], int start)
 {
@@ -188,7 +214,12 @@ __device__ __forceinline__ RowPart load_part(const float* parts, int slot)
 // FULL: the single-step entry point (azb_policy_step) with its optional diagnostics -- raw logits and the entropy term;
 // the persistent rollouts (azb_policy_rollout) never ask for either, and the sum of the legal logits that the entropy
 // needs is 2 of the 6.5 instructions per logit of the softmax pass (measured: 31 % of that pass).
-template <int POOL, int MODE, bool FULL>
+// OPP: the runner mode against a frozen policy opponent (azb_policy_rollout_vs_policy).  Each decision iteration is a pass of
+// the tile loop with the agent's image resident (act_filter 0, records), then -- with the opponent's image copied over it --
+// passes with act_filter 1 and no records until no game of the CTA is in the opponent's hands, then the runner block, whose
+// random opponent then has nothing to play; the agent's image comes back for the next decision.
+constexpr int MAX_OPP_PASSES = 64;           // the bound of the eager loop (selfplay.py _opponent_policy_moves)
+template <int POOL, int MODE, bool FULL, bool OPP = false>
 __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
 {
     extern __shared__ __align__(128) unsigned char smem[];
@@ -202,6 +233,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
     uint32_t* sample = reinterpret_cast<uint32_t*>(a_tile + OFF_SAMPLE);
     __shared__ unsigned long long cnt[AZB_N_COUNTERS];
     __shared__ uint64_t bar3_storage;                      // layer 1, critic half (bar1: actor half)
+    __shared__ uint32_t n_list;                            // length of the finishing phase's list
     const uint32_t bar3 = smem_u32(&bar3_storage);
     if (tid < AZB_N_COUNTERS) cnt[tid] = 0ull;
     SmemSink sink{cnt};
@@ -222,15 +254,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     asm volatile("griddepcontrol.wait;" ::: "memory");
-    if (tid == 0) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_w), "r"((uint32_t)PACKED_BYTES) : "memory");
-        constexpr uint32_t CHUNK = 32768;
-        for (uint32_t off = 0; off < (uint32_t)PACKED_BYTES; off += CHUNK) {
-            const uint32_t bytes = (uint32_t)PACKED_BYTES - off < CHUNK ? (uint32_t)PACKED_BYTES - off : CHUNK;
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(smem_u32(smem) + off), "l"(A.packed + off), "r"(bytes), "r"(bar_w) : "memory");
-        }
-    }
+    if (tid == 0) issue_image_copy(smem, A.packed, bar_w);
     if (warp == 0) {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(TMEM_COLS) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
@@ -257,8 +281,47 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
     // each of their games; between decisions the packed state stays in global memory (L2-resident: 68 B per game), written and
     // re-read by this CTA only, so block barriers order everything.
     const int64_t my_tiles = (int64_t)blockIdx.x < tiles ? (tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+
+    // ---- the rare, long part of Azul.step for this CTA's own games: the ones flagged by the tile loop (round over / fresh
+    // game) are collected into a dense list (the A region is free then) and finished 32 per warp with every lane busy,
+    // instead of under divergence inside the tile loop or in a second kernel launch.  OPP: `need` collects whether a
+    // finished game is in the opponent's hands in its new round ----
+    auto finish_flagged = [&](uint8_t* __restrict__ done_o, uint8_t* __restrict__ status_o, bool& need) {
+        // the list holds at most FINISH_GROUP tiles' worth of games (every game of a tile can be flagged, e.g. when a whole
+        // batch asks for fresh games), so a CTA with more tiles than that works through them in groups
+        constexpr int FINISH_GROUP = A_BYTES / 4 / TILE_M / PARTS * PARTS;         // 96 tiles = 12,288 entries
+        static_assert(FINISH_GROUP >= PARTS && FINISH_GROUP * TILE_M * 4 <= A_BYTES, "finish list exceeds the A region");
+        uint32_t* list = reinterpret_cast<uint32_t*>(a_tile);
+        for (int64_t j0 = 0; j0 < my_tiles; j0 += FINISH_GROUP) {
+            if (tid == 0) n_list = 0u;
+            __syncthreads();
+            const int64_t j1 = j0 + FINISH_GROUP < my_tiles ? j0 + FINISH_GROUP : my_tiles;
+            for (int64_t j = j0 + part; j < j1; j += PARTS) {
+                const int64_t g = ((int64_t)blockIdx.x + j * gridDim.x) * TILE_M + row;
+                if (g < A.n && (A.state[3 * A.n + g] & (FLAG_ROUND_OVER | FLAG_FRESH_GAME))) list[atomicAdd(&n_list, 1u)] = (uint32_t)g;
+            }
+            __syncthreads();
+            const uint32_t total = n_list;
+            for (uint32_t i = (uint32_t)tid; i < total; i += THREADS) {
+                const uint32_t gidx = list[i];
+                Game<2> h;
+                h.load(A.state, A.n, (int64_t)gidx);
+                const uint32_t flags = h.misc & (FLAG_ROUND_OVER | FLAG_FRESH_GAME);
+                h.misc &= ~(FLAG_ROUND_OVER | FLAG_FRESH_GAME);
+                finish_game<POOL>(h, gidx, flags, rng, A.gid0, A.first_rule, A.apply_step == 2, A.state, A.n, done_o, status_o, sink);
+                if (OPP) need |= opponent_to_move(h);
+            }
+            __syncthreads();                           // the list is reused by the next group
+        }
+    };
+
     int it = 0;
+    uint32_t w_phase = 0u, max_opp = 0u;               // OPP: parity of bar_w's next completion; most opponent passes
+    bool w_pending = true, opp_image = false;          // OPP: an image copy to wait for; the opponent's image is resident
     for (; it < A.k_decisions; it++) {
+    for (int pass = 0;; pass++) {                      // OPP: pass 0 takes the agent's decisions, passes >= 1 the opponent's
+    const bool record = !OPP || pass == 0;             // decision records and per-game outputs: the agent's pass only
+    bool need = false;                                 // OPP: a game this thread moved is (still) in the opponent's hands
     // software pipeline over tiles: the next tile's state is loaded during this tile's epilogues and its observation
     // is built by parts 1..3 while part 0 plays this tile's moves
     // (the next tile's state is held as the 17 RAW words: Game::load unpacks the MISC word on the spot, and that first use
@@ -275,7 +338,10 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
         first.load(nraw, 1, 0);
         build_obs_tile(first, a_tile, row, part);
     }
-    if (it == 0) mbar_wait(bar_w, 0);                     // weights and vectors have landed (every thread reads the vectors)
+    if (OPP ? w_pending : it == 0) {                       // weights and vectors have landed (every thread reads the vectors)
+        mbar_wait(bar_w, OPP ? w_phase : 0u);
+        if (OPP) { w_phase ^= 1u; w_pending = false; }
+    }
     for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
         const int64_t g = tile * TILE_M + row;
         const bool valid = g < A.n;
@@ -543,9 +609,12 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
             const float entropy = n_valid > 0 ? -(gsl / (float)n_valid - lse) : 0.0f;
             uint32_t status = n_valid > 0 ? 0u : (gm.ended() ? (uint32_t)ST_ENDED : (uint32_t)ST_STUCK);
             const bool agent_turn = gm.current_player() == 1u && n_valid >= 2;
-            const bool acts = A.act_filter == 0 || (A.act_filter == 1 ? !agent_turn : agent_turn);
+            // OPP: the agent's pass decides every game (act_filter 0), the opponent's passes the games outside seat 1's turn
+            // (act_filter 1); a game frozen at the opponent-pass bound (ST_STUCK in its state) takes no move from either network
+            const bool acts = OPP ? !(gm.status() & ST_STUCK) && (pass == 0 || !agent_turn)
+                                  : A.act_filter == 0 || (A.act_filter == 1 ? !agent_turn : agent_turn);
             if (!acts) { n_valid = 0; status = 0u; }      // filtered out: reported as AZB_ACTION_SKIP, state untouched
-            if (valid) {
+            if (valid && record) {
                 if (A.mask6_out) {
 #pragma unroll
                     for (int p = 0; p < 6; p++) A.mask6_out[p * A.n + g] = m[p];
@@ -555,7 +624,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
                 if (A.logp_out) A.logp_out[g] = logp;
                 if (FULL && A.entropy_out) A.entropy_out[g] = entropy;
             }
-            if (A.runner_mode) {
+            if (A.runner_mode && record) {
                 // NNRunner.run_episode's per-decision record (nn_runner.py:27-45) in compact form: the warp's deciding games take
                 // consecutive slots (one atomic per warp); the packed state the decision was taken on is what the update
                 // kernel rebuilds observation and mask from
@@ -588,7 +657,10 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
                 apply_move<2, POOL>(gm, action);                          // azul.py:304
                 gm.steps += 1u;
                 if (is_end_of_round(gm)) flags = FLAG_ROUND_OVER;         // azul.py:306 -> finishing phase
-                else next_player(gm);                                     // azul.py:313
+                else {
+                    next_player(gm);                                      // azul.py:313
+                    if (OPP) need |= valid && opponent_to_move(gm);
+                }
                 stepped = valid && A.apply_step == 2;
             } else if (A.apply_step == 2 && acts && (ended_before || stuck)) {
                 flags = FLAG_FRESH_GAME;                                  // GameRunner.reset, game_runner.py:76-80
@@ -600,7 +672,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
             }
             gm.misc |= flags;
             if (valid && A.apply_step) gm.store(A.state, A.n, g);
-            if (valid) {
+            if (valid && record) {
                 if (A.done_out) A.done_out[g] = ended_before ? 1 : 0;      // finalised by the finishing phase for flagged games
                 if (A.status_out) A.status_out[g] = (uint8_t)(status | gm.status());
             }
@@ -627,16 +699,44 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
         // all TMEM reads and scratch reads of this tile are complete before the next tile overwrites them
         if (!issuer) asm volatile("bar.sync 2, %0;" ::"n"(THREADS) : "memory");
     }
+    if (!OPP) break;
+    // ---- OPP: finish the rounds this pass ended (the opponent network must see the new round, as after
+    // azb_policy_step(apply_step = 1)), then vote: is any game of this CTA still in the opponent's hands? ----
+    __syncthreads();                                   // every state / done / status write of the tile loop is visible to the CTA
+    finish_flagged(record ? A.done_out : nullptr, record ? A.status_out : nullptr, need);
+    const bool more = __syncthreads_or(need ? 1 : 0) != 0;
+    if (pass > 0 && (uint32_t)pass > max_opp) max_opp = (uint32_t)pass;
+    if (!more) break;
+    if (pass == MAX_OPP_PASSES) {
+        // only a bug gets here (a round is at most 20 takes long): freeze the games the opponent still holds -- ST_STUCK
+        // ends their episode for the alive vote and azb_train_stats, and no later pass moves them
+        for (int64_t j = part; j < my_tiles; j += PARTS) {
+            const int64_t g = ((int64_t)blockIdx.x + j * gridDim.x) * TILE_M + row;
+            if (g >= A.n) continue;
+            Game<2> h;
+            h.load(A.state, A.n, g);
+            if (opponent_to_move(h)) { h.add_status(ST_STUCK); h.store(A.state, A.n, g); }
+        }
+        break;
+    }
+    if (pass == 0) {
+        // swap in the opponent's image: the barrier above closed every generic read of the agent's image (the critic vector),
+        // and every MMA that read it was waited for at bar1 / bar2 / bar3.  The next pass builds its first observation tile
+        // while the copy runs and waits for it before its first layer-1 issue.
+        if (tid == 0) { fence_async_smem(); issue_image_copy(smem, A.opponent_packed, bar_w); }
+        w_pending = opp_image = true;
+    }
+    }   // passes
 
-    // ---- the rare, long part of Azul.step for this CTA's own games: the ones flagged above (round over / fresh game) are
-    // collected into a dense list (the A region is free now) and finished 32 per warp with every lane busy, instead of under
-    // divergence inside the tile loop or in a second kernel launch ----
+    // ---- the rare, long part of Azul.step, or the runner mode's closing of the decision ----
     __syncthreads();                                   // every state / done / status write of the tile loop is visible to the CTA
     bool any_alive = true;
     if (A.runner_mode) {
         // GameRunner.step after the agent's move (game_runner.py:46-55), one thread per game of this CTA's tiles: finish the
         // round the move may have ended, let the random opponent play until seat 1 is to move with >= 2 legal actions (or the
-        // game is over), take the reward from a score preview, and close the decision's record
+        // game is over), take the reward from a score preview, and close the decision's record.  OPP: the policy opponent's
+        // passes already restored that invariant, so the random opponent plays no move (as the eager path's trailing
+        // azb_opponent_random(require_two = 1))
         bool alive = false;
         // (spreading a tile's 128 games over all 16 warps, 8 lanes each, was measured slower: 1.07 vs 0.97 ms per rollout of
         // 16,384 episodes -- the state loads lose their coalescing and every warp still walks the union of its games' paths)
@@ -652,7 +752,10 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
             const bool pending = (h.misc & FLAG_ROUND_OVER) != 0u;
             if (decided) h.misc &= ~(FLAG_ROUND_OVER | FLAG_FRESH_GAME);
             uint32_t m2[6];
-            const int32_t diff = opponent_random_warp<POOL>(h, rng, gid, decided, pending, m2);
+            // OPP: a game frozen at the pass bound gets no random move either (its mask is reported empty)
+            const bool frozen = OPP && (h.status() & ST_STUCK) != 0u;
+            if (frozen) for (int p = 0; p < 6; p++) m2[p] = 0u;
+            const int32_t diff = opponent_random_warp<POOL>(h, rng, gid, decided && !frozen, pending, m2);
             if (!decided) continue;
             h.store(A.state, A.n, g);
             const int32_t before = (int32_t)A.player_score[g];
@@ -670,36 +773,20 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
         }
         any_alive = __syncthreads_or(alive ? 1 : 0) != 0;
     } else if (A.apply_step) {
-        // the list holds at most FINISH_GROUP tiles' worth of games (every game of a tile can be flagged, e.g. when a whole
-        // batch asks for fresh games), so a CTA with more tiles than that works through them in groups
-        constexpr int FINISH_GROUP = A_BYTES / 4 / TILE_M / PARTS * PARTS;         // 96 tiles = 12,288 entries
-        static_assert(FINISH_GROUP >= PARTS && FINISH_GROUP * TILE_M * 4 <= A_BYTES, "finish list exceeds the A region");
-        uint32_t* list = reinterpret_cast<uint32_t*>(a_tile);
-        __shared__ uint32_t n_list;
-        for (int64_t j0 = 0; j0 < my_tiles; j0 += FINISH_GROUP) {
-            if (tid == 0) n_list = 0u;
-            __syncthreads();
-            const int64_t j1 = j0 + FINISH_GROUP < my_tiles ? j0 + FINISH_GROUP : my_tiles;
-            for (int64_t j = j0 + part; j < j1; j += PARTS) {
-                const int64_t g = ((int64_t)blockIdx.x + j * gridDim.x) * TILE_M + row;
-                if (g < A.n && (A.state[3 * A.n + g] & (FLAG_ROUND_OVER | FLAG_FRESH_GAME))) list[atomicAdd(&n_list, 1u)] = (uint32_t)g;
-            }
-            __syncthreads();
-            const uint32_t total = n_list;
-            for (uint32_t i = (uint32_t)tid; i < total; i += THREADS) {
-                const uint32_t gidx = list[i];
-                Game<2> h;
-                h.load(A.state, A.n, (int64_t)gidx);
-                const uint32_t flags = h.misc & (FLAG_ROUND_OVER | FLAG_FRESH_GAME);
-                h.misc &= ~(FLAG_ROUND_OVER | FLAG_FRESH_GAME);
-                finish_game<POOL>(h, gidx, flags, rng, A.gid0, A.first_rule, A.apply_step == 2, A.state, A.n, A.done_out, A.status_out, sink);
-            }
-            __syncthreads();                           // the list is reused by the next group
-        }
+        bool unused = false;
+        finish_flagged(A.done_out, A.status_out, unused);
     }
     __syncthreads();                                   // the next decision reads the states written above
+    if (OPP && opp_image && any_alive && it + 1 < A.k_decisions) {
+        // swap the agent's image back for the next decision (the barrier above closed every read of the opponent's; no
+        // copy is left in flight when the CTA exits)
+        if (tid == 0) { fence_async_smem(); issue_image_copy(smem, A.packed, bar_w); }
+        w_pending = true;
+        opp_image = false;
+    }
     if (!any_alive) { it++; break; }                   // runner mode: every episode of this CTA is over
     }   // decision loop
+    if (OPP && A.opp_passes && tid == 0) atomicMax(A.opp_passes, max_opp);
     if (A.steps_used && tid == 0) atomicMax(A.steps_used, (uint32_t)it);
     __syncthreads();
     if (A.counters && tid < AZB_N_COUNTERS && cnt[tid]) atomicAdd(&A.counters[tid], cnt[tid]);
@@ -750,17 +837,17 @@ __global__ void k_pack_weights(const float* __restrict__ w1a, const float* __res
     }
 }
 
-template <int POOL, int MODE, bool FULL>
+template <int POOL, int MODE, bool FULL, bool OPP = false>
 static int launch_policy(const PolicyArgs& A, int grid, cudaStream_t stream)
 {
-    AZB_CUDA(cudaFuncSetAttribute(k_policy<POOL, MODE, FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    AZB_CUDA(cudaFuncSetAttribute(k_policy<POOL, MODE, FULL, OPP>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;       // see griddepcontrol in k_policy
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    AZB_CUDA(cudaLaunchKernelEx(&cfg, k_policy<POOL, MODE, FULL>, A));
+    AZB_CUDA(cudaLaunchKernelEx(&cfg, k_policy<POOL, MODE, FULL, OPP>, A));
     return 0;
 }
 
@@ -802,7 +889,7 @@ int azb_policy_step(azb_t* h, uint32_t* state, const void* packed, int mode, int
     A.entropy_out = entropy_out; A.done_out = done_out; A.status_out = status_out; A.mask6_out = mask6_out;
     A.k_decisions = 1; A.runner_mode = 0; A.player_score = nullptr; A.n_dec = nullptr; A.rec_cap = 0; A.state_rec = nullptr;
     A.action_rec = nullptr; A.logp_rec = nullptr; A.value_rec = nullptr; A.slot_rec = nullptr; A.reward_rec = nullptr;
-    A.flags_rec = nullptr; A.steps_used = nullptr;
+    A.flags_rec = nullptr; A.steps_used = nullptr; A.opponent_packed = nullptr; A.opp_passes = nullptr;
     const int64_t tiles = (h->n_games + pol::TILE_M - 1) / pol::TILE_M;
     const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
     int rc = 0;
@@ -836,11 +923,46 @@ int azb_policy_rollout(azb_t* h, uint32_t* state, const void* packed, int mode, 
     A.k_decisions = k_decisions; A.runner_mode = runner_mode; A.player_score = player_score; A.n_dec = n_dec; A.rec_cap = rec_cap;
     A.state_rec = state_rec; A.action_rec = action_rec; A.logp_rec = logp_rec; A.value_rec = value_rec; A.slot_rec = slot_rec;
     A.reward_rec = reward_rec; A.flags_rec = flags_rec; A.steps_used = steps_used;
+    A.opponent_packed = nullptr; A.opp_passes = nullptr;
     const int64_t tiles = (h->n_games + pol::TILE_M - 1) / pol::TILE_M;
     const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
     int rc = 0;
     if (h->tile_pool == AZB_POOL_LID) rc = mode == 0 ? pol::launch_policy<1, 0, false>(A, grid, (cudaStream_t)stream) : pol::launch_policy<1, 1, false>(A, grid, (cudaStream_t)stream);
     else rc = mode == 0 ? pol::launch_policy<0, 0, false>(A, grid, (cudaStream_t)stream) : pol::launch_policy<0, 1, false>(A, grid, (cudaStream_t)stream);
+    if (rc) return rc;
+    CHECK_LAUNCH();
+    return 0;
+}
+
+int azb_policy_rollout_vs_policy(azb_t* h, uint32_t* state, const void* packed, const void* opponent_packed, int mode,
+                                 int k_decisions, int16_t* player_score, uint32_t* n_dec, int64_t rec_cap,
+                                 uint32_t* state_rec, uint8_t* action_rec, float* logp_rec, float* value_rec,
+                                 int32_t* slot_rec, int16_t* reward_rec, uint8_t* flags_rec, uint32_t* steps_used,
+                                 uint32_t* opp_passes, uint32_t* mask6_out, uint8_t* done_out, uint8_t* status_out,
+                                 void* stream)
+{
+    CHECK_HANDLE(h);
+    if (!state || !packed || !opponent_packed) return azb_fail(AZB_E_INVALID, "null buffer%s");
+    if (h->players != 2) return azb_fail(AZB_E_INVALID, "the policy network is defined for 2 players (136 inputs, agent.py:29)%s");
+    if (mode != 0 && mode != 1) return azb_fail(AZB_E_INVALID, "mode must be 0 (sample) or 1 (argmax)%s");
+    if (k_decisions < 1) return azb_fail(AZB_E_INVALID, "k_decisions must be >= 1%s");
+    if (!player_score || !n_dec || rec_cap < 1 || !state_rec || !action_rec || !slot_rec || !reward_rec || !flags_rec)
+        return azb_fail(AZB_E_INVALID, "runner mode needs player_score, n_dec, rec_cap and the state / action / slot / reward / flags records%s");
+    pol::PolicyArgs A;
+    A.state_in = state; A.state = state; A.n = h->n_games; A.packed = (const unsigned char*)packed;
+    A.k0 = (uint32_t)h->seed; A.k1 = (uint32_t)(h->seed >> 32); A.gid0 = (uint32_t)h->game_id_base;
+    A.mode = mode; A.apply_step = 1; A.first_rule = h->first_player; A.counters = nullptr; A.act_filter = 0;
+    A.logits_out = nullptr; A.value_out = nullptr; A.action_out = nullptr; A.logp_out = nullptr; A.entropy_out = nullptr;
+    A.done_out = done_out; A.status_out = status_out; A.mask6_out = mask6_out;
+    A.k_decisions = k_decisions; A.runner_mode = 1; A.player_score = player_score; A.n_dec = n_dec; A.rec_cap = rec_cap;
+    A.state_rec = state_rec; A.action_rec = action_rec; A.logp_rec = logp_rec; A.value_rec = value_rec; A.slot_rec = slot_rec;
+    A.reward_rec = reward_rec; A.flags_rec = flags_rec; A.steps_used = steps_used;
+    A.opponent_packed = (const unsigned char*)opponent_packed; A.opp_passes = opp_passes;
+    const int64_t tiles = (h->n_games + pol::TILE_M - 1) / pol::TILE_M;
+    const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
+    int rc = 0;
+    if (h->tile_pool == AZB_POOL_LID) rc = mode == 0 ? pol::launch_policy<1, 0, false, true>(A, grid, (cudaStream_t)stream) : pol::launch_policy<1, 1, false, true>(A, grid, (cudaStream_t)stream);
+    else rc = mode == 0 ? pol::launch_policy<0, 0, false, true>(A, grid, (cudaStream_t)stream) : pol::launch_policy<0, 1, false, true>(A, grid, (cudaStream_t)stream);
     if (rc) return rc;
     CHECK_LAUNCH();
     return 0;

@@ -435,11 +435,23 @@ class EpisodeRecords:
         self.reward_sum.zero_()
 
 
-def runner_rollout(engine, packed, records, player_score, mode=0, out=None):
+def runner_rollout(engine, packed, records, player_score, mode=0, out=None, opponent=None, opp_passes=None):
     """``NNRunner.run_episode`` for every game slot in ONE launch (``azb_policy_rollout``, runner mode): agent decisions by the
     fused policy kernel, opponent loop + reward after each, decision records into ``records``.  The episodes must have
-    been started (``BatchedGameRunner.reset``)."""
+    been started (``BatchedGameRunner.reset``, or :meth:`selfplay.PersistentEpisodes.start` against a policy opponent).
+
+    ``opponent``: None plays the random opponent; a :class:`PackedPolicy` plays a frozen network with the same ``mode``
+    (``azb_policy_rollout_vs_policy``).  ``opp_passes`` (uint32 / int32 [1], optional, zeroed by the caller) then receives
+    the most opponent passes one decision needed."""
     r = records
+    if opponent is not None:
+        _lib.check(engine.lib.azb_policy_rollout_vs_policy(
+            engine._h, _ptr(engine.state), _ptr(packed.buf), _ptr(opponent.buf), int(mode), r.k, _ptr(player_score),
+            _ptr(r.meta), r.cap, _ptr(r.state_rec), _ptr(r.action_rec), _ptr(r.logp_rec), _ptr(r.value_rec), _ptr(r.slot_rec),
+            _ptr(r.reward_rec), _ptr(r.flags_rec), ctypes.c_void_p(r.meta.data_ptr() + 4), _ptr(opp_passes),
+            _ptr(out["mask"]) if out else None, _ptr(out["done"]) if out else None, _ptr(out["status"]) if out else None,
+            engine._stream()))
+        return
     _lib.check(engine.lib.azb_policy_rollout(
         engine._h, _ptr(engine.state), _ptr(packed.buf), int(mode), r.k, 1, _ptr(player_score), _ptr(r.meta), r.cap,
         _ptr(r.state_rec), _ptr(r.action_rec), _ptr(r.logp_rec), _ptr(r.value_rec), _ptr(r.slot_rec), _ptr(r.reward_rec),

@@ -6,6 +6,8 @@ from the Philox schedule).  One agent decision costs three launches: observation
 when the caller records it), the fused policy kernel (``azb_policy_step``: MLP on tcgen05 + masked
 softmax + sampling + the agent's ``Azul.step``) and the opponent loop + reward (``azb_opponent_random``).
 """
+import os
+
 import torch
 
 from .engine import (BatchedAzul, EpisodeRecords, discounted_returns_records, mask_to_bool, policy_step, rules_to_ints,
@@ -222,14 +224,17 @@ class GraphedEpisodes:
 
 
 class PersistentEpisodes:
-    """``NNRunner.run_episode`` for every game slot with the whole episode loop on the device: ``GameRunner.reset`` (two
-    launches), then ONE persistent launch of the fused policy kernel that takes every agent decision, plays the random
-    opponent's moves, takes the rewards and writes the decision records, then the discounted returns (one launch).  The
-    recorded decisions are those of :func:`run_episodes` (same Philox schedule); only their storage differs (compact
-    slots in arbitrary order instead of [T, G])."""
+    """``NNRunner.run_episode`` for every game slot with the whole episode loop on the device: ``GameRunner.reset`` (a few
+    launches), then ONE persistent launch of the fused policy kernel that takes every agent decision, plays the opponent's
+    moves, takes the rewards and writes the decision records, then the discounted returns (one launch).  The recorded
+    decisions are those of :func:`run_episodes` (same Philox schedule); only their storage differs (compact slots in
+    arbitrary order instead of [T, G]).
+
+    The opponent is the runner's: the random agent (``runner.opponent`` None) or a frozen network (a ``PackedPolicy``,
+    ``GameRunner(opponent=Agent(...))``), which then plays with the same selection mode as the agent.  Nothing in
+    :meth:`run` waits for the GPU, so a whole batch can be captured in a CUDA graph."""
 
     def __init__(self, runner, packed, max_decisions=160, capacity=None, want_logp_value=False):
-        assert runner.opponent is None, "the persistent rollout plays the RandomAgent opponent"
         self.runner, self.packed = runner, packed
         n = runner.n_games
         if capacity is None:                       # ~30 decisions per episode on average; small batches get the full K x G
@@ -238,15 +243,56 @@ class PersistentEpisodes:
         self.out = {"mask": torch.zeros((6, n), dtype=torch.int32, device=runner.device),
                     "done": torch.zeros(n, dtype=torch.uint8, device=runner.device),
                     "status": torch.zeros(n, dtype=torch.uint8, device=runner.device)}
+        # policy opponent: the most opponent passes one decision of the last run needed
+        self.opp_passes = torch.zeros(1, dtype=torch.int32, device=runner.device)
+
+    def start(self, mode=0):
+        """``GameRunner.reset`` (game_runner.py:76-85) for every slot.  Against a policy opponent without the host reads of
+        ``BatchedGameRunner.reset``: on a fresh board the opponent moves at most once before seat 1 is to move with >= 2
+        legal actions, so ONE opponent launch replaces its loop; the resulting state is the same."""
+        runner = self.runner
+        if runner.opponent is None:
+            return runner.reset()
+        e = runner.engine
+        e.reset()
+        runner.player_score.zero_()
+        policy_step(e, runner.opponent, mode=mode, apply_step=True, want_mask=False, act_filter=1)
+        out = e.opponent_random(runner.player_score, require_two=False, want_obs=runner.record_obs)
+        runner.player_score.zero_()                  # game_runner.py:81: the score baseline restarts at 0
+        runner.mask, runner.obs = out["mask"], out.get("obs")
+        return out
 
     def run(self, gamma=0.99, mode=0):
+        opponent = self.runner.opponent
+        if opponent is not None and self.runner.opponent_mode != mode:
+            raise ValueError("the persistent rollout plays both seats with one selection mode: agent mode %d, opponent mode %d"
+                             % (mode, self.runner.opponent_mode))
         r = self.records
-        self.runner.reset()
+        self.start(mode)
         r.clear()
-        runner_rollout(self.runner.engine, self.packed, r, self.runner.player_score, mode=mode, out=self.out)
+        if opponent is not None:
+            self.opp_passes.zero_()
+        runner_rollout(self.runner.engine, self.packed, r, self.runner.player_score, mode=mode, out=self.out,
+                       opponent=opponent, opp_passes=self.opp_passes if opponent is not None else None)
         discounted_returns_records(self.runner.engine, r, gamma)
         self.runner.mask = self.out["mask"]
         return r
+
+
+def load_network(net, device=None):
+    """An ``ActorCritic`` from a module, a ``state_dict``, a trainer checkpoint dict (``{"ac_net": ...}``) or a file path (every
+    format ``Agent(base_net_file=...)`` accepts, through ``azulnet.agent.load_ac_net``)."""
+    from .azulnet.agent import load_ac_net
+    from .azulnet.model import ActorCritic
+    if isinstance(net, (str, os.PathLike)):
+        net = load_ac_net(os.fspath(net))
+    elif isinstance(net, dict):
+        sd = net["ac_net"] if "ac_net" in net else net
+        net = ActorCritic(136, 180)
+        net.load_state_dict(sd)
+    elif not isinstance(net, torch.nn.Module):
+        raise TypeError("expected an ActorCritic, a state_dict or a file path, got %r" % type(net).__name__)
+    return net.to(device) if device is not None else net
 
 
 def discounted_returns(reward, active, gamma):

@@ -2,6 +2,7 @@
 equivalent (reference scripts/training.py:8-22, nn_runner.py:53-84, agent.py:39-62).
 
     python -m azul_deep_reinforcement_learning_b200.train [batch_size] [net_name] [--batches N]
+                                                      [--opponent FILE] [--opponent-refresh N]
     torchrun --nproc-per-node 8 -m azul_deep_reinforcement_learning_b200.train 1024 run1
 
 ``batch_size`` episodes are played IN PARALLEL per rank (one game slot each) instead of one after the
@@ -24,7 +25,8 @@ import torch.distributed as dist
 from . import parallel
 from .azulnet.model import ActorCritic
 from .engine import PackedPolicy, UpdateGradients, train_stats
-from .selfplay import BatchedGameRunner, GraphedEpisodes, PersistentEpisodes, discounted_returns, run_episodes
+from .selfplay import (BatchedGameRunner, GraphedEpisodes, PersistentEpisodes, discounted_returns, load_network,
+                       run_episodes)
 
 ACTOR_COEFF, CRITIC_COEFF, ENTROPY_COEFF = 1.0, 0.5, 0.1          # agent.py:47-49
 
@@ -118,16 +120,40 @@ def global_count(n_local, device):
 STAT_FIELDS = 18        # n_decisions, 3 loss sums, reward sum, games, 10 game statistics sums, wins, unfinished
 
 
+def summarize_stats(s, update_sync_s=None):
+    """The STAT_FIELDS sums (``azb_train_stats`` order) -> the per-batch numbers: mean losses per decision, and per game the
+    reward and the ``GameStatistics`` fields (agent.py:12, game_runner.py:10-22)."""
+    n_global, games = max(s[0], 1.0), s[5]
+    out = {"transitions": s[0], "games": games, "actor_loss": s[1] / n_global, "critic_loss": s[2] / n_global,
+           "entropy_loss": s[3] / n_global, "reward": s[4] / games}
+    if update_sync_s is not None:
+        out["update_sync_s"] = update_sync_s
+    out["ac_loss"] = ACTOR_COEFF * out["actor_loss"] + CRITIC_COEFF * out["critic_loss"] + ENTROPY_COEFF * out["entropy_loss"]
+    g = [x / games for x in s[6:16]]
+    out.update(player_score=g[0], opponent_score=g[1], rounds=g[2],
+               percent_first_player=100.0 * s[9] / max(s[10], 1.0), floor_penalty=g[5], max_combo=g[6],
+               completed_rows=g[7], completed_columns=g[8], completed_colors=g[9])
+    out["win_percent"] = s[16] / games
+    out["unfinished"] = int(s[17])
+    return out
+
+
 class SelfPlayTrainer:
     """``NNRunner.train`` (nn_runner.py:53-84) with ``games_per_rank`` episodes played in parallel per rank.
 
     ``rollout``: "persistent" (default; whole episodes in one launch of the fused policy kernel), "graph" (CUDA-graph
     replay of one policy + one opponent launch per decision) or "eager".  ``update``: "tensor" (default with the persistent
     rollout: ``azb_a2c_update_gradients``, hand-written tcgen05 forward / backward on the decision records) or "autograd"
-    (PyTorch autograd over cuBLAS GEMMs, TF32 or -- ``tf32_update=False`` -- fp32: the reference path of the tests)."""
+    (PyTorch autograd over cuBLAS GEMMs, TF32 or -- ``tf32_update=False`` -- fp32: the reference path of the tests).
+
+    ``opponent``: None plays the random agent (``RandomAgent``); an ``ActorCritic``, a ``state_dict`` or a file path
+    (anything ``Agent(base_net_file=...)`` loads) plays a frozen network in seat 2 (``GameRunner(opponent=Agent(...))``),
+    sampling like the agent.  ``opponent_refresh`` = N > 0: the opponent's weights are replaced by the current network's
+    after every N batches -- self-play against a lagged copy of itself."""
 
     def __init__(self, games_per_rank=1024, learning_rate=3e-4, gamma=0.99, seed=0, device=0, rank=0, world=1,
-                 rules=None, max_decisions=160, use_cuda_graph=True, tf32_update=True, rollout=None, update=None):
+                 rules=None, max_decisions=160, use_cuda_graph=True, tf32_update=True, rollout=None, update=None,
+                 opponent=None, opponent_refresh=0):
         self.rank, self.world, self.gamma, self.max_decisions = rank, world, gamma, max_decisions
         self.tf32_update = tf32_update
         self.device = torch.device("cuda", device)
@@ -139,6 +165,15 @@ class SelfPlayTrainer:
                                         game_id_base=parallel.shard(rank, games_per_rank), record_obs=True)
         self.packed = PackedPolicy(self.runner.engine, self.net)
         self.rollout_kind = rollout if rollout is not None else ("persistent" if use_cuda_graph else "eager")
+        self.opponent, self.opponent_refresh, self.batches_done = None, int(opponent_refresh), 0
+        if opponent_refresh and opponent is None:
+            opponent = self.net                              # a lagged copy of the network itself
+        if opponent is not None:
+            if self.rollout_kind == "graph":
+                raise ValueError("the graph rollout plays the random opponent only; use the persistent or eager rollout")
+            # packed once into its own fixed buffer: a captured batch reads it there, a refresh re-packs it in place
+            self.opponent = PackedPolicy(self.runner.engine, load_network(opponent, self.device))
+            self.runner.opponent, self.runner.opponent_mode = self.opponent, 0
         self.graphed = self.episodes = None
         if self.rollout_kind == "persistent":
             self.runner.record_obs = False
@@ -251,6 +286,7 @@ class SelfPlayTrainer:
         assert self.rollout_kind == "persistent" and self.update_kind == "tensor"
         for _ in range(warmup):
             self.update(self.rollout())
+            self._batch_done()
         torch.cuda.synchronize(self.device)
         self._graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self._graph):
@@ -262,8 +298,19 @@ class SelfPlayTrainer:
         if getattr(self, "_graph", None) is not None:
             self._graph.replay()
             self._push_stats(self._graph_stats)
+            self._batch_done()
             return None if defer_stats else self.fetch_stats()
-        return self.update(self.rollout(), defer_stats)
+        out = self.update(self.rollout(), defer_stats)
+        self._batch_done()
+        return out
+
+    def _batch_done(self):
+        """Every ``opponent_refresh`` batches the opponent's image is re-packed from the current network: one launch of its
+        own, outside a captured batch, into the buffer that batch reads -- the next replay plays against the new weights."""
+        self.batches_done += 1
+        if self.opponent is not None and self.opponent_refresh > 0 and self.batches_done % self.opponent_refresh == 0:
+            with torch.no_grad():
+                self.opponent.update(self.net)
 
     def _update_device(self, batch):
         """``Agent.update`` (agent.py:39-62) on every recorded agent decision of the batch; returns the device statistics.
@@ -312,17 +359,7 @@ class SelfPlayTrainer:
         s = self._host_stats[slot].tolist()
         if s[17] >= 1e9:
             raise RuntimeError("decision records overflowed their capacity (raise max_decisions / capacity)")
-        n_global, games = max(s[0], 1.0), s[5]
-        out = {"transitions": s[0], "games": games, "actor_loss": s[1] / n_global, "critic_loss": s[2] / n_global,
-               "entropy_loss": s[3] / n_global, "reward": s[4] / games, "update_sync_s": time.perf_counter() - t0}
-        out["ac_loss"] = ACTOR_COEFF * out["actor_loss"] + CRITIC_COEFF * out["critic_loss"] + ENTROPY_COEFF * out["entropy_loss"]
-        g = [x / games for x in s[6:16]]
-        out.update(player_score=g[0], opponent_score=g[1], rounds=g[2],
-                   percent_first_player=100.0 * s[9] / max(s[10], 1.0), floor_penalty=g[5], max_combo=g[6],
-                   completed_rows=g[7], completed_columns=g[8], completed_colors=g[9])
-        out["win_percent"] = s[16] / games
-        out["unfinished"] = int(s[17])
-        return out
+        return summarize_stats(s, update_sync_s=time.perf_counter() - t0)
 
     def save_checkpoint(self, path, batch):
         """``<net_name>.pt``: network ``state_dict`` (parameter names of model.py:17-21, loadable by
@@ -392,7 +429,7 @@ class SelfPlayTrainer:
         return self.history
 
 
-def main(argv=None):
+def parse_args(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.split("\n\n")[0])
     ap.add_argument("batch_size", nargs="?", type=int, default=10, help="episodes per batch and rank (scripts/training.py:8-11)")
     ap.add_argument("net_name", nargs="?", default=None, help="write <net_name>.csv / .pt (scripts/training.py:12-15)")
@@ -403,12 +440,26 @@ def main(argv=None):
                     help="continue from a checkpoint written by this script (<net_name>.pt) or start from any saved "
                          "network Agent(base_net_file=...) accepts")
     ap.add_argument("--checkpoint-every", type=int, default=1000)
+    ap.add_argument("--opponent", default=None, metavar="FILE",
+                    help="play seat 2 with this frozen network (any file Agent(base_net_file=...) accepts) instead of "
+                         "the random agent")
+    ap.add_argument("--opponent-refresh", type=int, default=0, metavar="N",
+                    help="replace the opponent by the current network after every N batches (self-play against a lagged "
+                         "copy; without --opponent it starts as the initial network)")
     args = ap.parse_args(argv)
+    if args.opponent_refresh < 0:
+        ap.error("--opponent-refresh must be >= 0")
+    return args
+
+
+def main(argv=None):
+    args = parse_args(argv)
     rank, world, local = parallel.world()
     if world > 1:
         parallel.init("nccl", local)
     torch.cuda.set_device(local)
-    tr = SelfPlayTrainer(args.batch_size, learning_rate=args.lr, seed=args.seed, device=local, rank=rank, world=world)
+    tr = SelfPlayTrainer(args.batch_size, learning_rate=args.lr, seed=args.seed, device=local, rank=rank, world=world,
+                         opponent=args.opponent, opponent_refresh=args.opponent_refresh)
     start = tr.load_checkpoint(args.resume) if args.resume else 0
     tr.train(batches=args.batches, net_name=args.net_name, start_batch=start, checkpoint_every=args.checkpoint_every)
     if world > 1:

@@ -203,6 +203,27 @@ int azb_policy_rollout(azb_t* h, uint32_t* state, const void* packed, int mode, 
                        uint32_t* steps_used, uint8_t* action_out, float* logp_out, float* value_out, uint32_t* mask6_out,
                        uint8_t* done_out, uint8_t* status_out, unsigned long long* counters, void* stream);
 
+/* ---- K4, persistent runner mode against a frozen policy opponent: GameRunner(opponent=Agent(base_net_file=...))
+ * (game_runner.py:26-30, scripts/run_batch.py) for one episode per slot in ONE launch.  As azb_policy_rollout's runner mode
+ * (same records, outputs and checks), but seat 2 -- and seat 1 when it has a single legal action -- is played by the
+ * network in `opponent_packed` (azb_policy_pack_weights image; may be `packed` itself) with the same `mode` as the agent:
+ * after each agent decision the opponent takes one move per game that is in its hands, pass after pass, until seat 1 is
+ * to move with >= 2 legal actions or the game is over; then the reward.  The decisions equal those of azb_policy_step
+ * (act_filter 0 for the agent, then act_filter 1 with the opponent's image until no game acts) followed by
+ * azb_opponent_random(require_two = 1): the sampling word depends only on the game and its step count.
+ * The caller starts the episodes with azb_reset, then ONE azb_policy_step(opponent_packed, the same mode, apply_step = 1,
+ * act_filter = 1) -- on a fresh board the opponent moves at most once before seat 1 is to move with >= 2 legal actions --
+ * then azb_opponent_random(require_two = 0), and zeroes player_score; no host synchronisation is needed.
+ * opp_passes uint32 [1] (optional, zeroed by the caller): the most opponent passes one decision needed (max over CTAs and
+ * decisions).  At most 64 passes are run per decision; a game still in the opponent's hands then (only a bug can cause
+ * it) gets AZB_ST_STUCK, takes no further move and counts as unfinished. */
+int azb_policy_rollout_vs_policy(azb_t* h, uint32_t* state, const void* packed, const void* opponent_packed, int mode,
+                                 int k_decisions, int16_t* player_score, uint32_t* n_dec, int64_t rec_cap,
+                                 uint32_t* state_rec, uint8_t* action_rec, float* logp_rec, float* value_rec,
+                                 int32_t* slot_rec, int16_t* reward_rec, uint8_t* flags_rec, uint32_t* steps_used,
+                                 uint32_t* opp_passes, uint32_t* mask6_out, uint8_t* done_out, uint8_t* status_out,
+                                 void* stream);
+
 /* Discounted returns of NNRunner.train (nn_runner.py:72-75) over the records of azb_policy_rollout's runner mode:
  * q_t = r_t + gamma * q_{t+1} over each game's decisions (accumulated in double like the reference's numpy loop), written
  * as float to qval[slot] (float [rec_cap]); reward_sum (double [1], optional) += the sum of all rewards; steps_used
