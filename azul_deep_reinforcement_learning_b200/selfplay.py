@@ -2,9 +2,12 @@
 
 ``BatchedGameRunner`` is G copies of the reference's 2-player env wrapper advancing in lock-step on one
 GPU: seat 1 is the learning agent, seat 2 a random agent (``RandomAgent``, game_runner.py:87-97, drawing
-from the Philox schedule).  One agent decision costs three launches: observation (``azb_observe``, only
-when the caller records it), the fused policy kernel (``azb_policy_step``: MLP on tcgen05 + masked
-softmax + sampling + the agent's ``Azul.step``) and the opponent loop + reward (``azb_opponent_random``).
+from the Philox schedule) or a frozen network.  ``PersistentEpisodes`` plays whole episodes in one launch of
+the fused policy kernel; that is how the trainer plays.  ``run_episodes`` is the step-wise loop the persistent
+kernel is checked against: one agent decision costs up to three launches, the observation
+(``azb_observe_bf16``, only when the caller records it), the fused policy kernel (``azb_policy_step``: MLP on
+tcgen05 + masked softmax + sampling + the agent's ``Azul.step``) and the opponent loop + reward
+(``azb_opponent_random``).
 """
 import os
 
@@ -17,13 +20,10 @@ DEFAULT_RULES = {"first_player": "Random", "tile_pool": "Lid"}      # game_runne
 
 
 class BatchedGameRunner:
-    def __init__(self, n_games, rules=None, seed=0, device=0, game_id_base=0, opponent=None, opponent_mode=0,
-                 record_obs=False):
+    def __init__(self, n_games, rules=None, seed=0, device=0, game_id_base=0, opponent=None, opponent_mode=0):
         """``opponent``: None = RandomAgent (game_runner.py:29-30) or a ``PackedPolicy`` = a frozen ``Agent``
-        (scripts/run_batch.py:6-8) whose moves come from the fused policy kernel.  ``record_obs``: the opponent /
-        reward kernel also writes the next decision's observation (``self.obs``, bfloat16 [G, 136])."""
-        self.opponent, self.opponent_mode, self.record_obs = opponent, opponent_mode, record_obs
-        self.obs = None
+        (scripts/run_batch.py:6-8) whose moves come from the fused policy kernel."""
+        self.opponent, self.opponent_mode = opponent, opponent_mode
         rules = DEFAULT_RULES if rules is None else rules
         pool, first = rules_to_ints(2, rules)
         self.engine = BatchedAzul(n_games, 2, pool, first, seed=seed, device=device, game_id_base=game_id_base, reset=False)
@@ -38,9 +38,9 @@ class BatchedGameRunner:
         self.player_score.zero_()
         if self.opponent is not None:                 # a fresh board always offers seat 1 >= 2 actions, so the
             self._opponent_policy_moves()             # ":46" and ":84" loop conditions coincide here
-        out = self.engine.opponent_random(self.player_score, require_two=False, want_obs=self.record_obs)
+        out = self.engine.opponent_random(self.player_score, require_two=False)
         self.player_score.zero_()                     # game_runner.py:81: the score baseline restarts at 0
-        self.mask, self.obs = out["mask"], out.get("obs")
+        self.mask = out["mask"]
         return out
 
     def get_state(self):
@@ -67,8 +67,8 @@ class BatchedGameRunner:
     def _after_agent_move(self):
         if self.opponent is not None:
             self._opponent_policy_moves()
-        out = self.engine.opponent_random(self.player_score, require_two=True, want_obs=self.record_obs)
-        self.mask, self.obs = out["mask"], out.get("obs")
+        out = self.engine.opponent_random(self.player_score, require_two=True)
+        self.mask = out["mask"]
         return out
 
     def step(self, actions):
@@ -94,8 +94,8 @@ RAW_KEYS = ("obs", "mask", "reward", "value", "logp", "entropy", "action", "stat
 def _one_decision(runner, packed, rec, record_obs):
     """One agent decision for every game; appends the raw outputs of the kernels (what ``NNRunner.run_episode``
     records, nn_runner.py:27-45) without any per-decision bookkeeping -- see :func:`_alive_chain`."""
-    if record_obs:                           # the previous opponent / reward launch already wrote it when asked to
-        rec["obs"].append(runner.obs if runner.obs is not None else runner.engine.observe_bf16(0))
+    if record_obs:
+        rec["obs"].append(runner.engine.observe_bf16(0))
     rec["mask"].append(runner.mask)          # every opponent_random call returns a new tensor: no copy needed
     out = runner.step_policy(packed)
     rec["reward"].append(out["reward"])
@@ -156,73 +156,6 @@ def run_episodes(runner, packed, max_decisions=160, check_every=8, record_obs=Tr
     return _finish_batch(chunks, alive)
 
 
-class GraphedEpisodes:
-    """``run_episodes`` with its launch-bound inner loop captured in CUDA graphs.
-
-    One agent decision is five small kernels (observation record, policy, round finisher, opponent loop + reward,
-    and nothing else: the bookkeeping is vectorised over the decisions afterwards); the loop is bound by launch
-    latency, not by the GPU.  The first ``decisions`` decisions of an episode batch (reset included) are recorded
-    into one CUDA graph, and a second graph holds ``more`` further decisions; batches in which some game is still
-    running replay the second graph until all are done (its outputs are copied out after every replay).  Results
-    are identical to :func:`run_episodes`."""
-
-    def __init__(self, runner, packed, decisions=48, record_obs=True, more=8):
-        self.runner, self.packed, self.decisions, self.record_obs, self.more = runner, packed, decisions, record_obs, more
-        dev = runner.device
-        # warm-up on a side stream (lazy CUDA initialisation must not happen during capture)
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):
-            runner.reset()
-            self._body(2)
-        torch.cuda.current_stream(dev).wait_stream(side)
-        torch.cuda.synchronize(dev)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            runner.reset()
-            self.rec = self._body(decisions)
-            self.mask_out, self.obs_out = runner.mask, runner.obs
-        # continuation: starts from the engine's current state and the legal mask / observation in self.mask_in / self.obs_in (copied in before a
-        # replay: a graph reads fixed addresses)
-        self.mask_in = torch.zeros_like(self.mask_out)
-        self.obs_in = None if self.obs_out is None else torch.zeros_like(self.obs_out)
-        self.graph_more = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph_more, pool=self.graph.pool()):
-            runner.mask, runner.obs = self.mask_in, self.obs_in
-            self.rec_more = self._body(more)
-            self.mask_more, self.obs_more = runner.mask, runner.obs
-        # the first replay of a graph pays its upload (tens of ms): pay it here, not in the middle of training
-        # (every run() starts with the reset inside the first graph, so the games played here are discarded)
-        self.graph.replay()
-        self.graph_more.replay()
-        torch.cuda.synchronize(dev)
-
-    def _body(self, decisions):
-        rec = {k: [] for k in RAW_KEYS}
-        for _ in range(decisions):
-            _one_decision(self.runner, self.packed, rec, self.record_obs)
-        return {k: torch.stack(v) for k, v in rec.items() if v}
-
-    def run(self, max_decisions=160, check_every=8):
-        G, dev = self.runner.n_games, self.runner.device
-        self.graph.replay()
-        chunk = dict(self.rec)
-        chunk["active"], alive = _alive_chain(chunk["status"], chunk["done"], torch.ones(G, dtype=torch.bool, device=dev))
-        chunks, mask, obs, t = [chunk], self.mask_out, self.obs_out, self.decisions
-        while t < max_decisions and bool(alive.any()):
-            self.mask_in.copy_(mask)
-            if obs is not None:
-                self.obs_in.copy_(obs)
-            self.graph_more.replay()
-            chunk = {k: v.clone() for k, v in self.rec_more.items()}
-            chunk["active"], alive = _alive_chain(chunk["status"], chunk["done"], alive)
-            chunks.append(chunk)
-            mask, obs = self.mask_more, self.obs_more
-            t += self.more
-        self.runner.mask, self.runner.obs = mask, obs
-        return _finish_batch(chunks, alive)
-
-
 class PersistentEpisodes:
     """``NNRunner.run_episode`` for every game slot with the whole episode loop on the device: ``GameRunner.reset`` (a few
     launches), then ONE persistent launch of the fused policy kernel that takes every agent decision, plays the opponent's
@@ -257,9 +190,9 @@ class PersistentEpisodes:
         e.reset()
         runner.player_score.zero_()
         policy_step(e, runner.opponent, mode=mode, apply_step=True, want_mask=False, act_filter=1)
-        out = e.opponent_random(runner.player_score, require_two=False, want_obs=runner.record_obs)
+        out = e.opponent_random(runner.player_score, require_two=False)
         runner.player_score.zero_()                  # game_runner.py:81: the score baseline restarts at 0
-        runner.mask, runner.obs = out["mask"], out.get("obs")
+        runner.mask = out["mask"]
         return out
 
     def run(self, gamma=0.99, mode=0):

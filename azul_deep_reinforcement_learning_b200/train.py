@@ -25,8 +25,7 @@ import torch.distributed as dist
 from . import parallel
 from .azulnet.model import ActorCritic
 from .engine import PackedPolicy, UpdateGradients, train_stats
-from .selfplay import (BatchedGameRunner, GraphedEpisodes, PersistentEpisodes, discounted_returns, load_network,
-                       run_episodes)
+from .selfplay import BatchedGameRunner, PersistentEpisodes, load_network
 
 ACTOR_COEFF, CRITIC_COEFF, ENTROPY_COEFF = 1.0, 0.5, 0.1          # agent.py:47-49
 
@@ -71,36 +70,6 @@ def network_outputs(net, x):
     return logits, value.squeeze(1)
 
 
-def allreduce_gradients(params):
-    """C1: one flat all-reduce (sum) over every gradient; the caller already divided by the global count."""
-    if not (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
-        return
-    flat = torch.cat([p.grad.reshape(-1) for p in params])
-    dist.all_reduce(flat, op=dist.ReduceOp.SUM)
-    off = 0
-    for p in params:
-        n = p.numel()
-        p.grad.copy_(flat[off:off + n].view_as(p.grad))
-        off += n
-
-
-def allreduce_gradients_and_stats(params, stats):
-    """C1 + C2: every gradient (sums over the local decisions, not yet divided by a count) as ONE flat fp32 all-reduce
-    (82,081 values = 328 KB) and the statistics vector as a second, tiny float64 one; returns the reduced statistics.
-    No host synchronisation."""
-    stats = stats.double().reshape(-1).clone()
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        flat = torch.cat([p.grad.reshape(-1) for p in params])
-        dist.all_reduce(flat, op=dist.ReduceOp.SUM)
-        dist.all_reduce(stats, op=dist.ReduceOp.SUM)
-        off = 0
-        for p in params:
-            n = p.numel()
-            p.grad.copy_(flat[off:off + n].view_as(p.grad))
-            off += n
-    return stats
-
-
 def allreduce_flat_and_stats(flat, stats):
     """What the trainer does per update, in place: C1 = ONE fp32 all-reduce of the flat gradient buffer (82,081 sums), C2 =
     one float64 all-reduce of the statistics vector.  No-op for a single process."""
@@ -108,13 +77,6 @@ def allreduce_flat_and_stats(flat, stats):
         dist.all_reduce(flat, op=dist.ReduceOp.SUM)
         dist.all_reduce(stats, op=dist.ReduceOp.SUM)
     return flat, stats
-
-
-def global_count(n_local, device):
-    t = torch.tensor([float(n_local)], dtype=torch.float64, device=device)
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        dist.all_reduce(t, op=dist.ReduceOp.SUM)
-    return float(t.item())
 
 
 STAT_FIELDS = 18        # n_decisions, 3 loss sums, reward sum, games, 10 game statistics sums, wins, unfinished
@@ -141,10 +103,12 @@ def summarize_stats(s, update_sync_s=None):
 class SelfPlayTrainer:
     """``NNRunner.train`` (nn_runner.py:53-84) with ``games_per_rank`` episodes played in parallel per rank.
 
-    ``rollout``: "persistent" (default; whole episodes in one launch of the fused policy kernel), "graph" (CUDA-graph
-    replay of one policy + one opponent launch per decision) or "eager".  ``update``: "tensor" (default with the persistent
-    rollout: ``azb_a2c_update_gradients``, hand-written tcgen05 forward / backward on the decision records) or "autograd"
-    (PyTorch autograd over cuBLAS GEMMs, TF32 or -- ``tf32_update=False`` -- fp32: the reference path of the tests).
+    :meth:`rollout` plays the whole batch in one launch of the persistent fused policy kernel (``PersistentEpisodes``) and
+    returns its compact decision records; :meth:`update` runs ``Agent.update`` on them with ``azb_a2c_update_gradients``
+    (hand-written tcgen05 forward / backward).  :meth:`enable_step_graph` captures both as one CUDA graph.
+    :meth:`update_decisions` (PyTorch autograd over cuBLAS GEMMs, TF32 or -- ``tf32_update=False`` -- fp32) and
+    :meth:`update_states` (the tensor-core kernels) run one ``Agent.update`` on explicitly given decisions: the entry points
+    the tests hold against the reference.
 
     ``opponent``: None plays the random agent (``RandomAgent``); an ``ActorCritic``, a ``state_dict`` or a file path
     (anything ``Agent(base_net_file=...)`` loads) plays a frozen network in seat 2 (``GameRunner(opponent=Agent(...))``),
@@ -152,9 +116,8 @@ class SelfPlayTrainer:
     after every N batches -- self-play against a lagged copy of itself."""
 
     def __init__(self, games_per_rank=1024, learning_rate=3e-4, gamma=0.99, seed=0, device=0, rank=0, world=1,
-                 rules=None, max_decisions=160, use_cuda_graph=True, tf32_update=True, rollout=None, update=None,
-                 opponent=None, opponent_refresh=0):
-        self.rank, self.world, self.gamma, self.max_decisions = rank, world, gamma, max_decisions
+                 rules=None, max_decisions=160, tf32_update=True, opponent=None, opponent_refresh=0):
+        self.rank, self.world, self.gamma = rank, world, gamma
         self.tf32_update = tf32_update
         self.device = torch.device("cuda", device)
         torch.manual_seed(seed)                              # identical initial weights on every rank
@@ -162,30 +125,19 @@ class SelfPlayTrainer:
         self.params = list(self.net.parameters())
         self.opt = torch.optim.Adam(self.params, lr=learning_rate, fused=True, capturable=True)   # agent.py:37 (one fused kernel; graph-capturable)
         self.runner = BatchedGameRunner(games_per_rank, rules=rules, seed=seed, device=device,
-                                        game_id_base=parallel.shard(rank, games_per_rank), record_obs=True)
+                                        game_id_base=parallel.shard(rank, games_per_rank))
         self.packed = PackedPolicy(self.runner.engine, self.net)
-        self.rollout_kind = rollout if rollout is not None else ("persistent" if use_cuda_graph else "eager")
         self.opponent, self.opponent_refresh, self.batches_done = None, int(opponent_refresh), 0
         if opponent_refresh and opponent is None:
             opponent = self.net                              # a lagged copy of the network itself
         if opponent is not None:
-            if self.rollout_kind == "graph":
-                raise ValueError("the graph rollout plays the random opponent only; use the persistent or eager rollout")
             # packed once into its own fixed buffer: a captured batch reads it there, a refresh re-packs it in place
             self.opponent = PackedPolicy(self.runner.engine, load_network(opponent, self.device))
             self.runner.opponent, self.runner.opponent_mode = self.opponent, 0
-        self.graphed = self.episodes = None
-        if self.rollout_kind == "persistent":
-            self.runner.record_obs = False
-            self.episodes = PersistentEpisodes(self.runner, self.packed, max_decisions=max_decisions)
-        elif self.rollout_kind == "graph":
-            self.graphed = GraphedEpisodes(self.runner, self.packed)
-        self.update_kind = update if update is not None else ("tensor" if self.rollout_kind == "persistent" else "autograd")
-        assert self.update_kind in ("tensor", "autograd")
+        self.episodes = PersistentEpisodes(self.runner, self.packed, max_decisions=max_decisions)
         # every parameter gradient is a view into ONE flat fp32 buffer (PARAM_ORDER): the tensor-core kernels add into
         # it, autograd accumulates into the views in place, and the gradient all-reduce is a single collective on it
-        cap = self.episodes.records.cap if self.episodes is not None else 128
-        self.tc = UpdateGradients(self.runner.engine, cap)
+        self.tc = UpdateGradients(self.runner.engine, self.episodes.records.cap)
         for name, p in self.net.named_parameters():
             p.grad = self.tc.grads[name]
         self._host_stats = torch.zeros((2, STAT_FIELDS), dtype=torch.float64).pin_memory()
@@ -196,17 +148,11 @@ class SelfPlayTrainer:
 
     # ---- rollout ---------------------------------------------------------------------------
     def rollout(self):
+        """Every game slot plays one episode; returns the ``EpisodeRecords`` of the agent's decisions with their discounted
+        returns."""
         with torch.no_grad():
             self.packed.update(self.net)
-            if self.episodes is not None:
-                return {"records": self.episodes.run(self.gamma)}
-            if self.graphed is not None:
-                batch = self.graphed.run(max_decisions=self.max_decisions)
-            else:
-                batch = run_episodes(self.runner, self.packed, max_decisions=self.max_decisions)
-            batch["qval"] = discounted_returns(batch["reward"], batch["active"], self.gamma)
-            batch["stats"] = self.runner.engine.stats().to(torch.float64)
-        return batch
+            return self.episodes.run(self.gamma)
 
     def load_parameters(self, state_dict):
         """Replace the network parameters (e.g. a checkpoint or a reference ``ac_net.state_dict()``); Adam restarts."""
@@ -265,7 +211,7 @@ class SelfPlayTrainer:
 
     # ---- update ----------------------------------------------------------------------------
     def update(self, batch, defer_stats=False):
-        """``Agent.update`` (agent.py:39-62) on every recorded agent decision of the batch (see :meth:`_update_device`);
+        """``Agent.update`` (agent.py:39-62) on the decision records of :meth:`rollout` (see :meth:`_update_device`);
         then the statistics start their way to the host."""
         self._push_stats(self._update_device(batch))
         return None if defer_stats else self.fetch_stats()
@@ -282,8 +228,7 @@ class SelfPlayTrainer:
     def enable_step_graph(self, warmup=2):
         """Capture rollout + update (every launch of a batch, collectives and the fused Adam step included) in ONE CUDA
         graph: a batch is then a single graph launch (the ~60 small launches of a batch otherwise leave the GPU idle for a
-        fifth of the step).  Only for the persistent rollout + tensor-core update (no host decision inside a batch)."""
-        assert self.rollout_kind == "persistent" and self.update_kind == "tensor"
+        fifth of the step).  Nothing in a batch waits for the host."""
         for _ in range(warmup):
             self.update(self.rollout())
             self._batch_done()
@@ -295,7 +240,7 @@ class SelfPlayTrainer:
 
     def step(self, defer_stats=False):
         """One training batch: rollout + update (one graph launch when :meth:`enable_step_graph` was called)."""
-        if getattr(self, "_graph", None) is not None:
+        if self._graph is not None:
             self._graph.replay()
             self._push_stats(self._graph_stats)
             self._batch_done()
@@ -312,40 +257,18 @@ class SelfPlayTrainer:
             with torch.no_grad():
                 self.opponent.update(self.net)
 
-    def _update_device(self, batch):
-        """``Agent.update`` (agent.py:39-62) on every recorded agent decision of the batch; returns the device statistics.
+    def _update_device(self, recs):
+        """``Agent.update`` (agent.py:39-62) on the ``EpisodeRecords`` of a rollout; returns the device statistics.
 
         Gradients are accumulated as SUMS over the local decisions in the flat fp32 buffer; one fp32 all-reduce carries
         them and a tiny float64 one the decision count and the batch statistics; every rank then divides by the global
         count (the means of agent.py:47-56 over the global batch) and takes the same Adam step.  Nothing here waits for
         the GPU: the statistics travel to pinned host memory asynchronously and are read by :meth:`fetch_stats`
         (``defer_stats=True``: later -- the training loop reads them one batch late -- otherwise right away)."""
-        G = self.runner.n_games
-        if "records" in batch:                        # compact decision records of the persistent rollout
-            recs = batch["records"]
-            if self.update_kind == "tensor":
-                self.tc.run(self.packed, recs.state_rec, recs.action_rec, recs.qval, n_dec=recs.meta[:1],
-                            coeffs=(ACTOR_COEFF, CRITIC_COEFF, ENTROPY_COEFF))
-                sums = self.tc.sums
-            else:
-                n = min(int(recs.meta[0]), recs.cap)
-                obs = recs.view.observe_bf16(-1)[:n]
-                masks = recs.view.legal_mask().t()[:n]
-                sums = self.accumulate_gradients(obs, masks, recs.action_rec[:n].long(), recs.qval[:n])
-            stats = train_stats(self.runner.engine, recs, sums, torch.empty(STAT_FIELDS, dtype=torch.float64, device=self.device))
-        else:
-            act = batch["active"]
-            T = act.shape[0]
-            sel = act.reshape(-1).nonzero(as_tuple=True)[0]
-            n_local = torch.full((1,), float(sel.numel()), dtype=torch.float64, device=self.device)
-            obs = batch["obs"].reshape(T * G, -1)[sel]
-            masks = batch["mask"].permute(0, 2, 1).reshape(T * G, 6)[sel]
-            sums = self.accumulate_gradients(obs, masks, batch["action"].reshape(-1)[sel], batch["qval"].reshape(-1)[sel])
-            reward_total = batch["reward"].double().mul(act).sum().reshape(1)
-            unfinished = torch.full((1,), float(batch["unfinished"]), dtype=torch.float64, device=self.device)
-            one = torch.ones(1, dtype=torch.float64, device=self.device)
-            wins = (batch["stats"][:, 0] > batch["stats"][:, 1]).double().sum().reshape(1)
-            stats = torch.cat([n_local, sums, reward_total, one * G, batch["stats"].sum(dim=0), wins, unfinished])
+        self.tc.run(self.packed, recs.state_rec, recs.action_rec, recs.qval, n_dec=recs.meta[:1],
+                    coeffs=(ACTOR_COEFF, CRITIC_COEFF, ENTROPY_COEFF))
+        stats = train_stats(self.runner.engine, recs, self.tc.sums,
+                            torch.empty(STAT_FIELDS, dtype=torch.float64, device=self.device))
         allreduce_flat_and_stats(self.tc.flat, stats)                    # C1: 82,081 fp32 gradient sums, C2: 18 float64 counters
         self.tc.flat.mul_((1.0 / stats[0].clamp_min(1.0)).float())
         self.opt.step()
@@ -411,9 +334,8 @@ class SelfPlayTrainer:
                     b, st["games_per_sec"], st["reward"], st["player_score"], st["opponent_score"],
                     100 * st["win_percent"], st["ac_loss"]))
 
-        can_graph = graph and self.rollout_kind == "persistent" and self.update_kind == "tensor"
         for b in range(start_batch, batches):
-            if can_graph and self._graph is None and b >= start_batch + 2:
+            if graph and self._graph is None and b >= start_batch + 2:
                 self.enable_step_graph(warmup=0)             # the first two batches ran launch by launch (lazy initialisation)
             t0 = time.perf_counter()
             self.step(defer_stats=True)

@@ -11,7 +11,7 @@
 Tolerances (DESIGN.md §0): integer outputs bit-exact.  Logits / value (fp16 tensor-core operands, fp32 accumulation)
 per element |got - ref| <= 1e-3 * max(|ref|, floor) with floor = the largest |logit| of that decision's row (the largest
 |value| of the batch for the value head); log-probabilities and the entropy term 2e-3 + 1e-3 * floor absolute (they are differences of logits and a
-log-sum-exp).  Gradients of the update: see test_trainer_update_matches_reference_agent_update."""
+log-sum-exp).  Gradients of the update: see test_trainer_decision_updates_match_reference_agent_update."""
 import numpy as np
 import pytest
 
@@ -171,7 +171,7 @@ def test_policy_kernel_sampled_logp_matches_reference(tag, scale):
 
 
 @pytest.mark.parametrize("path,grad_tol,flip_frac", [("autograd-fp32", 2e-4, 2e-3), ("autograd-tf32", 6e-2, 0.06), ("tensor", 6e-2, 0.06)])
-def test_trainer_update_matches_reference_agent_update(path, grad_tol, flip_frac):
+def test_trainer_decision_updates_match_reference_agent_update(path, grad_tol, flip_frac):
     """Two ``Agent.update`` calls of the live reference (update.npz) through the trainer: the loss terms, the gradient of the
     first update and the parameters after both Adam steps -- for the fp32 autograd path, the TF32 autograd path and the
     hand-written tensor-core path (azb_a2c_update_gradients on packed decision states).  Gradient tolerance per tensor,
@@ -181,7 +181,7 @@ def test_trainer_update_matches_reference_agent_update(path, grad_tol, flip_frac
     from azul_deep_reinforcement_learning_b200.engine import BatchedAzul
     from azul_deep_reinforcement_learning_b200.train import SelfPlayTrainer
     z = load_update_golden()
-    tr = SelfPlayTrainer(64, learning_rate=float(z["learning_rate"]), gamma=float(z["gamma"]), seed=0, device=0, use_cuda_graph=False,
+    tr = SelfPlayTrainer(64, learning_rate=float(z["learning_rate"]), gamma=float(z["gamma"]), seed=0, device=0,
                          tf32_update=(path != "autograd-fp32"))
     tr.load_parameters({n: torch.from_numpy(z["param0_" + n]) for n in PARAM_NAMES})
     named = dict(tr.net.named_parameters())

@@ -111,31 +111,6 @@ def test_agent_opponent_in_batched_runner():
     assert batch["unfinished"] < n // 20 and float(batch["reward"].abs().sum()) > 0
 
 
-def test_cuda_graph_rollout_equals_eager():
-    """The CUDA-graph replay of the episode loop produces exactly the eager loop's batch."""
-    from azul_deep_reinforcement_learning_b200.azulnet.model import ActorCritic
-    from azul_deep_reinforcement_learning_b200.engine import PackedPolicy
-    from azul_deep_reinforcement_learning_b200.selfplay import BatchedGameRunner, GraphedEpisodes, run_episodes
-    torch.manual_seed(2)
-    net = ActorCritic(136, 180)
-    a = BatchedGameRunner(768, seed=21)                   # records observations with a separate azb_observe_bf16 launch
-    b = BatchedGameRunner(768, seed=21, record_obs=True)  # the opponent / reward kernel writes them
-    pa, pb = PackedPolicy(a.engine, net), PackedPolicy(b.engine, net)
-    graphed = GraphedEpisodes(b, pb, decisions=40)        # (its warm-up advances b's per-slot RNG position)
-    for rep in range(2):                                  # replaying twice: buffers are reused correctly
-        a.engine.state.copy_(b.engine.state)              # same RNG position: reset keeps the step counters
-        eager = run_episodes(a, pa)
-        g = graphed.run()
-        T = min(eager["active"].shape[0], g["active"].shape[0])
-        assert eager["unfinished"] == g["unfinished"] == 0
-        assert not bool(eager["active"][T:].any()) and not bool(g["active"][T:].any())
-        act = eager["active"][:T]
-        assert torch.equal(act, g["active"][:T])
-        for k in ("reward", "action", "logp", "value", "entropy", "obs"):
-            assert torch.equal(eager[k][:T][act], g[k][:T][act]), (rep, k)
-        assert torch.equal(a.engine.state, b.engine.state)
-
-
 def test_fused_a2c_loss_gradient_matches_autograd():
     """azb_a2c_loss_grad (one kernel: masked log-softmax, the three terms of Agent.update, their gradient) against PyTorch
     autograd of train.a2c_loss_terms -- the formula test_train_cpu pins to the reference's Agent.update -- on recorded
@@ -320,7 +295,7 @@ def test_discounted_returns_on_synthetic_records(k):
     assert float(recs.reward_sum) == total
 
 
-def test_training_cli_csv_checkpoint_and_resume(tmp_path):
+def test_training_cli_csv_checkpoint_resume_and_reload(tmp_path):
     """scripts/training.py equivalent (train.py main): writes <net>.csv (one row per batch) and <net>.pt; --resume continues
     the batch numbering, appends to the CSV, restores parameters + Adam state; the checkpoint loads as an opponent Agent."""
     import csv
@@ -344,7 +319,7 @@ def test_training_cli_csv_checkpoint_and_resume(tmp_path):
     assert ck2["batch"] == 4 and ck2["optimizer"]["state"][0]["step"] == 4
     assert not torch.equal(ck["ac_net"]["actor_linear1.weight"], ck2["ac_net"]["actor_linear1.weight"])
     # a resumed trainer starts from exactly the saved parameters
-    tr = train.SelfPlayTrainer(64, seed=3, use_cuda_graph=False)
+    tr = train.SelfPlayTrainer(64, seed=3)
     assert tr.load_checkpoint(name + ".pt") == 4
     for k, v in tr.net.state_dict().items():
         assert torch.equal(v.cpu(), ck2["ac_net"][k])

@@ -99,30 +99,33 @@ def _worker(rank, world, port, out_dir):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
     from azul_deep_reinforcement_learning_b200 import parallel
     from azul_deep_reinforcement_learning_b200.azulnet.model import ActorCritic
-    from azul_deep_reinforcement_learning_b200.train import (a2c_loss_terms, allreduce_gradients, allreduce_gradients_and_stats,
-                                                             global_count)
+    from azul_deep_reinforcement_learning_b200.engine import PARAM_ORDER
+    from azul_deep_reinforcement_learning_b200.train import a2c_loss_terms, allreduce_flat_and_stats
     parallel.init("gloo")
     torch.manual_seed(0)
     net = ActorCritic(136, 180)
     n = 40 + 25 * rank                                      # ranks hold different numbers of transitions
     obs, mask, action, qval = _fake_batch(n, 10 + rank)
-    n_global = global_count(n, "cpu")
-    a, c, e = a2c_loss_terms(net, obs, mask, action, qval)
-    ((a + 0.5 * c + 0.1 * e) / n_global).backward()
-    params = list(net.parameters())
-    allreduce_gradients(params)
-    torch.save([p.grad.clone() for p in params], os.path.join(out_dir, "grads%d.pt" % rank))
-    # the trainer's form: unscaled gradient sums + the count in ONE collective, divided afterwards
-    net.zero_grad()
+    # the trainer's form: unscaled gradient sums in ONE flat fp32 buffer (PARAM_ORDER) + the count in the statistics
+    # vector, both all-reduced, then divided by the global count
     a, c, e = a2c_loss_terms(net, obs, mask, action, qval)
     (a + 0.5 * c + 0.1 * e).backward()
-    stats = allreduce_gradients_and_stats(params, torch.tensor([float(n), 7.0 + rank]))
+    named = dict(net.named_parameters())
+    flat = torch.cat([named[name].grad.reshape(-1) for name in PARAM_ORDER]).float()
+    stats = torch.tensor([float(n), 7.0 + rank], dtype=torch.float64)
+    allreduce_flat_and_stats(flat, stats)
     assert stats.tolist() == [105.0, 15.0]
-    torch.save([p.grad / stats[0].float() for p in params], os.path.join(out_dir, "grads_one%d.pt" % rank))
+    flat /= stats[0].float()
+    grads, off = {}, 0
+    for name in PARAM_ORDER:
+        k = named[name].numel()
+        grads[name] = flat[off:off + k].view_as(named[name])
+        off += k
+    torch.save([grads[name] for name, _ in net.named_parameters()], os.path.join(out_dir, "grads%d.pt" % rank))
     torch.distributed.destroy_process_group()
 
 
-def test_two_rank_gradient_allreduce_matches_global_batch(tmp_path):
+def test_two_rank_flat_gradient_allreduce_matches_global_batch(tmp_path):
     from azul_deep_reinforcement_learning_b200.azulnet.model import ActorCritic
     from azul_deep_reinforcement_learning_b200.train import a2c_loss_terms
     from tests.helpers import free_port
@@ -134,10 +137,9 @@ def test_two_rank_gradient_allreduce_matches_global_batch(tmp_path):
     a, c, e = a2c_loss_terms(net, obs, mask, action, qval)
     ref = torch.autograd.grad((a + 0.5 * c + 0.1 * e) / 105, list(net.parameters()))
     for r in range(2):
-        for name in ("grads%d.pt", "grads_one%d.pt"):
-            got = torch.load(tmp_path / (name % r))
-            for g1, g2 in zip(got, ref):
-                assert torch.allclose(g1, g2, rtol=1e-4, atol=1e-6), name
+        got = torch.load(tmp_path / ("grads%d.pt" % r))
+        for g1, g2 in zip(got, ref):
+            assert torch.allclose(g1, g2, rtol=1e-4, atol=1e-6), r
 
 
 def _flat_worker(rank, world, port, out):

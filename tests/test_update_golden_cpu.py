@@ -27,7 +27,7 @@ def test_facade_actor_critic_matches_reference_forward():
 
 
 def test_discounted_returns_match_nn_runner_train():
-    """nn_runner.py:72-75 on the recorded episodes, through the batched [T, G] routine the trainer uses."""
+    """nn_runner.py:72-75 on the recorded episodes, through the batched [T, G] routine of the step-wise episode loop."""
     from azul_deep_reinforcement_learning_b200.selfplay import discounted_returns
     z = load_update_golden()
     reward, done, qref = z["reward"].astype(np.float64), z["done"], z["qvals"]
