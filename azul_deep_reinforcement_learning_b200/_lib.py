@@ -14,6 +14,7 @@ SYMBOLS = [
     "azb_stats", "azb_move", "azb_next_player", "azb_count_score", "azb_new_round", "azb_round_flags",
     "azb_opponent_random", "azb_policy_packed_bytes", "azb_policy_pack_weights", "azb_policy_step",
     "azb_observe_bf16", "azb_a2c_loss_grad", "azb_policy_rollout", "azb_policy_rollout_vs_policy", "azb_discounted_returns",
+    "azb_greedy_action", "azb_opponent_greedy", "azb_policy_rollout_vs_greedy",
     "azb_update_workspace_bytes", "azb_a2c_update_gradients", "azb_update_set_chunk_rows", "azb_train_stats",
     "azb_v_state_words", "azb_v_record_size", "azb_v_n_actions", "azb_v_reset", "azb_v_legal_mask", "azb_v_step",
     "azb_v_rollout_random", "azb_v_import_state", "azb_v_export_state",
@@ -59,12 +60,15 @@ def load():
     L.azb_new_round.argtypes = [vp, vp, vp, vp]
     L.azb_round_flags.argtypes = [vp, vp, vp, vp]
     L.azb_opponent_random.argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, vp, vp]
+    L.azb_opponent_greedy.argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, vp, vp]
+    L.azb_greedy_action.argtypes = [vp, vp, vp, vp]
     L.azb_policy_pack_weights.argtypes = [vp] * 11
     L.azb_policy_step.argtypes = [vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp]
     f32 = ctypes.c_float
     L.azb_a2c_loss_grad.argtypes = [vp, i64, vp, vp, vp, vp, vp, f32, f32, f32, f32, vp, vp, vp, vp]
     L.azb_policy_rollout.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp, i64] + [vp] * 16
     L.azb_policy_rollout_vs_policy.argtypes = [vp, vp, vp, vp, i32, i32, vp, vp, i64] + [vp] * 13
+    L.azb_policy_rollout_vs_greedy.argtypes = [vp, vp, vp, i32, i32, vp, vp, i64] + [vp] * 15
     L.azb_discounted_returns.argtypes = [vp, i32, ctypes.c_double, vp, vp, vp, vp, vp, vp, vp]
     L.azb_update_set_chunk_rows.argtypes = [i64]
     L.azb_train_stats.argtypes = [vp, vp, vp, i64, vp, vp, vp, vp]

@@ -751,12 +751,13 @@ __global__ void k_op(Launch L, const uint8_t* __restrict__ action, const int8_t*
 
 // a14: GameRunner.step after the agent's own move: opponent loop, reward, done, next mask -- and, optionally, the
 // observation of the resulting state from seat 1's perspective (the next decision's network input) in bfloat16, so
-// that a training rollout needs no separate observation launch.  Blocks are whole warps.
-template <int P, int POOL>
-__global__ void k_opponent_random(Launch L, int require_two, int16_t* __restrict__ player_score,
-                                  int16_t* __restrict__ reward_out, uint8_t* __restrict__ done_out,
-                                  uint8_t* __restrict__ status_out, uint32_t* __restrict__ mask6_out,
-                                  __nv_bfloat16* __restrict__ obs_out)
+// that a training rollout needs no separate observation launch.  Blocks are whole warps.  GREEDY: the greedy agent is
+// the opponent (k_opponent_greedy), else the random agent (k_opponent_random).
+template <int P, int POOL, bool GREEDY>
+__device__ __forceinline__ void opponent_turns(Launch L, int require_two, int16_t* __restrict__ player_score,
+                                               int16_t* __restrict__ reward_out, uint8_t* __restrict__ done_out,
+                                               uint8_t* __restrict__ status_out, uint32_t* __restrict__ mask6_out,
+                                               __nv_bfloat16* __restrict__ obs_out)
 {
     constexpr int D = 32 + 52 * P;
     extern __shared__ __align__(16) unsigned char opp_smem[];          // [warp][32][D + 1] bf16 when obs_out
@@ -767,7 +768,7 @@ __global__ void k_opponent_random(Launch L, int require_two, int16_t* __restrict
     if (valid) {
         const Philox rng{L.k0, L.k1};
         uint32_t m[6];
-        const int32_t diff = opponent_random<P, POOL>(gm, rng, L.gid0 + (uint32_t)g, require_two != 0, m);
+        const int32_t diff = opponent_random<P, POOL, GREEDY>(gm, rng, L.gid0 + (uint32_t)g, require_two != 0, m);
         gm.store(L.state, L.n, g);
         if (player_score) {
             if (reward_out) reward_out[g] = (int16_t)(diff - (int32_t)player_score[g]);    // game_runner.py:51
@@ -784,6 +785,44 @@ __global__ void k_opponent_random(Launch L, int require_two, int16_t* __restrict
         observe_row<P, __nv_bfloat16>(gm, 0, tile + lane * (D + 1));
         if (g0 < L.n) observe_flush<P, __nv_bfloat16>(tile, obs_out + g0 * D, L.n - g0 < 32 ? L.n - g0 : 32, lane);
     }
+}
+
+template <int P, int POOL>
+__global__ void k_opponent_random(Launch L, int require_two, int16_t* __restrict__ player_score,
+                                  int16_t* __restrict__ reward_out, uint8_t* __restrict__ done_out,
+                                  uint8_t* __restrict__ status_out, uint32_t* __restrict__ mask6_out,
+                                  __nv_bfloat16* __restrict__ obs_out)
+{
+    opponent_turns<P, POOL, false>(L, require_two, player_score, reward_out, done_out, status_out, mask6_out, obs_out);
+}
+
+template <int P, int POOL>
+__global__ void k_opponent_greedy(Launch L, int require_two, int16_t* __restrict__ player_score,
+                                  int16_t* __restrict__ reward_out, uint8_t* __restrict__ done_out,
+                                  uint8_t* __restrict__ status_out, uint32_t* __restrict__ mask6_out,
+                                  __nv_bfloat16* __restrict__ obs_out)
+{
+    opponent_turns<P, POOL, true>(L, require_two, player_score, reward_out, done_out, status_out, mask6_out, obs_out);
+}
+
+// the greedy agent's action for the seat to move (greedy_action, the word of the game's current env step); state untouched
+template <int P, int POOL>
+__global__ void k_greedy_action(Launch L, uint8_t* __restrict__ action_out)
+{
+    const int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (g >= L.n) return;
+    Game<P> gm;
+    gm.load(L.state, L.n, g);
+    uint32_t a = 180u;
+    if (!gm.ended()) {
+        uint32_t m[6], w[4];
+        legal_mask(gm, m);
+        const Philox rng{L.k0, L.k1};
+        rng(L.gid0 + (uint32_t)g, gm.steps >> 2, PURPOSE_ACTION, 0u, w);
+        const uint32_t idx = gm.steps & 3u;
+        a = greedy_action<P, POOL>(gm, m, idx == 0u ? w[0] : idx == 1u ? w[1] : idx == 2u ? w[2] : w[3]);
+    }
+    action_out[g] = a < 180u ? (uint8_t)a : (uint8_t)AZB_ACTION_SKIP;
 }
 
 template <int P>
@@ -836,6 +875,30 @@ static int launch_step(const azb_t* h, const Launch& L, const uint8_t* action, c
     const int64_t resident = (int64_t)h->sm_count * per_sm;
     if (blocks > resident) blocks = resident;
     kern<<<dim3((unsigned)blocks), 32 * WARPS, smem, stream>>>(L, action, draws, O, aligned, h->sched);
+    return 0;
+}
+
+// azb_opponent_random / azb_opponent_greedy
+template <bool GREEDY>
+static int launch_opponent(azb_t* h, uint32_t* state, int require_two, int16_t* player_score, int16_t* reward_out,
+                           uint8_t* done_out, uint8_t* status_out, uint32_t* mask6_out, void* obs_bf16_out, void* stream)
+{
+    CHECK_HANDLE(h);
+    if (!state) return azb_fail(AZB_E_INVALID, "state is null%s");
+    const Launch L = make_launch(h, state);
+    // with the observation output every warp stages 32 rows in shared memory (32 x (33 + 52P) bf16 per warp): 128-thread
+    // blocks for 2 / 3 players (35 / 47 KB), 64-thread blocks for 4 players (31 KB) stay under the 48 KB default limit
+    const int threads = obs_bf16_out ? (h->players == 4 ? 64 : 128) : h->block_threads;
+    const size_t smem = obs_bf16_out ? (size_t)(threads / 32) * 32 * (32 + 52 * h->players + 1) * sizeof(__nv_bfloat16) : 0;
+    const dim3 grid((unsigned)((h->n_games + threads - 1) / threads));
+    __nv_bfloat16* obs = (__nv_bfloat16*)obs_bf16_out;
+    if (GREEDY)
+        DISPATCH_PP(h, (k_opponent_greedy<P, POOL><<<grid, threads, smem, (cudaStream_t)stream>>>(
+                           L, require_two, player_score, reward_out, done_out, status_out, mask6_out, obs)))
+    else
+        DISPATCH_PP(h, (k_opponent_random<P, POOL><<<grid, threads, smem, (cudaStream_t)stream>>>(
+                           L, require_two, player_score, reward_out, done_out, status_out, mask6_out, obs)))
+    CHECK_LAUNCH();
     return 0;
 }
 
@@ -1088,16 +1151,23 @@ int azb_new_round(azb_t* h, uint32_t* state, const int8_t* draws20, void* stream
 int azb_opponent_random(azb_t* h, uint32_t* state, int require_two, int16_t* player_score, int16_t* reward_out,
                         uint8_t* done_out, uint8_t* status_out, uint32_t* mask6_out, void* obs_bf16_out, void* stream)
 {
+    return launch_opponent<false>(h, state, require_two, player_score, reward_out, done_out, status_out, mask6_out,
+                                  obs_bf16_out, stream);
+}
+
+int azb_opponent_greedy(azb_t* h, uint32_t* state, int require_two, int16_t* player_score, int16_t* reward_out,
+                        uint8_t* done_out, uint8_t* status_out, uint32_t* mask6_out, void* obs_bf16_out, void* stream)
+{
+    return launch_opponent<true>(h, state, require_two, player_score, reward_out, done_out, status_out, mask6_out,
+                                 obs_bf16_out, stream);
+}
+
+int azb_greedy_action(azb_t* h, const uint32_t* state, uint8_t* action_out, void* stream)
+{
     CHECK_HANDLE(h);
-    if (!state) return azb_fail(AZB_E_INVALID, "state is null%s");
-    const Launch L = make_launch(h, state);
-    // with the observation output every warp stages 32 rows in shared memory (32 x (33 + 52P) bf16 per warp): 128-thread
-    // blocks for 2 / 3 players (35 / 47 KB), 64-thread blocks for 4 players (31 KB) stay under the 48 KB default limit
-    const int threads = obs_bf16_out ? (h->players == 4 ? 64 : 128) : h->block_threads;
-    const size_t smem = obs_bf16_out ? (size_t)(threads / 32) * 32 * (32 + 52 * h->players + 1) * sizeof(__nv_bfloat16) : 0;
-    const dim3 grid((unsigned)((h->n_games + threads - 1) / threads));
-    DISPATCH_PP(h, (k_opponent_random<P, POOL><<<grid, threads, smem, (cudaStream_t)stream>>>(
-                       L, require_two, player_score, reward_out, done_out, status_out, mask6_out, (__nv_bfloat16*)obs_bf16_out)));
+    if (!state || !action_out) return azb_fail(AZB_E_INVALID, "null buffer%s");
+    const Launch L = make_launch(h, const_cast<uint32_t*>(state));
+    DISPATCH_PP(h, (k_greedy_action<P, POOL><<<grid_of(h), h->block_threads, 0, (cudaStream_t)stream>>>(L, action_out)));
     CHECK_LAUNCH();
     return 0;
 }

@@ -111,15 +111,15 @@ __device__ __forceinline__ void finish_game(Game<2>& h, uint32_t gidx, uint32_t 
     if (status_out) status_out[gidx] |= (uint8_t)h.status();
 }
 
-// GameRunner.step's opponent loop (game_runner.py:46-52; opponent_random() in azb_rules.cuh is the one-game form) for the 32
-// games of a warp TOGETHER: every lane makes the same sequence of rule calls on its own game as the one-game form, but a game
+// GameRunner.step's opponent loop (game_runner.py:46-52; opponent_random() / opponent_greedy() in azb_rules.cuh are the one-game
+// forms) for the 32 games of a warp TOGETHER, with the random agent's or -- GREEDY -- the greedy agent's pick: every lane makes the same sequence of rule calls on its own game as the one-game form, but a game
 // whose round ended -- by the agent's move (`pending`) or by an opponent move -- waits until no lane of the warp can move any
 // more, and ONE count_score + refill pass serves all of them (the rollout kernel's light / heavy split).  Run one game at a
 // time under divergence, the ~1,300-instruction pass was walked by the warp once for the agent's move and again at every
 // loop iteration in which some lane's opponent move ended a round.  Inactive lanes take part in the votes only.
-template <int POOL>
-__device__ __forceinline__ int32_t opponent_random_warp(Game<2>& h, const Philox& rng, uint32_t gid, bool active, bool pending,
-                                                        uint32_t m[6])
+template <int POOL, bool GREEDY>
+__device__ __forceinline__ int32_t opponent_warp(Game<2>& h, const Philox& rng, uint32_t gid, bool active, bool pending,
+                                                 uint32_t m[6])
 {
     int phase = !active ? 2 : pending ? 1 : 0;            // 0 to move, 1 round over: waits for the pass, 2 handed back
     for (;;) {
@@ -139,7 +139,7 @@ __device__ __forceinline__ int32_t opponent_random_warp(Game<2>& h, const Philox
                     rng(gid, h.steps >> 2, PURPOSE_ACTION, 0u, w);
                     const uint32_t idx = h.steps & 3u;
                     const uint32_t word = idx == 0u ? w[0] : idx == 1u ? w[1] : idx == 2u ? w[2] : w[3];
-                    apply_move<2, POOL>(h, random_action(m, word));        // azul.py:304
+                    apply_move<2, POOL>(h, opponent_pick<2, POOL, GREEDY>(h, m, word));   // azul.py:304
                     h.steps += 1u;
                     if (is_end_of_round(h)) phase = 1;                     // azul.py:306
                     else next_player(h);                                   // azul.py:313
@@ -218,10 +218,13 @@ __device__ __forceinline__ RowPart load_part(const float* parts, int slot)
 // the tile loop with the agent's image resident (act_filter 0, records), then -- with the opponent's image copied over it --
 // passes with act_filter 1 and no records until no game of the CTA is in the opponent's hands, then the runner block, whose
 // random opponent then has nothing to play; the agent's image comes back for the next decision.
+// GREEDY: the runner mode against the greedy agent (azb_policy_rollout_vs_greedy): the runner block's opponent loop picks the
+// greedy agent's moves instead of the random agent's; nothing else differs.
 constexpr int MAX_OPP_PASSES = 64;           // the bound of the eager loop (selfplay.py _opponent_policy_moves)
-template <int POOL, int MODE, bool FULL, bool OPP = false>
+template <int POOL, int MODE, bool FULL, bool OPP = false, bool GREEDY = false>
 __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
 {
+    static_assert(!(GREEDY && OPP), "one opponent per launch: a frozen network or the greedy agent");
     extern __shared__ __align__(128) unsigned char smem[];
     const int tid = threadIdx.x, warp = tid >> 5, row = tid & (TILE_M - 1), part = tid >> 7;
     unsigned char* a_tile = smem + OFF_A;
@@ -733,8 +736,9 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
     bool any_alive = true;
     if (A.runner_mode) {
         // GameRunner.step after the agent's move (game_runner.py:46-55), one thread per game of this CTA's tiles: finish the
-        // round the move may have ended, let the random opponent play until seat 1 is to move with >= 2 legal actions (or the
-        // game is over), take the reward from a score preview, and close the decision's record.  OPP: the policy opponent's
+        // round the move may have ended, let the random opponent (GREEDY: the greedy agent) play until seat 1 is to move with
+        // >= 2 legal actions (or the game is over), take the reward from a score preview, and close the decision's record.
+        // OPP: the policy opponent's
         // passes already restored that invariant, so the random opponent plays no move (as the eager path's trailing
         // azb_opponent_random(require_two = 1))
         bool alive = false;
@@ -755,7 +759,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
             // OPP: a game frozen at the pass bound gets no random move either (its mask is reported empty)
             const bool frozen = OPP && (h.status() & ST_STUCK) != 0u;
             if (frozen) for (int p = 0; p < 6; p++) m2[p] = 0u;
-            const int32_t diff = opponent_random_warp<POOL>(h, rng, gid, decided && !frozen, pending, m2);
+            const int32_t diff = opponent_warp<POOL, GREEDY>(h, rng, gid, decided && !frozen, pending, m2);
             if (!decided) continue;
             h.store(A.state, A.n, g);
             const int32_t before = (int32_t)A.player_score[g];
@@ -837,17 +841,17 @@ __global__ void k_pack_weights(const float* __restrict__ w1a, const float* __res
     }
 }
 
-template <int POOL, int MODE, bool FULL, bool OPP = false>
+template <int POOL, int MODE, bool FULL, bool OPP = false, bool GREEDY = false>
 static int launch_policy(const PolicyArgs& A, int grid, cudaStream_t stream)
 {
-    AZB_CUDA(cudaFuncSetAttribute(k_policy<POOL, MODE, FULL, OPP>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    AZB_CUDA(cudaFuncSetAttribute(k_policy<POOL, MODE, FULL, OPP, GREEDY>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;       // see griddepcontrol in k_policy
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    AZB_CUDA(cudaLaunchKernelEx(&cfg, k_policy<POOL, MODE, FULL, OPP>, A));
+    AZB_CUDA(cudaLaunchKernelEx(&cfg, k_policy<POOL, MODE, FULL, OPP, GREEDY>, A));
     return 0;
 }
 
@@ -963,6 +967,39 @@ int azb_policy_rollout_vs_policy(azb_t* h, uint32_t* state, const void* packed, 
     int rc = 0;
     if (h->tile_pool == AZB_POOL_LID) rc = mode == 0 ? pol::launch_policy<1, 0, false, true>(A, grid, (cudaStream_t)stream) : pol::launch_policy<1, 1, false, true>(A, grid, (cudaStream_t)stream);
     else rc = mode == 0 ? pol::launch_policy<0, 0, false, true>(A, grid, (cudaStream_t)stream) : pol::launch_policy<0, 1, false, true>(A, grid, (cudaStream_t)stream);
+    if (rc) return rc;
+    CHECK_LAUNCH();
+    return 0;
+}
+
+int azb_policy_rollout_vs_greedy(azb_t* h, uint32_t* state, const void* packed, int mode, int k_decisions,
+                                 int16_t* player_score, uint32_t* n_dec, int64_t rec_cap, uint32_t* state_rec,
+                                 uint8_t* action_rec, float* logp_rec, float* value_rec, int32_t* slot_rec, int16_t* reward_rec,
+                                 uint8_t* flags_rec, uint32_t* steps_used, uint8_t* action_out, float* logp_out,
+                                 float* value_out, uint32_t* mask6_out, uint8_t* done_out, uint8_t* status_out, void* stream)
+{
+    CHECK_HANDLE(h);
+    if (!state || !packed) return azb_fail(AZB_E_INVALID, "null buffer%s");
+    if (h->players != 2) return azb_fail(AZB_E_INVALID, "the policy network is defined for 2 players (136 inputs, agent.py:29)%s");
+    if (mode != 0 && mode != 1) return azb_fail(AZB_E_INVALID, "mode must be 0 (sample) or 1 (argmax)%s");
+    if (k_decisions < 1) return azb_fail(AZB_E_INVALID, "k_decisions must be >= 1%s");
+    if (!player_score || !n_dec || rec_cap < 1 || !state_rec || !action_rec || !slot_rec || !reward_rec || !flags_rec)
+        return azb_fail(AZB_E_INVALID, "runner mode needs player_score, n_dec, rec_cap and the state / action / slot / reward / flags records%s");
+    pol::PolicyArgs A;
+    A.state_in = state; A.state = state; A.n = h->n_games; A.packed = (const unsigned char*)packed;
+    A.k0 = (uint32_t)h->seed; A.k1 = (uint32_t)(h->seed >> 32); A.gid0 = (uint32_t)h->game_id_base;
+    A.mode = mode; A.apply_step = 1; A.first_rule = h->first_player; A.counters = nullptr; A.act_filter = 0;
+    A.logits_out = nullptr; A.value_out = value_out; A.action_out = action_out; A.logp_out = logp_out; A.entropy_out = nullptr;
+    A.done_out = done_out; A.status_out = status_out; A.mask6_out = mask6_out;
+    A.k_decisions = k_decisions; A.runner_mode = 1; A.player_score = player_score; A.n_dec = n_dec; A.rec_cap = rec_cap;
+    A.state_rec = state_rec; A.action_rec = action_rec; A.logp_rec = logp_rec; A.value_rec = value_rec; A.slot_rec = slot_rec;
+    A.reward_rec = reward_rec; A.flags_rec = flags_rec; A.steps_used = steps_used;
+    A.opponent_packed = nullptr; A.opp_passes = nullptr;
+    const int64_t tiles = (h->n_games + pol::TILE_M - 1) / pol::TILE_M;
+    const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
+    int rc = 0;
+    if (h->tile_pool == AZB_POOL_LID) rc = mode == 0 ? pol::launch_policy<1, 0, false, false, true>(A, grid, (cudaStream_t)stream) : pol::launch_policy<1, 1, false, false, true>(A, grid, (cudaStream_t)stream);
+    else rc = mode == 0 ? pol::launch_policy<0, 0, false, false, true>(A, grid, (cudaStream_t)stream) : pol::launch_policy<0, 1, false, false, true>(A, grid, (cudaStream_t)stream);
     if (rc) return rc;
     CHECK_LAUNCH();
     return 0;

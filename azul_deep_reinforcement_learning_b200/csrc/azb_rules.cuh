@@ -688,6 +688,140 @@ AZB_HD uint32_t random_action(const uint32_t m[6], uint32_t word)
     return random_action_pb(m, word, p, b) ? 30u * p + b : 180u;
 }
 
+// The wall points (azul.py:211-290, without the bonus statistics) that the full pattern lines `full` (bit r = row r; its
+// colour at (pat >> 6r) & 7) earn when placed in row order on the colour-indexed wall `wall` / its column-space copy `wc`.
+// The placement arithmetic of score_player_g, kept separate so that the scoring pass's code stays as it is.
+AZB_HD int wall_gain(uint32_t pat, uint32_t wall, uint32_t wc, uint32_t full)
+{
+    int gain = 0;
+    AZB_ROLLED
+    while (full) {
+        const uint32_t r = (uint32_t)ctz(full);
+        full &= full - 1u;
+        const uint32_t sh5 = 5u * r, c = (pat >> (6u * r)) & 7u;
+        wall |= 1u << (sh5 + c);
+        uint32_t k = c + r;
+        k = k >= 5u ? k - 5u : k;
+        wc |= 1u << (sh5 + k);
+        const uint32_t rowbits = (wc >> sh5) & 31u;
+        const int hr = ctz(~(rowbits >> (k + 1u)));
+        const int hl = clz(~((rowbits << (31u - k)) << 1));
+        const uint32_t colbits = (wc >> k) & M5;
+        const int vd = (ctz(~(colbits >> (sh5 + 5u)) & M5) * 13) >> 6;
+        const int vu = (clz(~((colbits << (31u - sh5)) << 5) & 0x84210800u) * 13) >> 6;
+        const int h = hr + hl, v = vd + vu;
+        gain += h + v + 1 + ((h > 0 && v > 0) ? 1 : 0);
+        gain += rowbits == 31u ? 2 : 0;
+        gain += ((wall >> c) & M5) == M5 ? 10 : 0;
+        gain += colbits == M5 ? 7 : 0;
+    }
+    return gain;
+}
+
+// ---- the greedy agent: the best one-move score for the seat to move ----
+// Spec (shared with ao_greedy_action in tests/harness/greedy_oracle.c):
+//   v(a) = the mover's score after Azul.move(a) (azul.py:118-161) and count_score (azul.py:192-295) on a copy, WITHOUT the
+//          clamp at zero of azul.py:294-295: score + the wall points and bonuses of every full pattern line placed in row
+//          order - the floor penalty.  (With the clamp, at score 0 dumping tiles to the floor would tie with a placement.)
+//   T    = the legal actions of largest v, in ascending action index.
+//   pick = T[mulhi(word, |T|)], word = the random agent's word of this env step (word steps & 3 of
+//          Philox(gid, steps >> 2, ACTION, 0)); one best action uses no randomness.  180 when no action is legal.
+// v differs between actions only through the floor after the move and, for a move that completes line r with colour c,
+// the wall points with (r, c) added: so the value compared is u = (completes ? W(r, c) - W0 : 0) - penalty(floor after),
+// with W0 the wall points of the lines already full and W(r, c) computed once per (line, colour) that some source can
+// complete.  One game per thread: the loops run over colours and the sources holding them, never over all 180 actions.
+template <int P, int POOL>
+AZB_HD uint32_t greedy_action(const Game<P>& g, const uint32_t m[6], uint32_t word)
+{
+    const int s = g.seat();
+    const uint32_t pat = g.sel(g.pat, s), wall = g.sel(g.wall, s), scf = g.sel(g.scf, s);
+    const uint32_t f = (scf >> 16) & 7u, token = (g.misc >> 5) & 1u;
+    uint32_t wc = 0, full = 0;
+    int room[5];
+#pragma unroll
+    for (int r = 0; r < 5; r++) {
+        const uint32_t row = (wall >> (5 * r)) & 31u;
+        wc |= (((row << r) | (row >> (5 - r))) & 31u) << (5 * r);
+        room[r] = r + 1 - (int)((pat >> (6 * r + 3)) & 7u);
+        full |= (room[r] == 0 ? 1u : 0u) << r;
+    }
+    const int w0 = wall_gain(pat, wall, wc, full);
+    const uint32_t src = m[0];                           // every source / colour that holds a tile
+    int best = -1000;
+    uint32_t bm[6] = {0u, 0u, 0u, 0u, 0u, 0u};          // the legal actions of value `best`, as mask words
+    AZB_ROLLED
+    for (uint32_t c = 0; c < 5u; c++) {
+        uint32_t bits = (src >> (6u * c)) & 63u;
+        if (!bits) continue;
+        // the counts of colour c in its sources; the largest decides which lines a take of c can complete
+        int maxn = 0;
+        for (uint32_t t = bits; t; t &= t - 1u) {
+            const uint32_t b = (uint32_t)ctz(t) + 6u * c;
+            const int n = (int)(((g.pl0 >> b) & 1u) | (((g.pl1 >> b) & 1u) << 1) | (((g.pl2 >> b) & 1u) << 2) | (((g.pl3 >> b) & 1u) << 3));
+            maxn = n > maxn ? n : maxn;
+        }
+        int dw[5];
+#pragma unroll
+        for (int r = 0; r < 5; r++) {
+            dw[r] = 0;
+            // line r open for c (m[r + 1] holds c at some source) and completable by the largest take
+            const bool open = ((m[r + 1] >> (6u * c)) & 63u) != 0u;
+            if (open && room[r] > 0 && maxn >= room[r])
+                dw[r] = wall_gain((pat & ~(7u << (6 * r))) | (c << (6 * r)), wall, wc, full | (1u << r)) - w0;
+        }
+        AZB_ROLLED
+        for (; bits; bits &= bits - 1u) {
+            const uint32_t d = (uint32_t)ctz(bits), b = d + 6u * c;
+            const int n = (int)(((g.pl0 >> b) & 1u) | (((g.pl1 >> b) & 1u) << 1) | (((g.pl2 >> b) & 1u) << 2) | (((g.pl3 >> b) & 1u) << 3));
+            const int f0 = (int)f + (d == 0u ? (int)token : 0);
+            // the floor (p = 0) takes all n tiles; line r = p - 1 takes up to room[r], the rest falls
+            int lbest = -1000;
+            uint32_t lset = 0u;
+#pragma unroll
+            for (int p = 0; p < 6; p++) {
+                const int rm = p == 0 ? 0 : room[p - 1];
+                const int placed = p == 0 ? 0 : (n < rm ? n : rm);
+                int fl = f0 + n - placed;
+                fl = fl < 7 ? fl : 7;
+                const int pen = (int)((0xEB864210u >> (4 * fl)) & 15u);
+                const int u = (p > 0 && rm > 0 && n >= rm ? dw[p - 1] : 0) - pen;
+                const bool legal = (m[p] >> b) & 1u;
+                const bool gt = legal && u > lbest, eq = legal && u == lbest;
+                lset = gt ? 1u << p : (eq ? lset | (1u << p) : lset);
+                lbest = gt ? u : lbest;
+            }
+            // (the floor always takes a tile the source holds: lset is never empty)
+            const bool gt = lbest > best, take = lbest >= best;
+#pragma unroll
+            for (int p = 0; p < 6; p++) {
+                const uint32_t keep = gt ? 0u : bm[p];
+                bm[p] = take ? keep | (((lset >> p) & 1u) << b) : bm[p];
+            }
+            best = gt ? lbest : best;
+        }
+    }
+    // T in ascending action index: word 0 (the floor, actions 0..29) first, then lines 1..5
+    const uint32_t n0 = (uint32_t)popc(bm[0]), n1 = (uint32_t)popc(bm[1]), n2 = (uint32_t)popc(bm[2]),
+                   n3 = (uint32_t)popc(bm[3]), n4 = (uint32_t)popc(bm[4]), n5 = (uint32_t)popc(bm[5]);
+    const uint32_t e1 = n0, e2 = e1 + n1, e3 = e2 + n2, e4 = e3 + n3, e5 = e4 + n4, total = e5 + n5;
+    if (total == 0u) return 180u;
+    const uint32_t k = mulhi(word, total);
+    uint32_t before = 0u, w = bm[0], p = 0u;
+    before = k >= e1 ? e1 : before; w = k >= e1 ? bm[1] : w; p = k >= e1 ? 1u : p;
+    before = k >= e2 ? e2 : before; w = k >= e2 ? bm[2] : w; p = k >= e2 ? 2u : p;
+    before = k >= e3 ? e3 : before; w = k >= e3 ? bm[3] : w; p = k >= e3 ? 3u : p;
+    before = k >= e4 ? e4 : before; w = k >= e4 ? bm[4] : w; p = k >= e4 ? 4u : p;
+    before = k >= e5 ? e5 : before; w = k >= e5 ? bm[5] : w; p = k >= e5 ? 5u : p;
+    return 30u * p + select_bit(w, k - before);
+}
+
+// the opponent's pick at one env step: the random agent's, or the greedy agent's, from the same action word
+template <int P, int POOL, bool GREEDY>
+AZB_HD uint32_t opponent_pick(const Game<P>& g, const uint32_t m[6], uint32_t word)
+{
+    return GREEDY ? greedy_action<P, POOL>(g, m, word) : random_action(m, word);
+}
+
 // ---- unpacked record <-> packed game (kernel K7; record layout in layout.py) -----------------
 // Returns false (and flags ST_BAD_IMPORT) when the record cannot be represented: a pattern row
 // holding two colours, or a count outside its field.
@@ -946,8 +1080,9 @@ AZB_HD int rollout_steps(Game<P>& g, const Philox& rng, uint32_t gid, int first_
 // Plays random-agent moves (Philox ACTION words, like the rollout) until it is seat 1's turn with at
 // least two legal actions (require_two: the reference also lets the opponent agent play seat 1's
 // forced moves, game_runner.py:46; GameRunner.reset does not, :84-85) or the game is over.  Returns
-// the score difference seat 1 - seat 2 after a count_score on a copy (game_runner.py:48-50).
-template <int P, int POOL>
+// the score difference seat 1 - seat 2 after a count_score on a copy (game_runner.py:48-50).  GREEDY: the greedy agent
+// (greedy_action) picks the opponent's moves from the same words.
+template <int P, int POOL, bool GREEDY = false>
 AZB_HD int32_t opponent_random(Game<P>& g, const Philox& rng, uint32_t gid, bool require_two, uint32_t m[6])
 {
     AZB_ROLLED
@@ -961,11 +1096,20 @@ AZB_HD int32_t opponent_random(Game<P>& g, const Philox& rng, uint32_t gid, bool
         rng(gid, g.steps >> 2, PURPOSE_ACTION, 0u, w);
         const uint32_t idx = g.steps & 3u;
         const uint32_t word = idx == 0u ? w[0] : idx == 1u ? w[1] : idx == 2u ? w[2] : w[3];
-        advance<P, POOL>(g, random_action(m, word), [&](Game<P>& gg) { new_round_philox<P, POOL>(gg, rng, gid, PURPOSE_REFILL); });
+        advance<P, POOL>(g, opponent_pick<P, POOL, GREEDY>(g, m, word),
+                         [&](Game<P>& gg) { new_round_philox<P, POOL>(gg, rng, gid, PURPOSE_REFILL); });
     }
     Game<P> cp = g;
     count_score<P, POOL>(cp);
     return (int32_t)(cp.scf[0] & 0xFFFFu) - (int32_t)(cp.scf[1] & 0xFFFFu);
+}
+
+// GameRunner.step's opponent loop + reward with the greedy agent as the opponent (the loop rule and the return value of
+// opponent_random)
+template <int P, int POOL>
+AZB_HD int32_t opponent_greedy(Game<P>& g, const Philox& rng, uint32_t gid, bool require_two, uint32_t m[6])
+{
+    return opponent_random<P, POOL, true>(g, rng, gid, require_two, m);
 }
 
 }  // namespace azb

@@ -235,17 +235,31 @@ class BatchedAzul:
         """``GameRunner.step``'s opponent loop + reward for every game (K a14).  ``player_score`` (int16 [G]) is
         updated in place; returns dict(reward int16, done, status uint8[, mask][, obs bfloat16 [G, 32 + 52P]: the
         observation of the resulting state from seat 1's perspective])."""
+        return self._opponent(self.lib.azb_opponent_random, player_score, require_two, want_mask, want_obs)
+
+    def opponent_greedy(self, player_score, require_two=True, want_mask=True, want_obs=False):
+        """:meth:`opponent_random` with the greedy agent (``azb_greedy_action``) as the opponent."""
+        return self._opponent(self.lib.azb_opponent_greedy, player_score, require_two, want_mask, want_obs)
+
+    def _opponent(self, fn, player_score, require_two, want_mask, want_obs):
         n = self.n_games
         reward, done, status = self._new((n,), torch.int16), self._new((n,), torch.uint8), self._new((n,), torch.uint8)
         mask = self._new((MASK_WORDS, n), torch.int32) if want_mask else None
         obs = self._new((n, 32 + 52 * self.players), torch.bfloat16) if want_obs else None
-        _lib.check(self.lib.azb_opponent_random(self._h, _ptr(self.state), int(bool(require_two)), _ptr(player_score),
-                                               _ptr(reward), _ptr(done), _ptr(status), _ptr(mask), _ptr(obs), self._stream()))
+        _lib.check(fn(self._h, _ptr(self.state), int(bool(require_two)), _ptr(player_score), _ptr(reward), _ptr(done),
+                      _ptr(status), _ptr(mask), _ptr(obs), self._stream()))
         out = {"reward": reward, "done": done, "status": status}
         if want_mask:
             out["mask"] = mask
         if want_obs:
             out["obs"] = obs
+        return out
+
+    def greedy_action(self):
+        """The greedy agent's action for the seat to move in every game: uint8 [G] (``ACTION_SKIP`` when the game is over
+        or no action is legal).  The state is not touched."""
+        out = self._new((self.n_games,), torch.uint8)
+        _lib.check(self.lib.azb_greedy_action(self._h, _ptr(self.state), _ptr(out), self._stream()))
         return out
 
     # -- K4, persistent form ------------------------------------------------------------------
@@ -440,23 +454,29 @@ def runner_rollout(engine, packed, records, player_score, mode=0, out=None, oppo
     fused policy kernel, opponent loop + reward after each, decision records into ``records``.  The episodes must have
     been started (``BatchedGameRunner.reset``, or :meth:`selfplay.PersistentEpisodes.start` against a policy opponent).
 
-    ``opponent``: None plays the random opponent; a :class:`PackedPolicy` plays a frozen network with the same ``mode``
-    (``azb_policy_rollout_vs_policy``).  ``opp_passes`` (uint32 / int32 [1], optional, zeroed by the caller) then receives
-    the most opponent passes one decision needed."""
+    ``opponent``: None plays the random opponent; ``"greedy"`` the greedy agent (``azb_policy_rollout_vs_greedy``); a
+    :class:`PackedPolicy` plays a frozen network with the same ``mode`` (``azb_policy_rollout_vs_policy``).  ``opp_passes``
+    (uint32 / int32 [1], optional, zeroed by the caller) then receives the most opponent passes one decision needed."""
     r = records
+    mask, done, status = (_ptr(out["mask"]), _ptr(out["done"]), _ptr(out["status"])) if out else (None, None, None)
+    if isinstance(opponent, str):
+        assert opponent == "greedy", opponent
+        _lib.check(engine.lib.azb_policy_rollout_vs_greedy(
+            engine._h, _ptr(engine.state), _ptr(packed.buf), int(mode), r.k, _ptr(player_score), _ptr(r.meta), r.cap,
+            _ptr(r.state_rec), _ptr(r.action_rec), _ptr(r.logp_rec), _ptr(r.value_rec), _ptr(r.slot_rec), _ptr(r.reward_rec),
+            _ptr(r.flags_rec), ctypes.c_void_p(r.meta.data_ptr() + 4), None, None, None, mask, done, status, engine._stream()))
+        return
     if opponent is not None:
         _lib.check(engine.lib.azb_policy_rollout_vs_policy(
             engine._h, _ptr(engine.state), _ptr(packed.buf), _ptr(opponent.buf), int(mode), r.k, _ptr(player_score),
             _ptr(r.meta), r.cap, _ptr(r.state_rec), _ptr(r.action_rec), _ptr(r.logp_rec), _ptr(r.value_rec), _ptr(r.slot_rec),
             _ptr(r.reward_rec), _ptr(r.flags_rec), ctypes.c_void_p(r.meta.data_ptr() + 4), _ptr(opp_passes),
-            _ptr(out["mask"]) if out else None, _ptr(out["done"]) if out else None, _ptr(out["status"]) if out else None,
-            engine._stream()))
+            mask, done, status, engine._stream()))
         return
     _lib.check(engine.lib.azb_policy_rollout(
         engine._h, _ptr(engine.state), _ptr(packed.buf), int(mode), r.k, 1, _ptr(player_score), _ptr(r.meta), r.cap,
         _ptr(r.state_rec), _ptr(r.action_rec), _ptr(r.logp_rec), _ptr(r.value_rec), _ptr(r.slot_rec), _ptr(r.reward_rec),
-        _ptr(r.flags_rec), ctypes.c_void_p(r.meta.data_ptr() + 4), None, None, None,
-        _ptr(out["mask"]) if out else None, _ptr(out["done"]) if out else None, _ptr(out["status"]) if out else None,
+        _ptr(r.flags_rec), ctypes.c_void_p(r.meta.data_ptr() + 4), None, None, None, mask, done, status,
         None, engine._stream()))
 
 

@@ -2,27 +2,30 @@
 
 ``BatchedGameRunner`` is G copies of the reference's 2-player env wrapper advancing in lock-step on one
 GPU: seat 1 is the learning agent, seat 2 a random agent (``RandomAgent``, game_runner.py:87-97, drawing
-from the Philox schedule) or a frozen network.  ``PersistentEpisodes`` plays whole episodes in one launch of
-the fused policy kernel; that is how the trainer plays.  ``run_episodes`` is the step-wise loop the persistent
+from the Philox schedule), the greedy agent (``azb_greedy_action``: the best one-move score) or a frozen network.
+``PersistentEpisodes`` plays whole episodes in one launch of the fused policy kernel; that is how the trainer plays.  ``run_episodes`` is the step-wise loop the persistent
 kernel is checked against: one agent decision costs up to three launches, the observation
 (``azb_observe_bf16``, only when the caller records it), the fused policy kernel (``azb_policy_step``: MLP on
 tcgen05 + masked softmax + sampling + the agent's ``Azul.step``) and the opponent loop + reward
-(``azb_opponent_random``).
+(``azb_opponent_random`` / ``azb_opponent_greedy``).
 """
 import os
 
 import torch
 
-from .engine import (BatchedAzul, EpisodeRecords, discounted_returns_records, mask_to_bool, policy_step, rules_to_ints,
-                     runner_rollout)
+from .engine import (BatchedAzul, EpisodeRecords, PackedPolicy, discounted_returns_records, mask_to_bool, policy_step,
+                     rules_to_ints, runner_rollout)
 
 DEFAULT_RULES = {"first_player": "Random", "tile_pool": "Lid"}      # game_runner.py:23
+GREEDY = "greedy"                   # the opponent keyword of the greedy agent
 
 
 class BatchedGameRunner:
     def __init__(self, n_games, rules=None, seed=0, device=0, game_id_base=0, opponent=None, opponent_mode=0):
-        """``opponent``: None = RandomAgent (game_runner.py:29-30) or a ``PackedPolicy`` = a frozen ``Agent``
-        (scripts/run_batch.py:6-8) whose moves come from the fused policy kernel."""
+        """``opponent``: None = RandomAgent (game_runner.py:29-30), ``"greedy"`` = the greedy agent, or a ``PackedPolicy`` =
+        a frozen ``Agent`` (scripts/run_batch.py:6-8) whose moves come from the fused policy kernel."""
+        if isinstance(opponent, str) and opponent != GREEDY:
+            raise ValueError("unknown opponent %r: None (random), %r or a PackedPolicy" % (opponent, GREEDY))
         self.opponent, self.opponent_mode = opponent, opponent_mode
         rules = DEFAULT_RULES if rules is None else rules
         pool, first = rules_to_ints(2, rules)
@@ -36,9 +39,7 @@ class BatchedGameRunner:
         """``GameRunner.reset`` (game_runner.py:76-85): fresh games, the opponent plays until seat 1 is to move."""
         self.engine.reset()
         self.player_score.zero_()
-        if self.opponent is not None:                 # a fresh board always offers seat 1 >= 2 actions, so the
-            self._opponent_policy_moves()             # ":46" and ":84" loop conditions coincide here
-        out = self.engine.opponent_random(self.player_score, require_two=False)
+        out = self._opponent_moves(require_two=False)
         self.player_score.zero_()                     # game_runner.py:81: the score baseline restarts at 0
         self.mask = out["mask"]
         return out
@@ -64,10 +65,16 @@ class BatchedGameRunner:
         if bool((out["action"] != 255).any()):
             raise RuntimeError("opponent loop did not hand the move back to seat 1 within %d policy launches" % max_rounds)
 
+    def _opponent_moves(self, require_two):
+        """The opponent loop + reward (game_runner.py:46-52; :84-85 without ``require_two``)."""
+        if self.opponent == GREEDY:
+            return self.engine.opponent_greedy(self.player_score, require_two=require_two)
+        if self.opponent is not None:                 # a fresh board always offers seat 1 >= 2 actions, so the
+            self._opponent_policy_moves()             # ":46" and ":84" loop conditions coincide in reset
+        return self.engine.opponent_random(self.player_score, require_two=require_two)
+
     def _after_agent_move(self):
-        if self.opponent is not None:
-            self._opponent_policy_moves()
-        out = self.engine.opponent_random(self.player_score, require_two=True)
+        out = self._opponent_moves(require_two=True)
         self.mask = out["mask"]
         return out
 
@@ -163,9 +170,9 @@ class PersistentEpisodes:
     decisions are those of :func:`run_episodes` (same Philox schedule); only their storage differs (compact slots in
     arbitrary order instead of [T, G]).
 
-    The opponent is the runner's: the random agent (``runner.opponent`` None) or a frozen network (a ``PackedPolicy``,
-    ``GameRunner(opponent=Agent(...))``), which then plays with the same selection mode as the agent.  Nothing in
-    :meth:`run` waits for the GPU, so a whole batch can be captured in a CUDA graph."""
+    The opponent is the runner's: the random agent (``runner.opponent`` None), the greedy agent (``"greedy"``) or a frozen
+    network (a ``PackedPolicy``, ``GameRunner(opponent=Agent(...))``), which then plays with the same selection mode as the
+    agent.  Nothing in :meth:`run` waits for the GPU, so a whole batch can be captured in a CUDA graph."""
 
     def __init__(self, runner, packed, max_decisions=160, capacity=None, want_logp_value=False):
         self.runner, self.packed = runner, packed
@@ -184,7 +191,7 @@ class PersistentEpisodes:
         ``BatchedGameRunner.reset``: on a fresh board the opponent moves at most once before seat 1 is to move with >= 2
         legal actions, so ONE opponent launch replaces its loop; the resulting state is the same."""
         runner = self.runner
-        if runner.opponent is None:
+        if not isinstance(runner.opponent, PackedPolicy):        # the random or the greedy agent: no host reads
             return runner.reset()
         e = runner.engine
         e.reset()
@@ -197,16 +204,17 @@ class PersistentEpisodes:
 
     def run(self, gamma=0.99, mode=0):
         opponent = self.runner.opponent
-        if opponent is not None and self.runner.opponent_mode != mode:
+        policy = isinstance(opponent, PackedPolicy)
+        if policy and self.runner.opponent_mode != mode:
             raise ValueError("the persistent rollout plays both seats with one selection mode: agent mode %d, opponent mode %d"
                              % (mode, self.runner.opponent_mode))
         r = self.records
         self.start(mode)
         r.clear()
-        if opponent is not None:
+        if policy:
             self.opp_passes.zero_()
         runner_rollout(self.runner.engine, self.packed, r, self.runner.player_score, mode=mode, out=self.out,
-                       opponent=opponent, opp_passes=self.opp_passes if opponent is not None else None)
+                       opponent=opponent, opp_passes=self.opp_passes if policy else None)
         discounted_returns_records(self.runner.engine, r, gamma)
         self.runner.mask = self.out["mask"]
         return r
@@ -226,6 +234,15 @@ def load_network(net, device=None):
     elif not isinstance(net, torch.nn.Module):
         raise TypeError("expected an ActorCritic, a state_dict or a file path, got %r" % type(net).__name__)
     return net.to(device) if device is not None else net
+
+
+def resolve_opponent(engine, opponent, device=None):
+    """The runner's opponent for an opponent choice: None (the random agent) stays None, ``"greedy"`` selects the greedy
+    agent (a checkpoint file of that name is passed as ``./greedy``), anything else is a network (``load_network``) packed
+    for the policy kernel of ``engine``."""
+    if opponent is None or (isinstance(opponent, str) and opponent == GREEDY):
+        return opponent
+    return PackedPolicy(engine, load_network(opponent, device))
 
 
 def discounted_returns(reward, active, gamma):

@@ -2,7 +2,7 @@
 equivalent (reference scripts/training.py:8-22, nn_runner.py:53-84, agent.py:39-62).
 
     python -m azul_deep_reinforcement_learning_b200.train [batch_size] [net_name] [--batches N]
-                                                      [--opponent FILE] [--opponent-refresh N]
+                                                      [--opponent FILE|greedy] [--opponent-refresh N]
     torchrun --nproc-per-node 8 -m azul_deep_reinforcement_learning_b200.train 1024 run1
 
 ``batch_size`` episodes are played IN PARALLEL per rank (one game slot each) instead of one after the
@@ -25,7 +25,7 @@ import torch.distributed as dist
 from . import parallel
 from .azulnet.model import ActorCritic
 from .engine import PackedPolicy, UpdateGradients, train_stats
-from .selfplay import BatchedGameRunner, PersistentEpisodes, load_network
+from .selfplay import GREEDY, BatchedGameRunner, PersistentEpisodes, resolve_opponent
 
 ACTOR_COEFF, CRITIC_COEFF, ENTROPY_COEFF = 1.0, 0.5, 0.1          # agent.py:47-49
 
@@ -110,9 +110,9 @@ class SelfPlayTrainer:
     :meth:`update_states` (the tensor-core kernels) run one ``Agent.update`` on explicitly given decisions: the entry points
     the tests hold against the reference.
 
-    ``opponent``: None plays the random agent (``RandomAgent``); an ``ActorCritic``, a ``state_dict`` or a file path
-    (anything ``Agent(base_net_file=...)`` loads) plays a frozen network in seat 2 (``GameRunner(opponent=Agent(...))``),
-    sampling like the agent.  ``opponent_refresh`` = N > 0: the opponent's weights are replaced by the current network's
+    ``opponent``: None plays the random agent (``RandomAgent``); ``"greedy"`` the greedy agent (the best one-move score, a
+    fixed-strength yardstick); an ``ActorCritic``, a ``state_dict`` or a file path (anything ``Agent(base_net_file=...)``
+    loads) plays a frozen network in seat 2 (``GameRunner(opponent=Agent(...))``), sampling like the agent.  ``opponent_refresh`` = N > 0: the opponent's weights are replaced by the current network's
     after every N batches -- self-play against a lagged copy of itself."""
 
     def __init__(self, games_per_rank=1024, learning_rate=3e-4, gamma=0.99, seed=0, device=0, rank=0, world=1,
@@ -128,12 +128,15 @@ class SelfPlayTrainer:
                                         game_id_base=parallel.shard(rank, games_per_rank))
         self.packed = PackedPolicy(self.runner.engine, self.net)
         self.opponent, self.opponent_refresh, self.batches_done = None, int(opponent_refresh), 0
+        is_greedy = isinstance(opponent, str) and opponent == GREEDY
+        if opponent_refresh and is_greedy:
+            raise ValueError("opponent_refresh replaces a network opponent: the greedy agent has no weights")
         if opponent_refresh and opponent is None:
             opponent = self.net                              # a lagged copy of the network itself
-        if opponent is not None:
-            # packed once into its own fixed buffer: a captured batch reads it there, a refresh re-packs it in place
-            self.opponent = PackedPolicy(self.runner.engine, load_network(opponent, self.device))
-            self.runner.opponent, self.runner.opponent_mode = self.opponent, 0
+        # a network is packed once into its own fixed buffer: a captured batch reads it there, a refresh re-packs it in place
+        self.runner.opponent, self.runner.opponent_mode = resolve_opponent(self.runner.engine, opponent, self.device), 0
+        if isinstance(self.runner.opponent, PackedPolicy):
+            self.opponent = self.runner.opponent
         self.episodes = PersistentEpisodes(self.runner, self.packed, max_decisions=max_decisions)
         # every parameter gradient is a view into ONE flat fp32 buffer (PARAM_ORDER): the tensor-core kernels add into
         # it, autograd accumulates into the views in place, and the gradient all-reduce is a single collective on it
@@ -362,15 +365,18 @@ def parse_args(argv=None):
                     help="continue from a checkpoint written by this script (<net_name>.pt) or start from any saved "
                          "network Agent(base_net_file=...) accepts")
     ap.add_argument("--checkpoint-every", type=int, default=1000)
-    ap.add_argument("--opponent", default=None, metavar="FILE",
-                    help="play seat 2 with this frozen network (any file Agent(base_net_file=...) accepts) instead of "
-                         "the random agent")
+    ap.add_argument("--opponent", default=None, metavar="FILE|greedy",
+                    help="play seat 2 with this frozen network (any file Agent(base_net_file=...) accepts), or with the "
+                         "greedy agent ('greedy': the move with the best one-move score), instead of the random agent; "
+                         "pass a network file named greedy as ./greedy")
     ap.add_argument("--opponent-refresh", type=int, default=0, metavar="N",
                     help="replace the opponent by the current network after every N batches (self-play against a lagged "
                          "copy; without --opponent it starts as the initial network)")
     args = ap.parse_args(argv)
     if args.opponent_refresh < 0:
         ap.error("--opponent-refresh must be >= 0")
+    if args.opponent == GREEDY and args.opponent_refresh:
+        ap.error("--opponent-refresh replaces a network opponent: it does not apply to --opponent greedy")
     return args
 
 

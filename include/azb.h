@@ -152,6 +152,18 @@ int azb_round_flags(azb_t* h, const uint32_t* state, uint8_t* flags, void* strea
 int azb_opponent_random(azb_t* h, uint32_t* state, int require_two, int16_t* player_score, int16_t* reward_out,
                         uint8_t* done_out, uint8_t* status_out, uint32_t* mask6_out, void* obs_bf16_out, void* stream);
 
+/* The greedy agent (no counterpart in the reference; DESIGN.md "Greedy agent"): for the seat to move, the legal action
+ * whose move followed by count_score on a copy leaves the mover's score highest -- without the clamp at zero of
+ * azul.py:294-295 -- ties broken by the random agent's Philox word of that env step over the tied actions in ascending
+ * action index.  Deterministic given (seed, game id, step count), like every agent here.
+ *   azb_greedy_action    uint8 [G]: the greedy agent's action in every game (AZB_ACTION_SKIP when the game is over or no
+ *                        action is legal); the state is not touched.
+ *   azb_opponent_greedy  azb_opponent_random with the greedy agent as the opponent: the same arguments, loop rule
+ *                        (require_two), reward, outputs and optional bf16 observation. */
+int azb_greedy_action(azb_t* h, const uint32_t* state, uint8_t* action_out, void* stream);
+int azb_opponent_greedy(azb_t* h, uint32_t* state, int require_two, int16_t* player_score, int16_t* reward_out,
+                        uint8_t* done_out, uint8_t* status_out, uint32_t* mask6_out, void* obs_bf16_out, void* stream);
+
 /* ---- K4: the policy/value network of azulnet/model.py:12-41 fused with its callers ------------
  * ActorCritic(136, 180, hidden 180): actor 136 -> 180 -> ReLU -> 180 logits, critic 136 -> 180 -> ReLU -> 1.
  * azb_policy_pack_weights converts the eight fp32 parameter tensors (torch layout [out][in], device
@@ -223,6 +235,18 @@ int azb_policy_rollout_vs_policy(azb_t* h, uint32_t* state, const void* packed, 
                                  int32_t* slot_rec, int16_t* reward_rec, uint8_t* flags_rec, uint32_t* steps_used,
                                  uint32_t* opp_passes, uint32_t* mask6_out, uint8_t* done_out, uint8_t* status_out,
                                  void* stream);
+
+/* ---- K4, persistent runner mode against the greedy agent: azb_policy_rollout's runner mode (the same records, outputs and
+ * checks; always runner mode, no counters) with azb_greedy_action's agent as the opponent in place of the random agent:
+ * after each agent decision the greedy agent moves until seat 1 is to move with >= 2 legal actions or the game is over, then
+ * the reward.  The decisions equal those of azb_policy_step(apply_step = 1) followed by azb_opponent_greedy(require_two = 1).
+ * The caller starts the episodes with azb_reset + azb_opponent_greedy(require_two = 0) and zeroes player_score; no host
+ * synchronisation is needed. */
+int azb_policy_rollout_vs_greedy(azb_t* h, uint32_t* state, const void* packed, int mode, int k_decisions,
+                                 int16_t* player_score, uint32_t* n_dec, int64_t rec_cap, uint32_t* state_rec,
+                                 uint8_t* action_rec, float* logp_rec, float* value_rec, int32_t* slot_rec, int16_t* reward_rec,
+                                 uint8_t* flags_rec, uint32_t* steps_used, uint8_t* action_out, float* logp_out,
+                                 float* value_out, uint32_t* mask6_out, uint8_t* done_out, uint8_t* status_out, void* stream);
 
 /* Discounted returns of NNRunner.train (nn_runner.py:72-75) over the records of azb_policy_rollout's runner mode:
  * q_t = r_t + gamma * q_{t+1} over each game's decisions (accumulated in double like the reference's numpy loop), written

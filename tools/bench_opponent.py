@@ -1,10 +1,12 @@
-"""Whole-episode rollouts against the random opponent and against a frozen policy opponent, timed with CUDA events.
+"""Whole-episode rollouts against the random opponent, a frozen policy opponent and the greedy agent, timed with CUDA events.
 
     python tools/bench_opponent.py [--games 16384 131072] [--reps 5] [--out FILE]
 
 Per batch size: (a) the persistent runner-mode rollout vs the random opponent, (b) the persistent rollout vs a policy
 opponent (azb_policy_rollout_vs_policy), (c) the eager run_episodes vs the same policy opponent (one policy launch per
-agent decision, one or more opponent launches each followed by a host read, one reward launch).  A timed batch is a whole
+agent decision, one or more opponent launches each followed by a host read, one reward launch), (d) the persistent rollout
+vs the greedy agent (azb_policy_rollout_vs_greedy), (e) the eager run_episodes vs the greedy agent (one policy launch and
+one azb_opponent_greedy launch per agent decision, a host read every 8 decisions).  A timed batch is a whole
 PersistentEpisodes.run (episode start, the rollout, discounted returns) or a whole run_episodes, after one warm-up batch.
 Reported: ms per batch, episodes/s, agent decisions/s, and the opponent passes per agent decision -- the most any CTA
 needed in one decision (the kernel's counter) and, from a separate counting run of the eager path, the mean and maximum
@@ -97,7 +99,19 @@ def bench(n, reps):
     passes = count_eager_passes(rc, pc)
     res["c_eager_vs_policy"]["opponent_passes_per_decision_batch_mean"] = sum(passes) / max(len(passes), 1)
     res["c_eager_vs_policy"]["opponent_passes_per_decision_batch_max"] = max(passes) if passes else 0
+
+    rd = BatchedGameRunner(n, seed=11, opponent="greedy")
+    ed = PersistentEpisodes(rd, PackedPolicy(rd.engine, net))
+    ms, r = timed(lambda: ed.run(), reps)
+    res["d_persistent_vs_greedy"] = _rates(n, ms, int(r.meta[0]))
+
+    re_ = BatchedGameRunner(n, seed=11, opponent="greedy")
+    pe = PackedPolicy(re_.engine, net)
+    ms, batch = timed(lambda: run_episodes(re_, pe, max_decisions=160, record_obs=False), max(2, reps // 2))
+    res["e_eager_vs_greedy"] = _rates(n, ms, int(batch["active"].sum()))
     res["b_over_a"] = res["b_persistent_vs_policy"]["ms"] / res["a_persistent_vs_random"]["ms"]
+    res["d_over_a"] = res["d_persistent_vs_greedy"]["ms"] / res["a_persistent_vs_random"]["ms"]
+    res["e_over_d"] = res["e_eager_vs_greedy"]["ms"] / res["d_persistent_vs_greedy"]["ms"]
     res["c_over_b"] = res["c_eager_vs_policy"]["ms"] / res["b_persistent_vs_policy"]["ms"]
     return res
 
