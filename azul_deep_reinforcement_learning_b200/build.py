@@ -11,7 +11,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libazb.so")
 SOURCES = [os.path.join(CSRC, "azb.cu"), os.path.join(CSRC, "azb_policy.cu"), os.path.join(CSRC, "azb_a2c.cu"), os.path.join(CSRC, "azb_update.cu"), os.path.join(CSRC, "azb_variant.cu")]
-HEADERS = [os.path.join(CSRC, "azb_rules.cuh"), os.path.join(CSRC, "azb_tc.cuh"), os.path.join(CSRC, "azb_variant.cuh"), os.path.join(CSRC, "azb_internal.h"), os.path.join(CSRC, "azb_queue.cuh"), os.path.join(os.path.dirname(PKG_DIR), "include", "azb.h")]
+HEADERS = [os.path.join(CSRC, "azb_rules.cuh"), os.path.join(CSRC, "azb_tc.cuh"), os.path.join(CSRC, "azb_mbar.cuh"), os.path.join(CSRC, "azb_variant.cuh"), os.path.join(CSRC, "azb_internal.h"), os.path.join(CSRC, "azb_queue.cuh"), os.path.join(os.path.dirname(PKG_DIR), "include", "azb.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",   # B200 only: no other arch, no PTX fallback

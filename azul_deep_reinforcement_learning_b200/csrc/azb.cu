@@ -12,6 +12,7 @@
 #include <string.h>
 
 #include "azb_internal.h"
+#include "azb_mbar.cuh"
 #include "azb_rules.cuh"
 #include "azb_queue.cuh"
 
@@ -387,39 +388,73 @@ __global__ void __launch_bounds__(32 * STEP_WARPS, STEP_MINBLOCKS) k_step(Launch
 }
 
 // K1+K2+K3+K6 fused: k_steps random-agent env steps per game in one launch
+// The rollout counters of a block: every warp owns a row of AZB_N_COUNTERS partials in shared memory that only its own lanes
+// write, with plain 64-bit adds (sm_100a has no 64-bit shared-memory add: an atomic one is a compare-and-swap loop); the
+// block sums the rows once at the end (counters_out).  Which warp's row a batch's statistics land in does not matter.
 struct BlockSink {
-    unsigned long long* c;             // the block's counters in shared memory
+    unsigned long long (*part)[AZB_N_COUNTERS];   // the block's partials in shared memory, [warp][counter]
     uint32_t r[AZB_N_COUNTERS];        // this lane's share of the game statistics since the last flush
     uint32_t passes;
-    __device__ __forceinline__ explicit BlockSink(unsigned long long* shared) : c(shared), passes(0u)
+    __device__ __forceinline__ explicit BlockSink(unsigned long long (*shared)[AZB_N_COUNTERS]) : part(shared), passes(0u)
     {
 #pragma unroll
         for (int i = 0; i < AZB_N_COUNTERS; i++) r[i] = 0u;
     }
-    // rare events and the per-launch totals: straight to the block's counters
+    // whole warp, once per rollout_steps call: its steps and rounds.  One call can give a lane up to 2^31 - 1 steps, so a
+    // 32-bit sum over the warp could overflow: the sum is taken in 64 bits from the two 16-bit halves
     __device__ __forceinline__ void add(int i, uint32_t v)
     {
-        if (v) atomicAdd(&c[i], (unsigned long long)v);
+        const uint32_t lo = __reduce_add_sync(0xFFFFFFFFu, v & 0xFFFFu), hi = __reduce_add_sync(0xFFFFFFFFu, v >> 16);
+        if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5][i] += ((unsigned long long)hi << 16) + lo;
     }
-    // the statistics of finished games: a register add per counter.  (One REDUX + one 64-bit shared atomic per counter
-    // and end-of-round pass cost 17 instructions per env step and 5 % of the kernel's stall samples.)
-    __device__ __forceinline__ void add_group(int i, uint32_t v) { r[i] += v; }
+    // the statistics of finished games and the rare events: a register add per counter.  (One REDUX + one 64-bit shared atomic
+    // per counter and end-of-round pass cost 17 instructions per env step and 5 % of the kernel's stall samples.)  Counters 6
+    // (stuck round) and 7 (empty bag) ride in the high halves of counters 1 (games finished) and 5 (games seat 0 won): each of the
+    // four grows by at most 1 per lane and pass, so a half holds a warp's sum over 256 passes, and 6 and 7 take no registers of
+    // their own across the light step (two more cost a resident block per SM at 128 threads).
+    __device__ __forceinline__ void add_group(int i, uint32_t v)
+    {
+        if (i == 6) r[1] += v << 16;
+        else if (i == 7) r[5] += v << 16;
+        else r[i] += v;
+    }
     // whole warp, after every end-of-round pass: flush before a 32-bit warp sum could overflow (a pass adds at most
     // 4 * 65,535 per lane: 256 passes * 32 lanes stay below 2^32)
     __device__ __forceinline__ void pass_done()
     {
         if ((++passes & 255u) == 0u) flush();
     }
+    // whole warp: lane i adds the warp's total of counter i to its partial (one shared-memory add per lane, not 16 on lane 0)
     __device__ __forceinline__ void flush()
     {
+        const int lane = threadIdx.x & 31;
+        uint32_t mine = 0u;
 #pragma unroll
         for (int i = 0; i < AZB_N_COUNTERS; i++) {
+            if (i == 6 || i == 7) continue;
             const uint32_t tot = __reduce_add_sync(0xFFFFFFFFu, r[i]);
-            if (tot && (threadIdx.x & 31) == 0) atomicAdd(&c[i], (unsigned long long)tot);
+            if (i == 1 || i == 5) {
+                mine = lane == i ? (tot & 0xFFFFu) : mine;
+                mine = lane == (i == 1 ? 6 : 7) ? (tot >> 16) : mine;
+            } else {
+                mine = lane == i ? tot : mine;
+            }
             r[i] = 0u;
         }
+        if (lane < AZB_N_COUNTERS) part[threadIdx.x >> 5][lane] += mine;
     }
 };
+
+// whole block, after every warp's last flush: the sum of the warps' partials, added to the caller's uint64[AZB_N_COUNTERS]
+__device__ __forceinline__ void counters_out(const unsigned long long (*part)[AZB_N_COUNTERS], unsigned long long* counters)
+{
+    __syncthreads();
+    if (counters && threadIdx.x < AZB_N_COUNTERS) {
+        unsigned long long s = 0ull;
+        for (int w = 0; w < (int)(blockDim.x >> 5); w++) s += part[w][threadIdx.x];
+        if (s) atomicAdd(&counters[threadIdx.x], s);
+    }
+}
 
 // Action words of a whole round, computed by the full warp during the end-of-round pass (when all of its games
 // are at the same point) and parked in shared memory: ROUND_WORDS words per game, [word][thread] so that a warp
@@ -463,8 +498,8 @@ __global__ void k_rollout_random(Launch L, int k_steps, int defer, uint32_t* __r
                                  unsigned long long* __restrict__ counters)
 {
     extern __shared__ uint32_t round_words[];          // [ROUND_WORDS][blockDim.x]
-    __shared__ unsigned long long cnt[AZB_N_COUNTERS];
-    if (threadIdx.x < AZB_N_COUNTERS) cnt[threadIdx.x] = 0ull;
+    __shared__ unsigned long long cnt[32][AZB_N_COUNTERS];   // per-warp counter partials (BlockSink)
+    if ((threadIdx.x & 31) < AZB_N_COUNTERS) cnt[threadIdx.x >> 5][threadIdx.x & 31] = 0ull;
     __syncthreads();
     const int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     const bool valid = g < L.n;
@@ -486,8 +521,7 @@ __global__ void k_rollout_random(Launch L, int k_steps, int defer, uint32_t* __r
             store_mask(mask6_out, L.n, g, m);
         }
     }
-    __syncthreads();
-    if (counters && threadIdx.x < AZB_N_COUNTERS && cnt[threadIdx.x]) atomicAdd(&counters[threadIdx.x], cnt[threadIdx.x]);
+    counters_out(cnt, counters);
 }
 
 // ---- k_rollout_rotate: the same rollout with the 32-game batches ROTATING through the warps of the block ----
@@ -499,6 +533,10 @@ __global__ void k_rollout_random(Launch L, int k_steps, int defer, uint32_t* __r
 // (packed states, steps left) in that warp's shared-memory slot and becomes idle itself.  The two idle slots travel backwards
 // round the ring, the batches forwards: every batch spends its time on fuller and emptier schedulers alike, and so does
 // every scheduler.  Results cannot depend on it: a game's trajectory depends on its id and step counter only.
+// An idle warp waits on its own mbarrier (arrival count 1), suspended in hardware: a polling loop cost 5 % of the kernel's issue
+// slots.  Each barrier phase completes with exactly one arrival: the predecessor's after it parked a batch in the slot, or, once,
+// the termination arrival of the warp that finishes the block's last batch.  At that moment no batch is left anywhere, so every
+// other warp is idle with its last hand-over already taken in, and gets exactly one arrival for its last wait.
 __device__ __forceinline__ uint32_t ld_shared_volatile(const uint32_t* p) { return *reinterpret_cast<const volatile uint32_t*>(p); }
 __device__ __forceinline__ void st_shared_volatile(uint32_t* p, uint32_t v) { *reinterpret_cast<volatile uint32_t*>(p) = v; }
 
@@ -509,17 +547,20 @@ __global__ void __launch_bounds__(512) k_rollout_rotate(Launch L, int k_steps, i
 {
     constexpr int W = Game<P>::WORDS;
     extern __shared__ uint32_t rot_smem[];             // [ROUND_WORDS][blockDim.x] action words, then [warps][W + 1][32] parked batches
-    __shared__ unsigned long long cnt[AZB_N_COUNTERS];
+    __shared__ unsigned long long cnt[16][AZB_N_COUNTERS];   // per-warp counter partials (BlockSink)
+    __shared__ unsigned long long wake[16];            // per-warp mbarrier: a batch was parked in the slot, or every batch has finished
     __shared__ uint32_t slot_state[16];                // 0 playing, 1 idle, 3 a batch is parked in this warp's slot
     __shared__ uint32_t slot_batch[16];
     __shared__ uint32_t n_done;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = (int)(blockDim.x >> 5);
     uint32_t* park = rot_smem + ROUND_WORDS * blockDim.x;
+    const uint32_t wake0 = (uint32_t)__cvta_generic_to_shared(wake);
     const int64_t block_g0 = blockIdx.x * (int64_t)(32 * batches_per_block);
     const int64_t games_here = L.n - block_g0 < 32 * batches_per_block ? L.n - block_g0 : 32 * batches_per_block;
     const uint32_t n_batches = (uint32_t)((games_here + 31) / 32);
-    if (threadIdx.x < AZB_N_COUNTERS) cnt[threadIdx.x] = 0ull;
+    if (lane < AZB_N_COUNTERS) cnt[warp][lane] = 0ull;
     if (threadIdx.x < 16) slot_state[threadIdx.x] = (uint32_t)threadIdx.x < n_batches ? 0u : 1u;
+    if (threadIdx.x < warps) mbar_init(wake0 + 8u * threadIdx.x, 1u);
     if (threadIdx.x == 0) n_done = 0u;
     __syncthreads();
     const Philox rng{L.k0, L.k1};
@@ -536,6 +577,7 @@ __global__ void __launch_bounds__(512) k_rollout_rotate(Launch L, int k_steps, i
     int64_t gl = g < L.n ? g : L.n - 1;
     if (have) { gm.load(L.state, L.n, gl); remaining = valid ? k_steps : 0; }
     const int succ = warp + 1 == warps ? 0 : warp + 1;
+    uint32_t parity = 0u;                              // of the phase of this warp's barrier that the next wait completes
     for (;;) {
         if (have) {
             remaining = rollout_steps<P, POOL, true>(gm, rng, L.gid0 + (uint32_t)gl, L.first_rule, remaining, sink, WarpLanes{}, valid, defer,
@@ -550,8 +592,12 @@ __global__ void __launch_bounds__(512) k_rollout_rotate(Launch L, int k_steps, i
                     }
                 }
                 have = false;
-                __syncwarp();
-                if (lane == 0) { atomicAdd(&n_done, 1u); __threadfence_block(); st_shared_volatile(&slot_state[warp], 1u); }
+                uint32_t last = 0u;
+                if (lane == 0) { last = atomicAdd(&n_done, 1u) == n_batches - 1u; st_shared_volatile(&slot_state[warp], 1u); }
+                if (__shfl_sync(0xFFFFFFFFu, last, 0)) {                      // the block's last batch: wake every other warp to exit
+                    if (lane < warps && lane != warp) mbar_arrive(wake0 + 8u * lane);
+                    break;
+                }
             } else if (ld_shared_volatile(&slot_state[succ]) == 1u) {         // the next warp is idle: the batch moves on
                 uint32_t* dst = park + (size_t)succ * (W + 1) * 32;
                 gm.store(dst, 32, lane);
@@ -560,21 +606,16 @@ __global__ void __launch_bounds__(512) k_rollout_rotate(Launch L, int k_steps, i
                 __threadfence_block();
                 __syncwarp();
                 have = false;
-                if (lane == 0) { st_shared_volatile(&slot_state[succ], 3u); st_shared_volatile(&slot_state[warp], 1u); }
-            }
-        } else {
-            uint32_t s = 0u;
-            if (lane == 0) {
-                for (;;) {
-                    s = ld_shared_volatile(&slot_state[warp]);
-                    if (s == 3u) break;
-                    if (ld_shared_volatile(&n_done) >= n_batches) break;      // every batch has finished: none can arrive
-                    __nanosleep(400);
+                if (lane == 0) {
+                    st_shared_volatile(&slot_state[succ], 3u);
+                    st_shared_volatile(&slot_state[warp], 1u);
+                    mbar_arrive(wake0 + 8u * succ);                           // release: the parked batch is visible to succ
                 }
             }
-            s = __shfl_sync(0xFFFFFFFFu, s, 0);
-            if (s != 3u) break;
-            __threadfence_block();
+        } else {
+            mbar_wait(wake0 + 8u * warp, parity);                             // every lane waits, and so acquires
+            parity ^= 1u;
+            if (ld_shared_volatile(&slot_state[warp]) != 3u) break;           // the termination arrival
             const uint32_t* src = park + (size_t)warp * (W + 1) * 32;
             gm.load(src, 32, lane);
             remaining = (int)src[W * 32 + lane];
@@ -588,8 +629,7 @@ __global__ void __launch_bounds__(512) k_rollout_rotate(Launch L, int k_steps, i
         }
     }
     sink.flush();
-    __syncthreads();
-    if (counters && threadIdx.x < AZB_N_COUNTERS && cnt[threadIdx.x]) atomicAdd(&counters[threadIdx.x], cnt[threadIdx.x]);
+    counters_out(cnt, counters);
 }
 
 // K5: score preview on a copy

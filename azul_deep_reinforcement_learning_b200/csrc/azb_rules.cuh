@@ -934,10 +934,11 @@ AZB_HD void export_record(const Game<P>& g, Wr wr)
 // 3 sum score seat 0, 4 sum score seat 1, 5 games seat 0 won, 6 stuck aborts, 7 games that ran the
 // bag empty, 8 sum turn_counter, 9 sum -floor_penalty seat 0, 10 sum max_combo seat 0, 11 completed
 // rows, 12 completed columns, 13 completed colours (seat 0), 14 sum first_player_stats seat 0,
-// 15 sum of all seats' scores.  Sink::add(index, value) receives the increments.
-// `fin` selects the games of the calling group that just ended; Sink::add_group may aggregate the
-// increments of all calling lanes (the rollout kernel keeps them in registers and reduces them with one REDUX per
-// counter and warp every 256 end-of-round passes: Sink::pass_done() is called by the whole group after each pass).
+// 15 sum of all seats' scores.  Sink::add_group(index, value) receives a lane's increments and may aggregate
+// those of all lanes (the rollout kernel keeps them in registers and reduces them with one REDUX per counter and warp
+// every 256 end-of-round passes: Sink::pass_done() is called by the whole group after each pass); rollout_steps
+// hands its per-call totals of steps and rounds to Sink::add(index, value), called by the whole group.
+// `fin` selects the games of the calling group that just ended.
 template <class GT, typename Sink>
 AZB_HD void tally_finished(const GT& g, Sink& sink, bool fin = true)
 {
@@ -1020,7 +1021,7 @@ AZB_HD int rollout_steps(Game<P>& g, const Philox& rng, uint32_t gid, int first_
             uint32_t m[6];
             legal_mask_open(g, open, m);
             if (m[0] == 0u) {                                         // words 1..5 are subsets of word 0 (the floor takes any source)
-                sink.add(6, 1);                                       // stuck round (SURVEY §5): abort the game
+                sink.add_group(6, 1);                                 // stuck round (SURVEY §5): abort the game
                 phase = 2;
             } else {
                 uint32_t mp, mb;
@@ -1061,7 +1062,7 @@ AZB_HD int rollout_steps(Game<P>& g, const Philox& rng, uint32_t gid, int first_
                 }
                 const uint32_t bag_before = g.status() & ST_BAG_EMPTY;
                 new_round_philox<P, POOL>(g, rng, gid, purpose);      // azul.py:311 / game_runner.py:80
-                if (!bag_before && (g.status() & ST_BAG_EMPTY)) sink.add(7, 1);
+                if (!bag_before && (g.status() & ST_BAG_EMPTY)) sink.add_group(7, 1);
 #pragma unroll
                 for (int p = 0; p < P; p++) open[p] = open_rows(g, p);   // scoring emptied lines and filled the wall
                 words.prefetch(rng, gid, g.steps);                    // the whole warp is here: words for the next round
@@ -1072,7 +1073,8 @@ AZB_HD int rollout_steps(Game<P>& g, const Philox& rng, uint32_t gid, int first_
             break;
         }
     }
-    if (valid) { sink.add(0, (uint32_t)(k_steps - remaining)); sink.add(2, rounds); }
+    sink.add(0, valid ? (uint32_t)(k_steps - remaining) : 0u);        // the whole group is here
+    sink.add(2, valid ? rounds : 0u);
     return remaining;
 }
 

@@ -1,10 +1,11 @@
 // azb_tc.cuh -- pieces shared by the tensor-core kernels (azb_policy.cu: the fused policy step; azb_update.cu: the
-// Agent.update forward / backward): tile geometry and the shared-memory weight image, tcgen05 / TMEM / mbarrier / bulk-copy
-// PTX wrappers, the in-kernel observation builder (game_runner.py:56-72).  Device only.
+// Agent.update forward / backward): tile geometry and the shared-memory weight image, tcgen05 / TMEM / bulk-copy PTX
+// wrappers (the mbarrier ones are in azb_mbar.cuh), the in-kernel observation builder (game_runner.py:56-72).  Device only.
 #pragma once
 #include <cuda_fp16.h>
 #include <stdint.h>
 
+#include "azb_mbar.cuh"
 #include "azb_rules.cuh"
 
 using namespace azb;
@@ -59,21 +60,6 @@ constexpr uint32_t TMEM_COLS = 512;
 // ---- PTX wrappers --------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
-{
-    uint32_t ok;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    } while (!ok);
-}
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
