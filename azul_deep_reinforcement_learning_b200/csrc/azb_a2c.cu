@@ -132,7 +132,9 @@ __global__ void k_returns(int64_t n, int k, double gamma, const int16_t* __restr
 {
     const int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (steps_used && (int)*steps_used < k) k = (int)*steps_used;      // decision iterations the rollout actually ran
-    double q = 0.0, total = 0.0;
+    // one running return per seat, picked by flags bit 2 (two-seat self-play records seat 2's decisions with it; the runner
+    // modes never set it, so their returns are those of the one recurrence)
+    double q1 = 0.0, q2 = 0.0, total = 0.0;
     if (g < n) {
         // backwards in groups of four: the twelve loads of a group are independent of the recurrence and in flight together
         for (int t1 = k; t1 > 0; t1 -= 4) {
@@ -146,7 +148,9 @@ __global__ void k_returns(int64_t n, int k, double gamma, const int16_t* __restr
 #pragma unroll
             for (int j = 0; j < 4; j++) {
                 if (!(f[j] & 1)) continue;
-                q = (double)r[j] + gamma * q;
+                const bool seat2 = (f[j] & 4) != 0;
+                const double q = (double)r[j] + gamma * (seat2 ? q2 : q1);
+                if (seat2) q2 = q; else q1 = q;
                 total += (double)r[j];
                 if (sl[j] >= 0) qval[sl[j]] = (float)q;
             }

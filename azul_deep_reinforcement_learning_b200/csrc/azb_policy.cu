@@ -67,6 +67,8 @@ struct PolicyArgs {
     // ---- runner mode against a frozen policy opponent (azb_policy_rollout_vs_policy, k_policy<..., OPP = true>) ----
     const unsigned char* __restrict__ opponent_packed;   // the opponent's weight image (seat 2 and seat 1's forced moves)
     uint32_t* __restrict__ opp_passes;       // [1] optional: max over CTAs and decisions of the opponent passes in one decision
+    // ---- two-seat self-play (azb_policy_rollout_selfplay, k_policy<..., BOTH = true>): player_score is then [2][n] ----
+    int32_t* __restrict__ pending;           // [2][n] scratch: decision iteration of each seat's open decision, -1 none
 };
 
 constexpr uint32_t PURPOSE_POLICY = 4;
@@ -220,11 +222,16 @@ __device__ __forceinline__ RowPart load_part(const float* parts, int slot)
 // random opponent then has nothing to play; the agent's image comes back for the next decision.
 // GREEDY: the runner mode against the greedy agent (azb_policy_rollout_vs_greedy): the runner block's opponent loop picks the
 // greedy agent's moves instead of the random agent's; nothing else differs.
+// BOTH: two-seat self-play (azb_policy_rollout_selfplay): each decision iteration is one pass of the tile loop in which every
+// live game's mover plays the network's move (act_filter 0) and a mover with >= 2 legal actions is recorded, with its seat in
+// flags bit 2; then the rounds that pass ended are finished (no fresh games), and a closing block takes each seat's reward
+// when that seat is next to decide, or when the game is over or stuck.  There is no opponent and no runner block.
 constexpr int MAX_OPP_PASSES = 64;           // the bound of the eager loop (selfplay.py _opponent_policy_moves)
-template <int POOL, int MODE, bool FULL, bool OPP = false, bool GREEDY = false>
+template <int POOL, int MODE, bool FULL, bool OPP = false, bool GREEDY = false, bool BOTH = false>
 __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
 {
     static_assert(!(GREEDY && OPP), "one opponent per launch: a frozen network or the greedy agent");
+    static_assert(!(BOTH && (OPP || GREEDY)), "two-seat self-play has no opponent");
     extern __shared__ __align__(128) unsigned char smem[];
     const int tid = threadIdx.x, warp = tid >> 5, row = tid & (TILE_M - 1), part = tid >> 7;
     unsigned char* a_tile = smem + OFF_A;
@@ -317,6 +324,15 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
             __syncthreads();                           // the list is reused by the next group
         }
     };
+
+    if (BOTH) {
+        // no seat has an open decision yet.  The closing block's thread of a game is the one that clears its entries here
+        // (same loop over this CTA's tiles), so program order is all the ordering needed
+        for (int64_t j = part; j < my_tiles; j += PARTS) {
+            const int64_t g = ((int64_t)blockIdx.x + j * gridDim.x) * TILE_M + row;
+            if (g < A.n) { A.pending[g] = -1; A.pending[A.n + g] = -1; }
+        }
+    }
 
     int it = 0;
     uint32_t w_phase = 0u, max_opp = 0u;               // OPP: parity of bar_w's next completion; most opponent passes
@@ -631,7 +647,8 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
                 // NNRunner.run_episode's per-decision record (nn_runner.py:27-45) in compact form: the warp's deciding games take
                 // consecutive slots (one atomic per warp); the packed state the decision was taken on is what the update
                 // kernel rebuilds observation and mask from
-                const bool decides = valid && n_valid > 0 && !gm.ended();
+                // BOTH: either seat's move is recorded when it had a choice (game_runner.py:46 applied to both seats)
+                const bool decides = valid && (BOTH ? n_valid >= 2 : n_valid > 0) && !gm.ended();
                 const uint32_t votes = __ballot_sync(0xFFFFFFFFu, decides);
                 uint32_t base = 0;
                 if (votes && (tid & 31) == 0) base = atomicAdd(A.n_dec, (uint32_t)__popc(votes));
@@ -646,7 +663,8 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
                 }
                 if (valid) {
                     A.slot_rec[(int64_t)it * A.n + g] = fits ? (int32_t)slot : -1;
-                    A.flags_rec[(int64_t)it * A.n + g] = decides ? 1 : 0;         // bit 1 (done) is added by the opponent phase
+                    // bit 1 (done) is added by the opponent phase (BOTH: the closing block); BOTH: bit 2 = seat 2 decided
+                    A.flags_rec[(int64_t)it * A.n + g] = decides ? (BOTH && gm.current_player() != 1u ? 5 : 1) : 0;
                 }
             }
             // Only the cheap, uniform part of Azul.step runs here (move, next player).  Games whose round just ended --
@@ -734,7 +752,61 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
     // ---- the rare, long part of Azul.step, or the runner mode's closing of the decision ----
     __syncthreads();                                   // every state / done / status write of the tile loop is visible to the CTA
     bool any_alive = true;
-    if (A.runner_mode) {
+    if (BOTH) {
+        // two-seat self-play: finish the rounds the pass ended (as azb_policy_step(apply_step = 1) does), then, one thread per
+        // game, open the decision the pass recorded and close the decisions whose seat is next to decide (or all of them
+        // when the game is over or stuck): reward = d_s - player_score[s], then player_score[s] = d_s, where d_s is seat s's
+        // score preview minus the other seat's.  For a finished episode a seat's rewards therefore sum to d_s at the end.
+        bool unused = false;
+        finish_flagged(A.done_out, A.status_out, unused);
+        bool alive = false;
+        for (int64_t j = part; j < my_tiles; j += PARTS) {                 // warp-uniform trip count
+            const int64_t g = ((int64_t)blockIdx.x + j * gridDim.x) * TILE_M + row;
+            if (g >= A.n) continue;
+            const int64_t cell = (int64_t)it * A.n + g;
+            const uint8_t f = A.flags_rec[cell];
+            A.reward_rec[cell] = 0;                                        // until the decision is closed
+            if (f & 1) A.pending[((f & 4) ? A.n : 0) + g] = it;
+            Game<2> h;
+            h.load(A.state, A.n, g);
+            uint32_t m2[6];
+            legal_mask(h, m2);
+            const int n_valid = popc(m2[0]) + popc(m2[1]) + popc(m2[2]) + popc(m2[3]) + popc(m2[4]) + popc(m2[5]);
+            const bool over = h.ended();
+            if (!over && n_valid == 0 && !(h.status() & ST_STUCK)) {
+                h.add_status(ST_STUCK);
+                h.store(A.state, A.n, g);
+            }
+            const bool stuck = (h.status() & ST_STUCK) != 0u;
+            const int mover = h.current_player() == 1u ? 0 : 1;
+            const bool all = over || stuck;
+            if (all || n_valid >= 2) {
+                Game<2> cp = h;                                            // game_runner.py:48-50: score preview on a copy
+                count_score<2, POOL>(cp);
+                const int32_t d1 = (int32_t)(cp.scf[0] & 0xFFFFu) - (int32_t)(cp.scf[1] & 0xFFFFu);
+#pragma unroll
+                for (int s = 0; s < 2; s++) {
+                    if (!all && s != mover) continue;
+                    const int32_t t = A.pending[s * A.n + g];
+                    if (t < 0) continue;
+                    const int32_t d = s == 0 ? d1 : -d1;
+                    const int64_t sg = s * A.n + g, tg = (int64_t)t * A.n + g;
+                    A.reward_rec[tg] = (int16_t)(d - (int32_t)A.player_score[sg]);
+                    A.player_score[sg] = (int16_t)d;
+                    A.flags_rec[tg] = (uint8_t)(1 | (over ? 2 : 0) | (s ? 4 : 0));
+                    A.pending[sg] = -1;
+                }
+            }
+            if (A.done_out) A.done_out[g] = over ? 1 : 0;
+            if (A.status_out) A.status_out[g] |= (uint8_t)h.status();
+            if (A.mask6_out) {
+#pragma unroll
+                for (int p = 0; p < 6; p++) A.mask6_out[p * A.n + g] = m2[p];
+            }
+            alive |= !all;
+        }
+        any_alive = __syncthreads_or(alive ? 1 : 0) != 0;
+    } else if (A.runner_mode) {
         // GameRunner.step after the agent's move (game_runner.py:46-55), one thread per game of this CTA's tiles: finish the
         // round the move may have ended, let the random opponent (GREEDY: the greedy agent) play until seat 1 is to move with
         // >= 2 legal actions (or the game is over), take the reward from a score preview, and close the decision's record.
@@ -841,17 +913,17 @@ __global__ void k_pack_weights(const float* __restrict__ w1a, const float* __res
     }
 }
 
-template <int POOL, int MODE, bool FULL, bool OPP = false, bool GREEDY = false>
+template <int POOL, int MODE, bool FULL, bool OPP = false, bool GREEDY = false, bool BOTH = false>
 static int launch_policy(const PolicyArgs& A, int grid, cudaStream_t stream)
 {
-    AZB_CUDA(cudaFuncSetAttribute(k_policy<POOL, MODE, FULL, OPP, GREEDY>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    AZB_CUDA(cudaFuncSetAttribute(k_policy<POOL, MODE, FULL, OPP, GREEDY, BOTH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;       // see griddepcontrol in k_policy
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    AZB_CUDA(cudaLaunchKernelEx(&cfg, k_policy<POOL, MODE, FULL, OPP, GREEDY>, A));
+    AZB_CUDA(cudaLaunchKernelEx(&cfg, k_policy<POOL, MODE, FULL, OPP, GREEDY, BOTH>, A));
     return 0;
 }
 
@@ -893,7 +965,7 @@ int azb_policy_step(azb_t* h, uint32_t* state, const void* packed, int mode, int
     A.entropy_out = entropy_out; A.done_out = done_out; A.status_out = status_out; A.mask6_out = mask6_out;
     A.k_decisions = 1; A.runner_mode = 0; A.player_score = nullptr; A.n_dec = nullptr; A.rec_cap = 0; A.state_rec = nullptr;
     A.action_rec = nullptr; A.logp_rec = nullptr; A.value_rec = nullptr; A.slot_rec = nullptr; A.reward_rec = nullptr;
-    A.flags_rec = nullptr; A.steps_used = nullptr; A.opponent_packed = nullptr; A.opp_passes = nullptr;
+    A.flags_rec = nullptr; A.steps_used = nullptr; A.opponent_packed = nullptr; A.opp_passes = nullptr; A.pending = nullptr;
     const int64_t tiles = (h->n_games + pol::TILE_M - 1) / pol::TILE_M;
     const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
     int rc = 0;
@@ -927,7 +999,7 @@ int azb_policy_rollout(azb_t* h, uint32_t* state, const void* packed, int mode, 
     A.k_decisions = k_decisions; A.runner_mode = runner_mode; A.player_score = player_score; A.n_dec = n_dec; A.rec_cap = rec_cap;
     A.state_rec = state_rec; A.action_rec = action_rec; A.logp_rec = logp_rec; A.value_rec = value_rec; A.slot_rec = slot_rec;
     A.reward_rec = reward_rec; A.flags_rec = flags_rec; A.steps_used = steps_used;
-    A.opponent_packed = nullptr; A.opp_passes = nullptr;
+    A.opponent_packed = nullptr; A.opp_passes = nullptr; A.pending = nullptr;
     const int64_t tiles = (h->n_games + pol::TILE_M - 1) / pol::TILE_M;
     const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
     int rc = 0;
@@ -961,7 +1033,7 @@ int azb_policy_rollout_vs_policy(azb_t* h, uint32_t* state, const void* packed, 
     A.k_decisions = k_decisions; A.runner_mode = 1; A.player_score = player_score; A.n_dec = n_dec; A.rec_cap = rec_cap;
     A.state_rec = state_rec; A.action_rec = action_rec; A.logp_rec = logp_rec; A.value_rec = value_rec; A.slot_rec = slot_rec;
     A.reward_rec = reward_rec; A.flags_rec = flags_rec; A.steps_used = steps_used;
-    A.opponent_packed = (const unsigned char*)opponent_packed; A.opp_passes = opp_passes;
+    A.opponent_packed = (const unsigned char*)opponent_packed; A.opp_passes = opp_passes; A.pending = nullptr;
     const int64_t tiles = (h->n_games + pol::TILE_M - 1) / pol::TILE_M;
     const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
     int rc = 0;
@@ -994,12 +1066,45 @@ int azb_policy_rollout_vs_greedy(azb_t* h, uint32_t* state, const void* packed, 
     A.k_decisions = k_decisions; A.runner_mode = 1; A.player_score = player_score; A.n_dec = n_dec; A.rec_cap = rec_cap;
     A.state_rec = state_rec; A.action_rec = action_rec; A.logp_rec = logp_rec; A.value_rec = value_rec; A.slot_rec = slot_rec;
     A.reward_rec = reward_rec; A.flags_rec = flags_rec; A.steps_used = steps_used;
-    A.opponent_packed = nullptr; A.opp_passes = nullptr;
+    A.opponent_packed = nullptr; A.opp_passes = nullptr; A.pending = nullptr;
     const int64_t tiles = (h->n_games + pol::TILE_M - 1) / pol::TILE_M;
     const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
     int rc = 0;
     if (h->tile_pool == AZB_POOL_LID) rc = mode == 0 ? pol::launch_policy<1, 0, false, false, true>(A, grid, (cudaStream_t)stream) : pol::launch_policy<1, 1, false, false, true>(A, grid, (cudaStream_t)stream);
     else rc = mode == 0 ? pol::launch_policy<0, 0, false, false, true>(A, grid, (cudaStream_t)stream) : pol::launch_policy<0, 1, false, false, true>(A, grid, (cudaStream_t)stream);
+    if (rc) return rc;
+    CHECK_LAUNCH();
+    return 0;
+}
+
+int azb_policy_rollout_selfplay(azb_t* h, uint32_t* state, const void* packed, int mode, int k_decisions,
+                                int16_t* player_score, int32_t* pending, uint32_t* n_dec, int64_t rec_cap, uint32_t* state_rec,
+                                uint8_t* action_rec, float* logp_rec, float* value_rec, int32_t* slot_rec, int16_t* reward_rec,
+                                uint8_t* flags_rec, uint32_t* steps_used, uint32_t* mask6_out, uint8_t* done_out,
+                                uint8_t* status_out, void* stream)
+{
+    CHECK_HANDLE(h);
+    if (!state || !packed) return azb_fail(AZB_E_INVALID, "null buffer%s");
+    if (h->players != 2) return azb_fail(AZB_E_INVALID, "the policy network is defined for 2 players (136 inputs, agent.py:29)%s");
+    if (mode != 0 && mode != 1) return azb_fail(AZB_E_INVALID, "mode must be 0 (sample) or 1 (argmax)%s");
+    if (k_decisions < 1) return azb_fail(AZB_E_INVALID, "k_decisions must be >= 1%s");
+    if (!player_score || !pending || !n_dec || rec_cap < 1 || !state_rec || !action_rec || !slot_rec || !reward_rec || !flags_rec)
+        return azb_fail(AZB_E_INVALID, "self-play needs player_score, pending, n_dec, rec_cap and the state / action / slot / reward / flags records%s");
+    pol::PolicyArgs A;
+    A.state_in = state; A.state = state; A.n = h->n_games; A.packed = (const unsigned char*)packed;
+    A.k0 = (uint32_t)h->seed; A.k1 = (uint32_t)(h->seed >> 32); A.gid0 = (uint32_t)h->game_id_base;
+    A.mode = mode; A.apply_step = 1; A.first_rule = h->first_player; A.counters = nullptr; A.act_filter = 0;
+    A.logits_out = nullptr; A.value_out = nullptr; A.action_out = nullptr; A.logp_out = nullptr; A.entropy_out = nullptr;
+    A.done_out = done_out; A.status_out = status_out; A.mask6_out = mask6_out;
+    A.k_decisions = k_decisions; A.runner_mode = 1; A.player_score = player_score; A.n_dec = n_dec; A.rec_cap = rec_cap;
+    A.state_rec = state_rec; A.action_rec = action_rec; A.logp_rec = logp_rec; A.value_rec = value_rec; A.slot_rec = slot_rec;
+    A.reward_rec = reward_rec; A.flags_rec = flags_rec; A.steps_used = steps_used;
+    A.opponent_packed = nullptr; A.opp_passes = nullptr; A.pending = pending;
+    const int64_t tiles = (h->n_games + pol::TILE_M - 1) / pol::TILE_M;
+    const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
+    int rc = 0;
+    if (h->tile_pool == AZB_POOL_LID) rc = mode == 0 ? pol::launch_policy<1, 0, false, false, false, true>(A, grid, (cudaStream_t)stream) : pol::launch_policy<1, 1, false, false, false, true>(A, grid, (cudaStream_t)stream);
+    else rc = mode == 0 ? pol::launch_policy<0, 0, false, false, false, true>(A, grid, (cudaStream_t)stream) : pol::launch_policy<0, 1, false, false, false, true>(A, grid, (cudaStream_t)stream);
     if (rc) return rc;
     CHECK_LAUNCH();
     return 0;

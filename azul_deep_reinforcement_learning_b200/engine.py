@@ -480,6 +480,23 @@ def runner_rollout(engine, packed, records, player_score, mode=0, out=None, oppo
         None, engine._stream()))
 
 
+def selfplay_rollout(engine, packed, records, player_score, pending, mode=0, out=None):
+    """Two-seat self-play for every game slot in ONE launch (``azb_policy_rollout_selfplay``): the network plays both seats,
+    every decision with >= 2 legal actions is recorded into ``records`` (flags bit 2 marks seat 2's), and each seat's reward
+    is its score-preview lead gained since its previous decision.  ``player_score``: int16 [2, G], zeroed when the episodes
+    start (``azb_reset``, no opening moves); ``pending``: int32 [2, G] scratch.  ``out``: optional dict of mask / done /
+    status buffers that receive the final state's."""
+    r = records
+    mask, done, status = (_ptr(out["mask"]), _ptr(out["done"]), _ptr(out["status"])) if out else (None, None, None)
+    assert player_score.dtype == torch.int16 and player_score.shape == (2, engine.n_games) and player_score.is_contiguous()
+    assert pending.dtype == torch.int32 and pending.shape == (2, engine.n_games) and pending.is_contiguous()
+    _lib.check(engine.lib.azb_policy_rollout_selfplay(
+        engine._h, _ptr(engine.state), _ptr(packed.buf), int(mode), r.k, _ptr(player_score), _ptr(pending), _ptr(r.meta),
+        r.cap, _ptr(r.state_rec), _ptr(r.action_rec), _ptr(r.logp_rec), _ptr(r.value_rec), _ptr(r.slot_rec),
+        _ptr(r.reward_rec), _ptr(r.flags_rec), ctypes.c_void_p(r.meta.data_ptr() + 4), mask, done, status,
+        engine._stream()))
+
+
 def train_stats(engine, records, loss_sums, out):
     """The 18 batch statistics (``azb_train_stats``) into ``out`` (float64 [18]) in one launch."""
     _lib.check(engine.lib.azb_train_stats(engine._h, _ptr(engine.state), _ptr(records.meta), records.cap, _ptr(loss_sums),

@@ -3,7 +3,9 @@
 ``BatchedGameRunner`` is G copies of the reference's 2-player env wrapper advancing in lock-step on one
 GPU: seat 1 is the learning agent, seat 2 a random agent (``RandomAgent``, game_runner.py:87-97, drawing
 from the Philox schedule), the greedy agent (``azb_greedy_action``: the best one-move score) or a frozen network.
-``PersistentEpisodes`` plays whole episodes in one launch of the fused policy kernel; that is how the trainer plays.  ``run_episodes`` is the step-wise loop the persistent
+``PersistentEpisodes`` plays whole episodes in one launch of the fused policy kernel; that is how the trainer plays.
+``SelfPlayEpisodes`` plays both seats with the one network in one such launch and keeps both seats' decisions.
+``run_episodes`` is the step-wise loop the persistent
 kernel is checked against: one agent decision costs up to three launches, the observation
 (``azb_observe_bf16``, only when the caller records it), the fused policy kernel (``azb_policy_step``: MLP on
 tcgen05 + masked softmax + sampling + the agent's ``Azul.step``) and the opponent loop + reward
@@ -14,7 +16,7 @@ import os
 import torch
 
 from .engine import (BatchedAzul, EpisodeRecords, PackedPolicy, discounted_returns_records, mask_to_bool, policy_step,
-                     rules_to_ints, runner_rollout)
+                     rules_to_ints, runner_rollout, selfplay_rollout)
 
 DEFAULT_RULES = {"first_player": "Random", "tile_pool": "Lid"}      # game_runner.py:23
 GREEDY = "greedy"                   # the opponent keyword of the greedy agent
@@ -220,6 +222,53 @@ class PersistentEpisodes:
         return r
 
 
+# Default record capacity per game of SelfPlayEpisodes.  Counted over 65,536 episodes of two untrained networks (both seats'
+# decisions, profiles/README.md "Two-seat self-play"): 70.2 - 71.3 per episode when sampling (single episodes up to 168),
+# 89 - 111 with argmax.  144 is twice the sampled mean and above the argmax means; overflow is reported, not silent.
+SELFPLAY_DECISIONS_PER_GAME = 144
+
+
+class SelfPlayEpisodes:
+    """Two-seat self-play for every game slot of ``engine`` (a 2-player ``BatchedAzul``) in ONE persistent launch of the
+    fused policy kernel (``azb_policy_rollout_selfplay``): the network in ``packed`` plays both seats, and every move made
+    with >= 2 legal actions -- seat 2's too -- becomes a decision record (flags bit 2 marks seat 2's).  A seat's reward is
+    the change of its score-preview lead (its score minus the other seat's after ``count_score`` on a copy) from its
+    decision to its next one, or to the end of the game, so a finished episode's rewards sum to the final lead per seat and
+    the two seats' sums cancel.  The discounted returns run per seat.
+
+    ``max_decisions`` bounds the decision iterations (one move per live game each, recorded or not); a game still running
+    then counts as unfinished.  ``capacity``: records for the whole batch (overflow is reported by ``azb_train_stats``).
+    :meth:`run` returns the ``EpisodeRecords``, like :meth:`PersistentEpisodes.run`; nothing in it waits for the GPU, so a
+    whole training batch can be captured in a CUDA graph."""
+
+    def __init__(self, engine, packed, max_decisions=320, capacity=None, want_logp_value=False):
+        if engine.players != 2:
+            raise ValueError("two-seat self-play needs a 2-player engine (the network's 136 inputs are 2-player)")
+        self.engine, self.packed = engine, packed
+        n, dev = engine.n_games, engine.device
+        if capacity is None:                       # small batches get the full K x G
+            capacity = max_decisions * n if n <= 4096 else SELFPLAY_DECISIONS_PER_GAME * n
+        self.records = EpisodeRecords(engine, max_decisions, capacity, want_logp_value)
+        self.player_score = torch.zeros((2, n), dtype=torch.int16, device=dev)     # [seat - 1, game]
+        self.pending = torch.full((2, n), -1, dtype=torch.int32, device=dev)       # kernel scratch
+        self.out = {"mask": torch.zeros((6, n), dtype=torch.int32, device=dev),
+                    "done": torch.zeros(n, dtype=torch.uint8, device=dev),
+                    "status": torch.zeros(n, dtype=torch.uint8, device=dev)}
+
+    def start(self):
+        """Fresh games in every slot (``azb_reset``; no opening moves) and both seats' score baselines at 0."""
+        self.engine.reset()
+        self.player_score.zero_()
+
+    def run(self, gamma=0.99, mode=0):
+        r = self.records
+        self.start()
+        r.clear()
+        selfplay_rollout(self.engine, self.packed, r, self.player_score, self.pending, mode=mode, out=self.out)
+        discounted_returns_records(self.engine, r, gamma)
+        return r
+
+
 def load_network(net, device=None):
     """An ``ActorCritic`` from a module, a ``state_dict``, a trainer checkpoint dict (``{"ac_net": ...}``) or a file path (every
     format ``Agent(base_net_file=...)`` accepts, through ``azulnet.agent.load_ac_net``)."""
@@ -243,6 +292,30 @@ def resolve_opponent(engine, opponent, device=None):
     if opponent is None or (isinstance(opponent, str) and opponent == GREEDY):
         return opponent
     return PackedPolicy(engine, load_network(opponent, device))
+
+
+def discounted_returns_two_seat(reward, flags, gamma):
+    """Per-seat discounted returns over two-seat self-play records, [T, G]: each seat's decisions (flags bit 0, seat 2's
+    with bit 2) form their own sequence, q = r + gamma * q' over it, where q' belongs to the same seat's next decision;
+    cells without a decision are 0.  Computed per seat on the decisions gathered in order, then scattered back."""
+    T, G = reward.shape
+    q = torch.zeros_like(reward)
+    on = (flags & 1) != 0
+    seat2 = (flags & 4) != 0
+    for sel in (on & ~seat2, on & seat2):
+        # rank of each decision among its game's decisions of this seat, counted from the back
+        rank = torch.flip(torch.cumsum(torch.flip(sel.long(), [0]), 0), [0]) - 1       # [T, G]
+        n_max = int(sel.sum(0).max()) if T else 0
+        dense = torch.zeros((n_max + 1, G), dtype=reward.dtype, device=reward.device)
+        col = torch.arange(G, device=reward.device).expand(T, G)
+        dense[rank[sel], col[sel]] = reward[sel]
+        run = torch.zeros_like(dense[0])
+        qd = torch.zeros_like(dense)
+        for i in range(n_max):                   # dense row i = the i-th decision from the back
+            run = dense[i] + gamma * run
+            qd[i] = run
+        q[sel] = qd[rank[sel], col[sel]]
+    return q
 
 
 def discounted_returns(reward, active, gamma):

@@ -3,6 +3,7 @@ equivalent (reference scripts/training.py:8-22, nn_runner.py:53-84, agent.py:39-
 
     python -m azul_deep_reinforcement_learning_b200.train [batch_size] [net_name] [--batches N]
                                                       [--opponent FILE|greedy] [--opponent-refresh N]
+                                                      [--self-play] [--eval-every N] [--eval-games E]
     torchrun --nproc-per-node 8 -m azul_deep_reinforcement_learning_b200.train 1024 run1
 
 ``batch_size`` episodes are played IN PARALLEL per rank (one game slot each) instead of one after the
@@ -25,7 +26,7 @@ import torch.distributed as dist
 from . import parallel
 from .azulnet.model import ActorCritic
 from .engine import PackedPolicy, UpdateGradients, train_stats
-from .selfplay import GREEDY, BatchedGameRunner, PersistentEpisodes, resolve_opponent
+from .selfplay import GREEDY, BatchedGameRunner, PersistentEpisodes, SelfPlayEpisodes, resolve_opponent
 
 ACTOR_COEFF, CRITIC_COEFF, ENTROPY_COEFF = 1.0, 0.5, 0.1          # agent.py:47-49
 
@@ -100,6 +101,9 @@ def summarize_stats(s, update_sync_s=None):
     return out
 
 
+EVAL_FIELDS = ("eval_win_percent", "eval_player_score", "eval_opponent_score")     # train(eval_every=N) columns
+
+
 class SelfPlayTrainer:
     """``NNRunner.train`` (nn_runner.py:53-84) with ``games_per_rank`` episodes played in parallel per rank.
 
@@ -113,11 +117,21 @@ class SelfPlayTrainer:
     ``opponent``: None plays the random agent (``RandomAgent``); ``"greedy"`` the greedy agent (the best one-move score, a
     fixed-strength yardstick); an ``ActorCritic``, a ``state_dict`` or a file path (anything ``Agent(base_net_file=...)``
     loads) plays a frozen network in seat 2 (``GameRunner(opponent=Agent(...))``), sampling like the agent.  ``opponent_refresh`` = N > 0: the opponent's weights are replaced by the current network's
-    after every N batches -- self-play against a lagged copy of itself."""
+    after every N batches -- self-play against a lagged copy of itself.
+
+    ``self_play=True``: the network plays BOTH seats (``SelfPlayEpisodes``, one persistent launch per batch) and learns from
+    every decision with a choice, seat 2's included; it takes no ``opponent`` or ``opponent_refresh``.  ``max_decisions``
+    then bounds the moves of both seats together (default 320; 160 agent decisions otherwise).  The batch statistics keep
+    their meaning -- seat 1 against seat 2, decisions of both seats -- so ``reward`` is 0 when every episode finished (the
+    two seats' rewards cancel) and the scores and ``win_percent`` are symmetric up to noise: ``train(eval_every=N)``
+    measures progress against the greedy agent instead."""
 
     def __init__(self, games_per_rank=1024, learning_rate=3e-4, gamma=0.99, seed=0, device=0, rank=0, world=1,
-                 rules=None, max_decisions=160, tf32_update=True, opponent=None, opponent_refresh=0):
+                 rules=None, max_decisions=None, tf32_update=True, opponent=None, opponent_refresh=0, self_play=False):
+        if self_play and (opponent is not None or opponent_refresh):
+            raise ValueError("self_play plays both seats with the network: it takes no opponent or opponent_refresh")
         self.rank, self.world, self.gamma = rank, world, gamma
+        self.rules, self.self_play = rules, bool(self_play)
         self.tf32_update = tf32_update
         self.device = torch.device("cuda", device)
         torch.manual_seed(seed)                              # identical initial weights on every rank
@@ -137,7 +151,10 @@ class SelfPlayTrainer:
         self.runner.opponent, self.runner.opponent_mode = resolve_opponent(self.runner.engine, opponent, self.device), 0
         if isinstance(self.runner.opponent, PackedPolicy):
             self.opponent = self.runner.opponent
-        self.episodes = PersistentEpisodes(self.runner, self.packed, max_decisions=max_decisions)
+        if self.self_play:
+            self.episodes = SelfPlayEpisodes(self.runner.engine, self.packed, max_decisions=max_decisions or 320)
+        else:
+            self.episodes = PersistentEpisodes(self.runner, self.packed, max_decisions=max_decisions or 160)
         # every parameter gradient is a view into ONE flat fp32 buffer (PARAM_ORDER): the tensor-core kernels add into
         # it, autograd accumulates into the views in place, and the gradient all-reduce is a single collective on it
         self.tc = UpdateGradients(self.runner.engine, self.episodes.records.cap)
@@ -151,8 +168,8 @@ class SelfPlayTrainer:
 
     # ---- rollout ---------------------------------------------------------------------------
     def rollout(self):
-        """Every game slot plays one episode; returns the ``EpisodeRecords`` of the agent's decisions with their discounted
-        returns."""
+        """Every game slot plays one episode; returns the ``EpisodeRecords`` of the agent's decisions (self-play: both
+        seats') with their discounted returns."""
         with torch.no_grad():
             self.packed.update(self.net)
             return self.episodes.run(self.gamma)
@@ -308,18 +325,34 @@ class SelfPlayTrainer:
         self.load_parameters(load_ac_net(path).state_dict())
         return 0
 
-    def train(self, batches=1000, net_name=None, log=print, start_batch=0, checkpoint_every=1000, graph=True):
+    def evaluate_greedy(self, games=2048):
+        """The current network (seat 1, argmax) against the greedy agent over ``games`` episodes: the ``EVAL_FIELDS``."""
+        from .evaluate import evaluate
+        ev = evaluate(self.net, "greedy", games=games, mode=1, seed=self.rank, device=self.device.index, rules=self.rules)
+        return {"eval_win_percent": ev["win_percent"], "eval_player_score": ev["player_score"],
+                "eval_opponent_score": ev["opponent_score"]}
+
+    def train(self, batches=1000, net_name=None, log=print, start_batch=0, checkpoint_every=1000, graph=True, eval_every=0,
+              eval_games=2048):
         """Batches ``start_batch + 1 .. batches``.  With ``net_name``: one CSV row per batch in ``<net_name>.csv``
         (appended to when resuming) and ``<net_name>.pt`` every ``checkpoint_every`` batches and at the end.  The host
-        never waits for the batch it just launched: a batch's statistics are read (and logged) while the next one runs."""
-        writer = fh = None
-        marks = []                                           # (batch number, host time at launch)
+        never waits for the batch it just launched: a batch's statistics are read (and logged) while the next one runs.
 
-        def finish(b, t_launch):
+        ``eval_every`` = N > 0: after every N-th batch rank 0 plays :meth:`evaluate_greedy` (``eval_games`` episodes) with
+        the network that batch produced; every row then has the ``EVAL_FIELDS`` columns, blank between evaluations.  An
+        evaluation waits for the GPU, and its time counts towards the evaluated batch's ``batch_s``."""
+        if eval_every < 0:
+            raise ValueError("eval_every must be >= 0")
+        writer = fh = None
+        marks = []                                           # (batch number, host time at launch, evaluation or None)
+
+        def finish(b, t_launch, ev):
             nonlocal writer, fh
             st = self.fetch_stats()
             now = time.perf_counter()
             st.update(batch=b, batch_s=now - t_launch, games_per_sec=st["games"] / max(now - t_launch, 1e-9))
+            if eval_every > 0:
+                st.update(ev or dict.fromkeys(EVAL_FIELDS))
             self.history.append(st)
             if self.rank != 0:
                 return
@@ -336,13 +369,18 @@ class SelfPlayTrainer:
                 log("batch %d: %.0f games/s  reward %.2f  score %.1f vs %.1f  win %.1f%%  loss %.3f" % (
                     b, st["games_per_sec"], st["reward"], st["player_score"], st["opponent_score"],
                     100 * st["win_percent"], st["ac_loss"]))
+                if ev:
+                    log("batch %d: vs greedy (argmax) win %.1f%%  score %.1f vs %.1f" % (
+                        b, 100 * ev["eval_win_percent"], ev["eval_player_score"], ev["eval_opponent_score"]))
 
         for b in range(start_batch, batches):
             if graph and self._graph is None and b >= start_batch + 2:
                 self.enable_step_graph(warmup=0)             # the first two batches ran launch by launch (lazy initialisation)
             t0 = time.perf_counter()
             self.step(defer_stats=True)
-            marks.append((b + 1, t0))
+            # the evaluation is queued behind this batch's update on the stream: it plays the network that batch produced
+            ev = self.evaluate_greedy(eval_games) if eval_every > 0 and self.rank == 0 and (b + 1) % eval_every == 0 else None
+            marks.append((b + 1, t0, ev))
             if len(marks) > 1:                               # the previous batch's numbers are on the host by now
                 finish(*marks.pop(0))
             if self.rank == 0 and net_name is not None and ((b + 1) % checkpoint_every == 0 or b + 1 == batches):
@@ -372,9 +410,22 @@ def parse_args(argv=None):
     ap.add_argument("--opponent-refresh", type=int, default=0, metavar="N",
                     help="replace the opponent by the current network after every N batches (self-play against a lagged "
                          "copy; without --opponent it starts as the initial network)")
+    ap.add_argument("--self-play", action="store_true",
+                    help="the network plays both seats and learns from both seats' decisions (no --opponent, no "
+                         "--opponent-refresh; the logged reward is then 0)")
+    ap.add_argument("--eval-every", type=int, default=0, metavar="N",
+                    help="after every N batches play the network (argmax) against the greedy agent and log "
+                         "eval_win_percent / eval_player_score / eval_opponent_score (default 0: never)")
+    ap.add_argument("--eval-games", type=int, default=2048, metavar="E", help="episodes per evaluation (default 2048)")
     args = ap.parse_args(argv)
     if args.opponent_refresh < 0:
         ap.error("--opponent-refresh must be >= 0")
+    if args.self_play and (args.opponent is not None or args.opponent_refresh):
+        ap.error("--self-play plays both seats with the network: it cannot be combined with --opponent or --opponent-refresh")
+    if args.eval_every < 0:
+        ap.error("--eval-every must be >= 0")
+    if args.eval_games < 1:
+        ap.error("--eval-games must be >= 1")
     if args.opponent == GREEDY and args.opponent_refresh:
         ap.error("--opponent-refresh replaces a network opponent: it does not apply to --opponent greedy")
     return args
@@ -387,9 +438,10 @@ def main(argv=None):
         parallel.init("nccl", local)
     torch.cuda.set_device(local)
     tr = SelfPlayTrainer(args.batch_size, learning_rate=args.lr, seed=args.seed, device=local, rank=rank, world=world,
-                         opponent=args.opponent, opponent_refresh=args.opponent_refresh)
+                         opponent=args.opponent, opponent_refresh=args.opponent_refresh, self_play=args.self_play)
     start = tr.load_checkpoint(args.resume) if args.resume else 0
-    tr.train(batches=args.batches, net_name=args.net_name, start_batch=start, checkpoint_every=args.checkpoint_every)
+    tr.train(batches=args.batches, net_name=args.net_name, start_batch=start, checkpoint_every=args.checkpoint_every,
+             eval_every=args.eval_every, eval_games=args.eval_games)
     if world > 1:
         dist.destroy_process_group()
 

@@ -248,10 +248,37 @@ int azb_policy_rollout_vs_greedy(azb_t* h, uint32_t* state, const void* packed, 
                                  uint8_t* flags_rec, uint32_t* steps_used, uint8_t* action_out, float* logp_out,
                                  float* value_out, uint32_t* mask6_out, uint8_t* done_out, uint8_t* status_out, void* stream);
 
+/* ---- K4, persistent two-seat self-play: one network plays both seats of every game for one episode per slot in ONE launch,
+ * and every decision with a choice is recorded -- seat 2's as well as seat 1's.  Seats are 1 and 2 (current_player 1 is seat
+ * 1); for a state, d_s = seat s's score preview (count_score on a copy, azb_score_preview) minus the other seat's.
+ *   Decision: in every iteration each live game's mover plays the network's move (mode 0 samples, 1 takes the argmax; the
+ *   Philox word is keyed by game and env step).  It is recorded only when the mover has >= 2 legal actions
+ *   (game_runner.py:46 applied to either seat); a single legal action is played unrecorded.  Rounds are then finished as in
+ *   azb_policy_step(apply_step = 1): the decisions equal those of repeated azb_policy_step(apply_step = 1, act_filter = 0).
+ *   Reward: player_score int16 [2][G] (seat s at [s - 1][g]) is zeroed by the caller when the episodes start (azb_reset;
+ *   there are no opening moves).  A seat's open decision is closed when that seat is next to move with >= 2 legal actions,
+ *   or when the game is over or stuck (then both seats' are): reward = d_s - player_score[s], then player_score[s] = d_s.
+ *   For a finished episode seat s's rewards therefore sum to d_s of the final state, and the two seats' sums negate each
+ *   other.  A game with no legal action gets AZB_ST_STUCK.  A reward is 0 until its decision is closed: a decision still
+ *   open when k_decisions stops the launch keeps 0, and its game counts as unfinished.
+ *   Records: those of azb_policy_rollout's runner mode, at most one decision per (iteration t, game g) cell; flags_rec bit 0
+ *   decision recorded, bit 1 game over when it was closed, bit 2 seat 2's decision.  The reward of iteration t is written
+ *   at a later iteration, when the decision is closed.
+ *   pending int32 [2][G]: device scratch (the open decision's iteration per seat), initialised by the kernel.
+ * mask6_out / done_out / status_out ([G], optional) describe the final state.  Checks as azb_policy_rollout_vs_greedy; no
+ * host synchronisation is needed, so a training batch stays one CUDA graph. */
+int azb_policy_rollout_selfplay(azb_t* h, uint32_t* state, const void* packed, int mode, int k_decisions,
+                                int16_t* player_score, int32_t* pending, uint32_t* n_dec, int64_t rec_cap, uint32_t* state_rec,
+                                uint8_t* action_rec, float* logp_rec, float* value_rec, int32_t* slot_rec, int16_t* reward_rec,
+                                uint8_t* flags_rec, uint32_t* steps_used, uint32_t* mask6_out, uint8_t* done_out,
+                                uint8_t* status_out, void* stream);
+
 /* Discounted returns of NNRunner.train (nn_runner.py:72-75) over the records of azb_policy_rollout's runner mode:
  * q_t = r_t + gamma * q_{t+1} over each game's decisions (accumulated in double like the reference's numpy loop), written
  * as float to qval[slot] (float [rec_cap]); reward_sum (double [1], optional) += the sum of all rewards; steps_used
- * (device uint32 [1], optional: azb_policy_rollout's output) bounds the walk to the decision iterations actually run. */
+ * (device uint32 [1], optional: azb_policy_rollout's output) bounds the walk to the decision iterations actually run.
+ * One running return per seat, picked by flags bit 2: two-seat self-play (azb_policy_rollout_selfplay) discounts each
+ * seat's decisions separately; the runner modes never set the bit. */
 int azb_discounted_returns(azb_t* h, int k_decisions, double gamma, const int16_t* reward_rec, const uint8_t* flags_rec,
                            const int32_t* slot_rec, float* qval, double* reward_sum, const uint32_t* steps_used, void* stream);
 

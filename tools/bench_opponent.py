@@ -1,4 +1,5 @@
-"""Whole-episode rollouts against the random opponent, a frozen policy opponent and the greedy agent, timed with CUDA events.
+"""Whole-episode rollouts against the random opponent, a frozen policy opponent and the greedy agent, and two-seat self-play,
+timed with CUDA events.
 
     python tools/bench_opponent.py [--games 16384 131072] [--reps 5] [--out FILE]
 
@@ -6,9 +7,11 @@ Per batch size: (a) the persistent runner-mode rollout vs the random opponent, (
 opponent (azb_policy_rollout_vs_policy), (c) the eager run_episodes vs the same policy opponent (one policy launch per
 agent decision, one or more opponent launches each followed by a host read, one reward launch), (d) the persistent rollout
 vs the greedy agent (azb_policy_rollout_vs_greedy), (e) the eager run_episodes vs the greedy agent (one policy launch and
-one azb_opponent_greedy launch per agent decision, a host read every 8 decisions).  A timed batch is a whole
-PersistentEpisodes.run (episode start, the rollout, discounted returns) or a whole run_episodes, after one warm-up batch.
-Reported: ms per batch, episodes/s, agent decisions/s, and the opponent passes per agent decision -- the most any CTA
+one azb_opponent_greedy launch per agent decision, a host read every 8 decisions), (f) the persistent two-seat self-play
+(azb_policy_rollout_selfplay: the agent's network plays both seats, and both seats' decisions are recorded).  A timed batch
+is a whole PersistentEpisodes.run / SelfPlayEpisodes.run (episode start, the rollout, discounted returns) or a whole
+run_episodes, after one warm-up batch.
+Reported: ms per batch, episodes/s, recorded decisions/s (row f: both seats'), and the opponent passes per agent decision -- the most any CTA
 needed in one decision (the kernel's counter) and, from a separate counting run of the eager path, the mean and maximum
 over decisions of the launches in which some game of the batch moved.  The card's name and power limit are read in the
 same run.  Both networks are randomly initialised (seed 0 / 1); the agent samples (mode 0)."""
@@ -24,7 +27,8 @@ import torch  # noqa: E402
 
 from azul_deep_reinforcement_learning_b200.azulnet.model import ActorCritic  # noqa: E402
 from azul_deep_reinforcement_learning_b200.engine import PackedPolicy, policy_step  # noqa: E402
-from azul_deep_reinforcement_learning_b200.selfplay import BatchedGameRunner, PersistentEpisodes, run_episodes  # noqa: E402
+from azul_deep_reinforcement_learning_b200.selfplay import (BatchedGameRunner, PersistentEpisodes,  # noqa: E402
+                                                            SelfPlayEpisodes, run_episodes)
 
 
 def card():
@@ -109,10 +113,18 @@ def bench(n, reps):
     pe = PackedPolicy(re_.engine, net)
     ms, batch = timed(lambda: run_episodes(re_, pe, max_decisions=160, record_obs=False), max(2, reps // 2))
     res["e_eager_vs_greedy"] = _rates(n, ms, int(batch["active"].sum()))
+
+    rf = BatchedGameRunner(n, seed=11)
+    ef = SelfPlayEpisodes(rf.engine, PackedPolicy(rf.engine, net))
+    ms, r = timed(lambda: ef.run(), reps)
+    res["f_persistent_selfplay"] = _rates(n, ms, int(r.meta[0]))
+    res["f_persistent_selfplay"]["unfinished"] = n - int(ef.out["done"].sum())
     res["b_over_a"] = res["b_persistent_vs_policy"]["ms"] / res["a_persistent_vs_random"]["ms"]
     res["d_over_a"] = res["d_persistent_vs_greedy"]["ms"] / res["a_persistent_vs_random"]["ms"]
     res["e_over_d"] = res["e_eager_vs_greedy"]["ms"] / res["d_persistent_vs_greedy"]["ms"]
     res["c_over_b"] = res["c_eager_vs_policy"]["ms"] / res["b_persistent_vs_policy"]["ms"]
+    res["f_over_a"] = res["f_persistent_selfplay"]["ms"] / res["a_persistent_vs_random"]["ms"]
+    res["f_over_b"] = res["f_persistent_selfplay"]["ms"] / res["b_persistent_vs_policy"]["ms"]
     return res
 
 
