@@ -477,8 +477,13 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
         // ---- epilogue 2a: per part -- critic partial sum and online softmax over its 48 columns ----
         // online softmax statistics over this part's legal logits, one 16-column chunk at a time and without
         // per-column branches (32 different games share a warp): chunk maximum first, one rescale, then the sum.
-        // The chunk sums (relative to the running maximum at that chunk) are kept for the sampling step.
-        float mx = -INFINITY, se = 0.0f, sl = 0.0f;
+        // The chunk sums are kept for the sampling step, rescaled to the part's maximum as it grows: the part's sum se is
+        // their sum, and the sampling step scales these same products by the part's factor 2^(mx - gmx), so that its chunk
+        // weights add up to the part's weight wq within a few roundings at any logit offset.  Every rescale is 2^ of an EXACT
+        // difference of two maxima: folding a maximum times LOG2E, rounded to fp32, into one side and not the other left a gap
+        // that grows with |mx| (3e-4 of a part's weight at |mx| ~ 1e4), where a target could land in no chunk, and below a row
+        // maximum of -88.7 gave a chunk before its part's first legal action the weight 0 * 2^(-gmx log2e) = 0 * inf = NaN.
+        float mx = -INFINITY, sl = 0.0f;
         float cs[3], cms[3];
         int amax = 0;
 #pragma unroll
@@ -513,10 +518,13 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
             // sampling mode: the weights 2^(logit - chunk maximum) -- exactly 0 for an illegal action -- replace the logits in
             // TMEM, so that the inverse-CDF scan below neither repeats the exponentials nor looks at the mask again
             if (MODE == 0) tmem_st16(tmem_row + c0, v);
-            se = se * ex2f(fmaf(mx, LOG2E, -ms2)) + sum;
+            const float r = ex2f((mx - ms) * LOG2E);                   // 2^(old - new maximum); 0 while mx = -inf
+#pragma unroll
+            for (int j = 0; j < c; j++) cs[j] *= r;
             cs[c] = sum; cms[c] = ms;
             mx = nm;
         }
+        const float se = cs[0] + cs[1] + cs[2];
         if (MODE == 0) tc_wait_st();
         {
             const int slot = part * TILE_M + row;
@@ -548,7 +556,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
         for (int q = 0; q < PARTS; q++) {
             const RowPart rp = load_part(parts, q * TILE_M + row);
             wq[q] = rp.n > 0 ? rp.s * ex2f((rp.m - gmx) * LOG2E) : 0.0f;
-            if (rp.n > 0) last_part = q;
+            if (wq[q] > 0.0f) last_part = q;
             if (q < part) prefix += wq[q];
             gse += wq[q];
         }
@@ -566,13 +574,14 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
                 run += wq[q];
                 if (owner < 0 && target < run) owner = q;
             }
-            if (owner < 0) owner = last_part;
+            if (owner < 0) owner = last_part;              // (target rounded up to gse): the last part of positive weight
             const bool mine = owner == part && n_valid > 0;
-            const float gm2 = (n_valid > 0 ? gmx : 0.0f) * LOG2E;
-            // chunk k: the first whose cumulative weight passes the target; `base` = weight before it (<= target)
-            float sc[3], wc[3];
+            // chunk k: the first whose cumulative weight passes the target; `base` = weight before it (<= target).  The chunk
+            // weights are this part's rescaled chunk sums (epilogue 2a) times the very factor wq[part] was formed with
+            const float fq = ex2f((mx - gmx) * LOG2E);
+            float wc[3];
 #pragma unroll
-            for (int c = 0; c < 3; c++) { sc[c] = ex2f(fmaf(cms[c], LOG2E, -gm2)); wc[c] = cs[c] * sc[c]; }
+            for (int c = 0; c < 3; c++) wc[c] = cs[c] * fq;
             int k = -1;
             float base = prefix, acc = prefix;
 #pragma unroll
@@ -583,11 +592,16 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
                 k = hit ? c : k;
                 acc = nacc;
             }
-            if (k < 0) {                                   // rounding left the target beyond the part: its last legal chunk
-                k = (mybits >> 32) ? 2 : ((mybits >> 16) & 0xFFFFull) ? 1 : 0;
+            if (k < 0) {
+                // rounding left the target beyond the part: its last chunk of positive weight.  A chunk of positive weight
+                // holds an action of positive weight (the scan below finds one), and the owner part has such a chunk: its
+                // weight wq > 0 is the sum of its chunks' (up to rounding), and cs > 0 at least in the chunk of its maximum.
+                // A legal chunk whose weights all underflowed against the running maximum has none -- never pick it
+                k = wc[2] > 0.0f ? 2 : wc[1] > 0.0f ? 1 : wc[0] > 0.0f ? 0 : cs[2] > 0.0f ? 2 : cs[1] > 0.0f ? 1 : 0;
                 base = prefix + (k > 0 ? wc[0] : 0.0f) + (k > 1 ? wc[1] : 0.0f);
             }
-            const float sk = k == 0 ? sc[0] : k == 1 ? sc[1] : sc[2], mk = k == 0 ? cms[0] : k == 1 ? cms[1] : cms[2];
+            const float mk = k == 0 ? cms[0] : k == 1 ? cms[1] : cms[2];
+            const float sk = ex2f((mk - mx) * LOG2E) * fq;          // chunk k's weights (relative to mk) -> the row's scale
             float vs[16];                                  // the chunk's weights relative to its own maximum mk (epilogue 2a)
 #pragma unroll
             for (int c = 0; c < 3; c++) {
@@ -619,8 +633,8 @@ __global__ void __launch_bounds__(THREADS, 1) k_policy(PolicyArgs A)
         bool issuer = false;                               // warp-uniform: this warp issues the next tile's layer 1 (below)
         if (part == 0) {
             uint32_t action = (uint32_t)gamax;
-            float la = gmx;                             // argmax mode, and the fallback if rounding left no part a winner
-            if (MODE == 0) {
+            float la = gmx;                             // argmax mode
+            if (MODE == 0) {                            // the owner part writes an action of positive weight when n_valid > 0
                 const int2 r = result[row];
                 if (r.x >= 0) { action = (uint32_t)r.x; la = __int_as_float(r.y); }
             }
@@ -878,12 +892,14 @@ __global__ void k_pack_weights(const float* __restrict__ w1a, const float* __res
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     // one thread per fp16 element of W1 / W2, then the fp32 vectors
-    // bias b as two fp16 inputs: hi = half(b), lo = half(b - hi)
-    auto split = [](float b, bool low) {
-        const float hi = __half2float(__float2half_rn(b));
+    // fp16 saturating at the largest finite value (an fp16 weight of +-inf would turn the products into inf / NaN)
+    auto to_half = [](float v) { return __float2half_rn(fminf(fmaxf(v, -65504.0f), 65504.0f)); };
+    // bias b as two fp16 inputs: hi = half(b), lo = half(b - hi), both saturating.  hi is taken from the clamped bias: for
+    // |b| >= 65520 half(b) is +-inf, lo = b - hi then clamps to -+65504 and hi to +-65504, and the bias entered as 0
+    auto split = [to_half](float b, bool low) {
+        const float hi = __half2float(to_half(b));
         return low ? b - hi : b;
     };
-    auto to_half = [](float v) { return __float2half_rn(fminf(fmaxf(v, -65504.0f), 65504.0f)); };
     if (i < N1 * K1) {
         const int n = i / K1, k = i % K1;
         float v = 0.0f;
